@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Gibbs sweeps/sec of the GP-IRT sampler (BASELINE.json metric) on synthetic data of a named n x m shape.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one Gibbs sweep (reference loop body, src/gpirtMCMC.cpp:68-78) over the whole response matrix.
   value : sweeps/s with everything resident in HBM, timed by CUDA events on the sampler's own stream inside the C library
@@ -12,6 +12,9 @@ A "step" is one Gibbs sweep (reference loop body, src/gpirtMCMC.cpp:68-78) over 
           workload) and the per-respondent log-posterior partial sums are all-reduced over NCCL once per sweep.
   --impl reference : the reference's own CPU sampler (its sources compiled against stand-in Armadillo headers,
           oracle/_ref; else the oracle port) on a bounded item sample, extrapolated linearly in m (stated in `sample`).
+  --dump-outputs DIR : after the timed sweeps, the sampler state they left (what gpirt_b200_sampler_get returns) goes to
+          DIR/<name>.npy, float64: theta and beta whole, f and f* on a fixed seeded sample of items (dump_outputs()).
+          Inputs and seeds depend on the arguments only, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -221,6 +224,29 @@ def cpu_reference_chain_ess(y, theta_init, S, B):
             "ess_per_sec_min": float(ess.min() / el), "note": "MEASURED full chain of the reference's own gpirtMCMC()"}
 
 
+DUMP_BYTES = 48 << 20    # f and f* samples of one dump, summed over ranks; theta and beta add n per rank + 2 m doubles
+DUMP_MAX_ITEMS = 256     # items sampled in all
+
+
+def dump_outputs(s, out_dir, rank=0, world=1):
+    """Writes the resident sampler's state after the last timed sweep as out_dir/<name>.npy (float64): theta (n),
+    beta (2 x m), and f (n x k) / fstar (1001 x k) of k items drawn without replacement by a fixed seed, whose indices
+    (0-based, local to this sampler's item block) go to `items`.  With world > 1 every rank writes its own item block as
+    rank<r>_<name>.npy and samples 1 / world of the items and of the byte budget.  Returns the names written."""
+    from gpirt_b200 import _lib
+    n, m = s.n, s.m
+    prefix = "rank%d_" % rank if world > 1 else ""
+    k = int(min(m, max(1, DUMP_MAX_ITEMS // world), max(1, DUMP_BYTES // world // ((n + N_GRID) * 8))))
+    items = np.sort(np.random.default_rng(synthetic.SEED + rank).choice(m, size=k, replace=False))
+    # one whole field on the host at a time: the sampled columns are copied out before the next field is read
+    arrays = {"theta": s.get(_lib.THETA), "beta": s.get(_lib.BETA), "items": items.astype(np.float64),
+              "f": s.get(_lib.F)[:, items], "fstar": s.get(_lib.FSTAR)[:, items]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+    return sorted(prefix + name for name in arrays)
+
+
 def shard_check(G, dist, rank, world, local_rank, fresh_uid):
     """N > 1: before anything is timed, the item-sharded sampler (CUDA path, NCCL exchanges) must reproduce the single-GPU
     chain on a small problem that takes the same code paths (fixed-point products, pipelined sweep, blocked-substitution
@@ -273,7 +299,11 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--ess-samples", type=int, default=300)
     ap.add_argument("--fstar-mode", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the sampler state after the last timed sweep to DIR/<name>.npy (B200 arm)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the state of the B200 sampler; --impl reference has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -365,6 +395,9 @@ def main():
         dist.barrier()
     clk = clocks.finish() if rank == 0 else None
     launches = s.launches() - launches0
+    dumped = None
+    if args.dump_outputs:                    # read-only copies of the state the timed sweeps left
+        dumped = dump_outputs(s, args.dump_outputs, rank, world)
     s.set_timing(True)                       # eager pass with CUDA-event timers around every step
     s.sweep(2)
     s.timings(reset=True)
@@ -480,6 +513,8 @@ def main():
             "data": "synthetic", "config": config, "gpu_launches": int(launches), "clocks": clk, "roofline": roofline}
     if shard_ok is not None:
         line["shard_check"] = shard_ok
+    if dumped is not None:
+        line["outputs"] = {"dir": args.dump_outputs, "arrays": dumped}
 
     # ------------------------------------------------------------------ chain-parallel mode (BASELINE config 4), N > 1 only
     # every rank runs an INDEPENDENT chain of the whole workload (own seed, no communication): aggregate sweeps/s

@@ -23,7 +23,7 @@ _bp = C.POINTER(C.c_uint8)
 
 
 def build(target="oracle"):
-    """Compile the oracle (and the compiled-reference library when /root/reference is present)."""
+    """Compile the oracle, or with target "ref" the compiled-reference library (needs have_ref_sources())."""
     subprocess.check_call(["make", "-s", "-C", _HERE, target])
 
 
@@ -262,8 +262,13 @@ def mcmc(y, theta_init, sample_iterations, burn_iterations, pm, psd, pstep, rng,
 _ref = None
 
 
+def have_ref_sources():
+    """True where oracle/Makefile finds the reference package's sources (its REF, overridden by GPIRT_REFERENCE)"""
+    return subprocess.run(["make", "-s", "-C", _HERE, "have-ref"], capture_output=True).returncode == 0
+
+
 def have_ref():
-    return os.path.exists(REF_SO) or os.path.isdir("/root/reference/src")
+    return os.path.exists(REF_SO) or have_ref_sources()
 
 
 def ref():

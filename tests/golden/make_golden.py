@@ -1,11 +1,12 @@
-"""Generates tests/golden/*.npz.  Run in the BUILD container only (needs /root/reference to compile oracle/_ref).
+"""Generates tests/golden/*.npz.  Needs the reference package's sources (a checkout of duckmayr/gpirt where
+oracle/Makefile looks for it, or named by GPIRT_REFERENCE) to compile oracle/_ref.
 
 Every golden output comes from the reference's OWN sampler sources (src/gpirtMCMC.cpp etc. compiled unmodified against
 the stand-in headers in oracle/refshim, = oracle/_ref/libgpirt_ref.so), driven by the tape of variates that the addressed
 Philox generator (oracle/gpo_rng.h) hands out for the recorded seed.  The oracle restatement and the CUDA sampler are
 both checked against these files (tests/test_oracle.py, tests/test_gpu_parity.py::test_golden_*).
 
-    python tests/golden/make_golden.py
+    GPIRT_REFERENCE=<checkout of duckmayr/gpirt> python tests/golden/make_golden.py
 """
 import os
 import sys

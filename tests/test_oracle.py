@@ -1,14 +1,16 @@
 """CPU tests of the oracle (no GPU): hand-computed values, the reference's compiled sources (oracle/_ref, only where
-/root/reference exists), and the committed golden vectors that those sources produced."""
+that library is built or oracle/Makefile finds a checkout of duckmayr/gpirt, see GPIRT_REFERENCE there), and the
+committed golden vectors that those sources produced."""
 import os
 
 import numpy as np
 import pytest
 
 from conftest import make_problem
+from oracle import oracle as _oracle
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-HAVE_REF_TREE = os.path.isdir("/root/reference/src")
+HAVE_REF = _oracle.have_ref()
 
 
 def test_philox_known_answer(O):
@@ -122,7 +124,8 @@ def test_oracle_reproduces_senate116_golden(O):
     assert np.max(np.abs(r["IRFs"][::10] - g["IRFs_every10"])) <= 1e-9
 
 
-@pytest.mark.skipif(not HAVE_REF_TREE, reason="/root/reference is only present in the build container")
+@pytest.mark.skipif(not HAVE_REF, reason="needs the reference package's own sources (GPIRT_REFERENCE: a checkout of "
+                                         "duckmayr/gpirt); without them only the whole-chain goldens above compare with it")
 class TestAgainstCompiledReference:
     """The restatement against the reference's own sources (oracle/_ref) on replayed tapes: bit-exact."""
 
