@@ -19,6 +19,7 @@ EXPORTS = [
     "gpirt_b200_sampler_launches", "gpirt_b200_sampler_uses",
     "gpirt_b200_sampler_destroy", "gpirt_b200_se_cov", "gpirt_b200_chol_lower", "gpirt_b200_dgemm", "gpirt_b200_dgemm_i8",
     "gpirt_b200_trsm_lower", "gpirt_b200_ll_bar", "gpirt_b200_fp64_peak_tflops", "gpirt_b200_int8_peak_tops", "gpirt_b200_int8_peak_tops_random", "gpirt_b200_rng_probe", "gpirt_b200_response_matrix", "gpirt_b200_theta_diagnostics",
+    "gpirt_b200_predictive_accumulate_time",
 ]
 
 # enums of include/gpirt_b200.h
@@ -35,11 +36,20 @@ class GpirtError(RuntimeError):
         self.status = status
 
 
+class Fit(C.Structure):
+    """gpirt_b200_fit: posterior predictive summaries accumulated on the device (include/gpirt_b200.h)"""
+    _fields_ = [("y_holdout", C.POINTER(C.c_double)), ("pred", C.POINTER(C.c_double)), ("lpd_cell", C.POINTER(C.c_double)),
+                ("pwaic_cell", C.POINTER(C.c_double)), ("elpd_item", C.POINTER(C.c_double)),
+                ("elpd_resp", C.POINTER(C.c_double)), ("lppd", C.c_double), ("p_waic", C.c_double),
+                ("elpd_waic", C.c_double), ("waic", C.c_double), ("se_elpd_waic", C.c_double), ("lpd_holdout", C.c_double),
+                ("n_obs", C.c_int64), ("n_holdout", C.c_int64)]
+
+
 class Opts(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("device", C.c_int32), ("fstar_mode", C.c_int32), ("skip_f_draws", C.c_int32),
                 ("use_graph", C.c_int32), ("rank", C.c_int32), ("world_size", C.c_int32), ("m_global", C.c_int64),
                 ("item_offset", C.c_int64), ("nccl_unique_id", C.c_void_p), ("thin", C.c_int32), ("reserved0", C.c_int32),
-                ("f_mean_out", C.POINTER(C.c_double)), ("f_sd_out", C.POINTER(C.c_double))]
+                ("f_mean_out", C.POINTER(C.c_double)), ("f_sd_out", C.POINTER(C.c_double)), ("fit", C.POINTER(Fit))]
 
 
 PROGRESS_CB = C.CFUNCTYPE(C.c_int, C.c_double, C.c_void_p)
@@ -94,6 +104,7 @@ def load():
     _ip64 = C.POINTER(C.c_int64)
     L.gpirt_b200_response_matrix.argtypes = [_dp, C.c_int64, C.c_int64, _dp, C.c_int, _dp, C.c_int, _dp, C.c_int, _dp, _ip64, _ip64, _ip64]
     L.gpirt_b200_theta_diagnostics.argtypes = [_dp, C.c_int64, C.c_int64, C.c_int, _dp, _dp]
+    L.gpirt_b200_predictive_accumulate_time.argtypes = [C.c_int64, C.c_int64, C.c_int, _dp, _dp]
     L.gpirt_b200_rng_probe.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, _dp, _dp]
     _lib = L
     return L

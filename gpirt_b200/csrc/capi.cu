@@ -329,6 +329,47 @@ int gpirt_b200_int8_peak_tops_random(double* tops) {
     return int8_peak_tops(tops, 1);
 }
 
+int gpirt_b200_predictive_accumulate_time(int64_t n, int64_t m, int reps, double* ms_accumulate, double* ms_copy) {
+    if (n <= 0 || m <= 0 || n > INT_MAX || m > INT_MAX || reps <= 0 || !ms_accumulate || !ms_copy) return GPIRT_B200_ERR_ARG;
+    GP_TRY(have_device());
+    const int64_t ld = round_up(n, 8), ldc = round_up(n, 16);
+    const size_t acc_doubles = 3 * (size_t)ld * m;
+    DevBuf f, acc, copy, theta, beta, code;
+    GP_TRY(f.alloc((size_t)ld * m)); GP_TRY(acc.alloc(acc_doubles)); GP_TRY(copy.alloc(acc_doubles));
+    GP_TRY(theta.alloc((size_t)ld)); GP_TRY(beta.alloc(2 * (size_t)m)); GP_TRY(code.alloc((size_t)ldc * m / 8 + 1));
+    // a sampler-like state: f, theta, beta standard normal, every cell observed (+1)
+    const RngKey key{12345u, 678u, 1u, nullptr};
+    GP_TRY(launch_fill_normal(0, f.p, (int)n, (int)m, ld, key, 0, 0));
+    GP_TRY(launch_fill_normal(0, theta.p, (int)n, 1, ld, key, 1, 0));
+    GP_TRY(launch_fill_normal(0, beta.p, 2, (int)m, 2, key, 2, 0));
+    int8_t* c8 = reinterpret_cast<int8_t*>(code.p);
+    GP_CUDA(cudaMemset(c8, 1, (size_t)ldc * m));
+    GP_TRY(launch_predictive_accumulate(0, f.p, ld, c8, ldc, theta.p, beta.p, (int)n, (int)m, 1.0, acc.p));   // count 1 initialises
+    GP_CUDA(cudaMemcpyAsync(copy.p, acc.p, acc_doubles * sizeof(double), cudaMemcpyDeviceToDevice, 0));
+    cudaEvent_t e[3];
+    for (auto& x : e) GP_CUDA(cudaEventCreate(&x));
+    int rc = GPIRT_B200_OK;
+    cudaEventRecord(e[0], 0);
+    for (int r = 0; r < reps && rc == GPIRT_B200_OK; ++r)
+        rc = launch_predictive_accumulate(0, f.p, ld, c8, ldc, theta.p, beta.p, (int)n, (int)m, 2.0 + r, acc.p);
+    cudaEventRecord(e[1], 0);
+    for (int r = 0; r < reps && rc == GPIRT_B200_OK; ++r)   // the same bytes read and written as the accumulator planes
+        if (cudaMemcpyAsync(r & 1 ? acc.p : copy.p, r & 1 ? copy.p : acc.p, acc_doubles * sizeof(double), cudaMemcpyDeviceToDevice, 0) != cudaSuccess)
+            rc = GPIRT_B200_ERR_CUDA;
+    cudaEventRecord(e[2], 0);
+    float t_acc = 0.f, t_copy = 0.f;
+    if (rc == GPIRT_B200_OK && cudaEventSynchronize(e[2]) != cudaSuccess) {
+        set_last_error("predictive accumulation timing failed: %s", cudaGetErrorString(cudaGetLastError()));
+        rc = GPIRT_B200_ERR_CUDA;
+    }
+    if (rc == GPIRT_B200_OK) { cudaEventElapsedTime(&t_acc, e[0], e[1]); cudaEventElapsedTime(&t_copy, e[1], e[2]); }
+    for (auto& x : e) cudaEventDestroy(x);
+    if (rc) return rc;
+    *ms_accumulate = t_acc / reps;
+    *ms_copy = t_copy / reps;
+    return GPIRT_B200_OK;
+}
+
 int gpirt_b200_rng_probe(uint64_t seed, uint32_t sweep, uint32_t purpose, uint32_t stream, uint32_t idx0, int count,
                          double* uniforms, double* normals) {
     if (count < 0 || !uniforms || !normals) return GPIRT_B200_ERR_ARG;

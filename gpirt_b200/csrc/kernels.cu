@@ -407,6 +407,9 @@ static int persistent_grid(K kernel, int threads, size_t smem, int m, int* grid)
         return std::tie(k, threads, smem, dev) < std::tie(o.k, o.threads, o.smem, o.dev); } };
     static std::mutex mu;
     static std::map<Key, int> cache;
+    // the shared-memory limit is an attribute of the kernel, not of a launch shape: it only ever grows, so that a smaller
+    // shape prepared later (another n) cannot take it below what a shape already in the cache launches with
+    static std::map<std::pair<const void*, int>, size_t> smem_limit;
     int dev = 0;
     GP_CUDA(cudaGetDevice(&dev));
     const Key key{(const void*)kernel, threads, smem, dev};
@@ -415,7 +418,11 @@ static int persistent_grid(K kernel, int threads, size_t smem, int m, int* grid)
     if (it == cache.end()) {
         int sms = 0, per_sm = 0;
         GP_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-        GP_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        size_t& limit = smem_limit[{(const void*)kernel, dev}];
+        if (smem > limit) {
+            GP_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+            limit = smem;
+        }
         GP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, threads, smem));
         if (per_sm < 1) { set_last_error("per-item kernel does not fit on an SM"); return GPIRT_B200_ERR_CUDA; }
         it = cache.emplace(key, sms * per_sm).first;
@@ -934,6 +941,189 @@ int launch_gather_columns(cudaStream_t st, const double* y, int n, const int64_t
     if (n <= 0 || m_kept <= 0) return GPIRT_B200_OK;
     dim3 grid((unsigned)m_kept, (unsigned)ceil_div(n, 256));
     GP_LAUNCH(k_gather_columns, grid, 256, 0, st, y, n, kept, out);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// Posterior predictive summaries (opts.fit).  Per cell and sampling iteration, with g = f + beta0 + beta1 theta and the
+// scoring orientation yt (y where observed, the held-out value where given, +1 otherwise):
+//   acc[0] += sigma(yt g)      acc[1], acc[2] = Welford mean / M2 of l = log sigma(yt g)
+// Orienting the sum by yt keeps log(mean sigma) accurate in badly predicted cells (tiny mean likelihood); pred for a
+// yt = -1 cell is then 1 - mean sigma(-g), accurate in absolute terms.  HBM-bound: 57 bytes per cell and iteration.
+// ------------------------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k_predictive_code(const int8_t* __restrict__ y8, int64_t ldy8,
+                                                         const double* __restrict__ y_holdout, int n,
+                                                         int8_t* __restrict__ code, unsigned long long* n_bad) {
+    const int i = blockIdx.y * blockDim.x + threadIdx.x, j = blockIdx.x;
+    if (i >= n) return;
+    int8_t c = y8[i + (int64_t)j * ldy8];
+    if (c == 0 && y_holdout) {                                   // held-out values are read where y is NA only
+        const double v = y_holdout[i + (int64_t)j * n];
+        if (v == 1.0) c = PRED_HOLDOUT;
+        else if (v == -1.0) c = -PRED_HOLDOUT;
+        else if (!isnan(v)) atomicAdd(n_bad, 1ull);
+    }
+    code[i + (int64_t)j * ldy8] = c;
+}
+int launch_predictive_code(cudaStream_t st, const int8_t* y8, int64_t ldy8, const double* y_holdout, int n, int m,
+                           int8_t* code, unsigned long long* n_bad) {
+    dim3 grid((unsigned)m, (unsigned)ceil_div(n, 256));
+    GP_LAUNCH(k_predictive_code, grid, 256, 0, st, y8, ldy8, y_holdout, n, code, n_bad);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+
+// sigma(a) and log sigma(a) from one exp and one log1p, both stable for either sign of a
+__device__ __forceinline__ void log_sigmoid(double a, double& sig, double& ls) {
+    const double e = exp(-fabs(a));
+    sig = (a >= 0.0 ? 1.0 : e) / (1.0 + e);
+    ls = -(fmax(-a, 0.0) + log1p(e));
+}
+__device__ __forceinline__ void predictive_update(double g, int8_t c, double count, double& s, double& mu, double& q) {
+    double sig, ls;
+    log_sigmoid(c < 0 ? -g : g, sig, ls);
+    if (count == 1.0) { s = sig; mu = ls; q = 0.0; return; }   // first sampling iteration: no memset of the accumulators
+    s += sig;
+    const double d = ls - mu;
+    mu += d / count;
+    q = fma(d, ls - mu, q);
+}
+// one thread = two consecutive respondents of one item (16-byte loads and stores; ld even, code pitch a multiple of 16)
+__global__ void __launch_bounds__(256) k_predictive_accumulate(const double* __restrict__ f, int64_t ld,
+                                                               const int8_t* __restrict__ code, int64_t ldc,
+                                                               const double* __restrict__ theta,
+                                                               const double* __restrict__ beta, int n, double count,
+                                                               double* __restrict__ acc, size_t plane) {
+    const int i0 = 2 * (blockIdx.y * blockDim.x + threadIdx.x), j = blockIdx.x;
+    if (i0 >= n) return;
+    const double b0 = __ldg(beta + 2 * j), b1 = __ldg(beta + 2 * j + 1);
+    const int64_t o = i0 + (int64_t)j * ld;
+    double* s = acc + o;
+    double* mu = acc + plane + o;
+    double* q = acc + 2 * plane + o;
+    if (i0 + 1 < n) {
+        const double2 fv = *reinterpret_cast<const double2*>(f + o);
+        const double2 th = __ldg(reinterpret_cast<const double2*>(theta + i0));
+        const char2 cv = *reinterpret_cast<const char2*>(code + i0 + (int64_t)j * ldc);
+        double2 sv = make_double2(0.0, 0.0), mv = sv, qv = sv;
+        if (count != 1.0) {
+            sv = *reinterpret_cast<const double2*>(s);
+            mv = *reinterpret_cast<const double2*>(mu);
+            qv = *reinterpret_cast<const double2*>(q);
+        }
+        predictive_update(fv.x + fma(th.x, b1, b0), cv.x, count, sv.x, mv.x, qv.x);
+        predictive_update(fv.y + fma(th.y, b1, b0), cv.y, count, sv.y, mv.y, qv.y);
+        *reinterpret_cast<double2*>(s) = sv;
+        *reinterpret_cast<double2*>(mu) = mv;
+        *reinterpret_cast<double2*>(q) = qv;
+    } else {
+        double sv = 0.0, mv = 0.0, qv = 0.0;
+        if (count != 1.0) { sv = *s; mv = *mu; qv = *q; }
+        predictive_update(f[o] + fma(theta[i0], b1, b0), code[i0 + (int64_t)j * ldc], count, sv, mv, qv);
+        *s = sv; *mu = mv; *q = qv;
+    }
+}
+int launch_predictive_accumulate(cudaStream_t st, const double* f, int64_t ld, const int8_t* code, int64_t ldc,
+                                 const double* theta, const double* beta, int n, int m, double count, double* acc) {
+    if (ld % 2) { set_last_error("predictive accumulation: leading dimension must be even"); return GPIRT_B200_ERR_ARG; }
+    dim3 grid((unsigned)m, (unsigned)ceil_div(ceil_div(n, 2), 256));
+    GP_LAUNCH(k_predictive_accumulate, grid, 256, 0, st, f, ld, code, ldc, theta, beta, n, count, acc, (size_t)ld * m);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+
+// the per-cell outputs of one finished cell: lpd = log(mean sigma(yt g)), pwaic = var_s(l) with denominator S - 1
+__device__ __forceinline__ void predictive_cell(const double* acc, size_t plane, int64_t o, double S, double& lpd, double& pw) {
+    lpd = log(acc[o] / S);
+    pw = acc[2 * plane + o] / (S - 1.0);   // S = 1: 0 / 0 = NaN
+}
+__global__ void __launch_bounds__(256) k_predictive_cells(const double* __restrict__ acc, int64_t ld, size_t plane,
+                                                          const int8_t* __restrict__ code, int64_t ldc, int n, double S,
+                                                          int which, double* __restrict__ out) {
+    const int i = blockIdx.y * blockDim.x + threadIdx.x, j = blockIdx.x;
+    if (i >= n) return;
+    const int64_t o = i + (int64_t)j * ld;
+    const int c = code[i + (int64_t)j * ldc];
+    double lpd, pw, v;
+    predictive_cell(acc, plane, o, S, lpd, pw);
+    if (which == PRED_OUT_PRED) {
+        const double p = acc[o] / S;
+        v = c < 0 ? 1.0 - p : p;
+    } else if (which == PRED_OUT_LPD) {
+        v = c != 0 ? lpd : nan("");
+    } else {
+        v = (c == 1 || c == -1) ? pw : nan("");
+    }
+    out[i + (int64_t)j * n] = v;
+}
+int launch_predictive_cells(cudaStream_t st, const double* acc, int64_t ld, const int8_t* code, int64_t ldc, int n, int m,
+                            double S, int which, double* out) {
+    dim3 grid((unsigned)m, (unsigned)ceil_div(n, 256));
+    GP_LAUNCH(k_predictive_cells, grid, 256, 0, st, acc, ld, (size_t)ld * m, code, ldc, n, S, which, out);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+
+// per item, one CTA, fixed order: stats[k * m + j] for k = lppd, p_waic, elpd, elpd^2, lpd_holdout, n_obs, n_holdout
+__global__ void __launch_bounds__(256) k_predictive_items(const double* __restrict__ acc, int64_t ld, size_t plane,
+                                                          const int8_t* __restrict__ code, int64_t ldc, int n, int m,
+                                                          double S, double* __restrict__ stats) {
+    __shared__ double red[2][32];
+    const int j = blockIdx.x;
+    double v[PRED_STATS] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+    for (int i = threadIdx.x; i < n; i += blockDim.x) {
+        const int c = code[i + (int64_t)j * ldc];
+        if (c == 0) continue;
+        double lpd, pw;
+        predictive_cell(acc, plane, i + (int64_t)j * ld, S, lpd, pw);
+        if (c == 1 || c == -1) {
+            const double e = lpd - pw;
+            v[0] += lpd; v[1] += pw; v[2] += e; v[3] += e * e; v[5] += 1.0;
+        } else {
+            v[4] += lpd; v[6] += 1.0;
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < PRED_STATS; ++k) {
+        const double t = block_sum(v[k], red[k & 1]);
+        if (threadIdx.x == 0) stats[(int64_t)k * m + j] = t;
+    }
+}
+// per respondent: partial[c * n + i] = sum of the elpd of the observed cells of item chunk c (then k_reduce_partials)
+__global__ void __launch_bounds__(128) k_predictive_resp(const double* __restrict__ acc, int64_t ld, size_t plane,
+                                                         const int8_t* __restrict__ code, int64_t ldc, int n, int m,
+                                                         double S, double* __restrict__ partial, int n_chunks) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x, chunk = blockIdx.y;
+    if (i >= n) return;
+    const int per = (int)ceil_div(m, n_chunks), j0 = chunk * per, j1 = min(m, j0 + per);
+    double t = 0.0;
+    for (int j = j0; j < j1; ++j) {
+        const int c = code[i + (int64_t)j * ldc];
+        if (c != 1 && c != -1) continue;
+        double lpd, pw;
+        predictive_cell(acc, plane, i + (int64_t)j * ld, S, lpd, pw);
+        t += lpd - pw;
+    }
+    partial[(int64_t)chunk * n + i] = t;
+}
+// totals[k] = sum over items of stats[k * m + j], one CTA per statistic, fixed order
+__global__ void __launch_bounds__(256) k_predictive_totals(const double* __restrict__ stats, int m, double* __restrict__ totals) {
+    __shared__ double red[32];
+    const int k = blockIdx.x;
+    double t = 0.0;
+    for (int j = threadIdx.x; j < m; j += blockDim.x) t += stats[(int64_t)k * m + j];
+    t = block_sum(t, red);
+    if (threadIdx.x == 0) totals[k] = t;
+}
+int launch_predictive_reduce(cudaStream_t st, const double* acc, int64_t ld, const int8_t* code, int64_t ldc, int n, int m,
+                             double S, double* stats, double* partial, int n_chunks, double* resp_totals) {
+    const size_t plane = (size_t)ld * m;
+    GP_LAUNCH(k_predictive_items, (unsigned)m, 256, 0, st, acc, ld, plane, code, ldc, n, m, S, stats);
+    dim3 grid((unsigned)ceil_div(n, 128), (unsigned)n_chunks);
+    GP_LAUNCH(k_predictive_resp, grid, 128, 0, st, acc, ld, plane, code, ldc, n, m, S, partial, n_chunks);
+    GP_LAUNCH(k_reduce_partials, (unsigned)ceil_div(n, 128), 128, 0, st, partial, n, n_chunks, resp_totals);
+    GP_LAUNCH(k_predictive_totals, (unsigned)PRED_STATS, 256, 0, st, stats, m, resp_totals + n);
     GP_CUDA(cudaGetLastError());
     return GPIRT_B200_OK;
 }

@@ -58,5 +58,25 @@ int launch_gather_columns(cudaStream_t st, const double* y, int n, const int64_t
 int launch_rng_probe(cudaStream_t st, RngKey key, uint32_t purpose, uint32_t stream, uint32_t idx0, int count,
                      double* uniforms, double* normals);
 
+// ---- posterior predictive summaries (opts.fit) ----
+// cell code (int8, pitch ldy8): +-1 observed y, +-PRED_HOLDOUT held-out value, 0 neither (scored as +1); sign = orientation
+constexpr int8_t PRED_HOLDOUT = 2;
+enum PredOut : int { PRED_OUT_PRED = 0, PRED_OUT_LPD = 1, PRED_OUT_PWAIC = 2 };
+// per-item statistics / totals: lppd, p_waic, elpd, elpd^2, lpd_holdout, n_obs, n_holdout (sums over the item's cells)
+constexpr int PRED_STATS = 7;
+// code from y8 and the optional held-out values (n x m, NaN = none; read where y is NA); counts values not in {+1,-1,NaN}
+int launch_predictive_code(cudaStream_t st, const int8_t* y8, int64_t ldy8, const double* y_holdout, int n, int m,
+                           int8_t* code, unsigned long long* n_bad);
+// one sampling iteration (count = 1, 2, ...) into acc = 3 planes of ld x m: sum sigma, Welford mean / M2 of log sigma
+int launch_predictive_accumulate(cudaStream_t st, const double* f, int64_t ld, const int8_t* code, int64_t ldc,
+                                 const double* theta, const double* beta, int n, int m, double count, double* acc);
+// one per-cell output (PredOut) of S accumulated iterations -> out, n x m tightly packed
+int launch_predictive_cells(cudaStream_t st, const double* acc, int64_t ld, const int8_t* code, int64_t ldc, int n, int m,
+                            double S, int which, double* out);
+// stats (PRED_STATS x m, per item), resp_totals = elpd per respondent (n) then the PRED_STATS totals; partial: n_chunks x n
+// scratch.  Every sum runs in a fixed order (bit-identical run to run, no floating-point atomics).
+int launch_predictive_reduce(cudaStream_t st, const double* acc, int64_t ld, const int8_t* code, int64_t ldc, int n, int m,
+                             double S, double* stats, double* partial, int n_chunks, double* resp_totals);
+
 
 }  // namespace gpirt

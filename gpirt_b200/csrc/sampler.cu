@@ -1559,6 +1559,7 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
     double* f_mean_out = opts ? opts->f_mean_out : nullptr;
     double* f_sd_out = opts ? opts->f_sd_out : nullptr;
     const bool summarise_f = f_mean_out || f_sd_out;
+    gpirt_b200_fit* const fit = opts ? opts->fit : nullptr;
     const bool trace = getenv("GPIRT_TIMING") != nullptr;
     auto now = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; };
     g_last_degenerate_theta = 0;
@@ -1585,6 +1586,7 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         double *f_mean, *f_m2, *agree_dev; int* h_poll; StoreWorker* worker;
         double* h_small[2]; cudaEvent_t ev_small[2];
         bool trace = false;
+        double* pred_acc = nullptr; int8_t* pred_code = nullptr; double* pred_aux = nullptr;   // opts.fit
         ~Guard() {
             auto now = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; };
             const double t0 = now();
@@ -1594,6 +1596,7 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
             for (int i = 0; i < 2; ++i) if (ev_small[i]) cudaEventDestroy(ev_small[i]);   // h_small / h_poll belong to g_bounce
             for (int i = 0; i < 2; ++i) { if (ev[i]) cudaEventDestroy(ev[i]); pool_free(snap_f[i], s->stream); pool_free(snap_small[i], s->stream); }
             pool_free(f_mean, s->stream); pool_free(f_m2, s->stream); pool_free(agree_dev, s->stream);
+            pool_free(pred_acc, s->stream); pool_free(pred_code, s->stream); pool_free(pred_aux, s->stream);
             const double t2 = now();
             gpirt_b200_sampler_destroy(s);
             if (trace) fprintf(stderr, "gpirt_b200_mcmc: teardown worker/copy stream %.3fs, host + pool frees %.3fs, sampler %.3fs\n", t1 - t0, t2 - t1, now() - t2);
@@ -1635,6 +1638,40 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
     }
     const bool sharded = s->comm.world > 1;
     if (sharded) GP_TRY(pool_alloc((void**)&gd.agree_dev, sizeof(double), s->stream));
+    // posterior predictive summaries: 3 accumulator planes (ldn x m), the cell code, per-item statistics, the per-respondent
+    // partial sums, elpd per respondent + totals, and the illegal-value counter of y_holdout
+    constexpr int PRED_CHUNKS = 64;
+    const size_t pred_plane = (size_t)s->ldn * m;
+    double *pred_stats = nullptr, *pred_partial = nullptr, *pred_resp = nullptr;
+    if (fit) {
+        GP_TRY(pool_alloc((void**)&gd.pred_acc, 3 * pred_plane * sizeof(double), s->stream));
+        GP_TRY(pool_alloc((void**)&gd.pred_code, (size_t)s->ldy8 * m, s->stream));
+        const size_t aux = (size_t)PRED_STATS * m + (size_t)PRED_CHUNKS * n + (size_t)n + PRED_STATS + 1;
+        GP_TRY(pool_alloc((void**)&gd.pred_aux, aux * sizeof(double), s->stream));
+        pred_stats = gd.pred_aux;
+        pred_partial = pred_stats + (size_t)PRED_STATS * m;
+        pred_resp = pred_partial + (size_t)PRED_CHUNKS * n;
+        unsigned long long* n_bad = reinterpret_cast<unsigned long long*>(pred_resp + n + PRED_STATS);
+        GP_CUDA(cudaMemsetAsync(n_bad, 0, sizeof(unsigned long long), s->stream));
+        // y_holdout goes up through the first accumulator plane (not in use before the first sampling iteration)
+        if (fit->y_holdout) GP_TRY(upload_pageable(gd.pred_acc, fit->y_holdout, nm * sizeof(double), s->stream));
+        GP_TRY(launch_predictive_code(s->stream, s->y8, s->ldy8, fit->y_holdout ? gd.pred_acc : nullptr, (int)n, (int)m,
+                                      gd.pred_code, n_bad));
+        unsigned long long bad = 0;
+        GP_CUDA(cudaMemcpyAsync(&bad, n_bad, sizeof(bad), cudaMemcpyDeviceToHost, s->stream));
+        GP_CUDA(cudaStreamSynchronize(s->stream));
+        double bad_all = (double)bad;
+        if (sharded) {   // every rank refuses together: one that returned alone would leave its peers in the first collective
+            GP_CUDA(cudaMemcpyAsync(gd.agree_dev, &bad_all, sizeof(double), cudaMemcpyHostToDevice, s->stream));
+            GP_TRY(comm_allreduce_sum_f64(s->comm, gd.agree_dev, 1, s->stream));
+            GP_CUDA(cudaMemcpyAsync(&bad_all, gd.agree_dev, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+            GP_CUDA(cudaStreamSynchronize(s->stream));
+        }
+        if (bad_all != 0.0) {
+            set_last_error("y_holdout holds %.0f values that are not +1, -1 or NA", bad_all);
+            return GPIRT_B200_ERR_Y_VALUE;
+        }
+    }
     double t_c = now();
     GP_TRY(s->init_draws());
     double t_d = now();
@@ -1744,6 +1781,9 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
             dim3 grid((unsigned)m, (unsigned)ceil_div(n, 256));
             GP_LAUNCH(k_f_welford, grid, 256, 0, s->stream, s->f, s->ldn, (int)n, (double)(++n_summarised), gd.f_mean, gd.f_m2);
         }
+        if (sampling && fit)
+            GP_TRY(launch_predictive_accumulate(s->stream, s->f, s->ldn, gd.pred_code, s->ldy8, s->theta, s->beta, (int)n, (int)m,
+                                                (double)si, gd.pred_acc));
         if (store) {
             const int slot = si / thin;                                             // :99-103
             worker.wait_buffer_free(slot & 1);                                      // slot - 2 has left this snapshot buffer
@@ -1788,6 +1828,38 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         GP_CUDA(cudaStreamSynchronize(s->stream));
         if (f_mean_out) GP_TRY(chunked_d2h(f_mean_out, gd.f_mean, nm, 0, gd.copy));
         if (f_sd_out) GP_TRY(chunked_d2h(f_sd_out, gd.f_m2, nm, 1, gd.copy));
+    }
+    if (fit) {
+        const double S = (double)sample_iterations;
+        if (sample_iterations == 0) {   // NaN accumulators: every output NaN, the cell counts still hold
+            GP_CUDA(cudaMemsetAsync(gd.pred_acc, 0xff, pred_plane * sizeof(double), s->stream));
+            GP_CUDA(cudaMemsetAsync(gd.pred_acc + 2 * pred_plane, 0xff, pred_plane * sizeof(double), s->stream));
+        }
+        GP_TRY(launch_predictive_reduce(s->stream, gd.pred_acc, s->ldn, gd.pred_code, s->ldy8, (int)n, (int)m, S, pred_stats,
+                                        pred_partial, PRED_CHUNKS, pred_resp));
+        if (sharded) GP_TRY(comm_allreduce_sum_f64(s->comm, pred_resp, (size_t)n + PRED_STATS, s->stream));
+        double tot[PRED_STATS];
+        GP_CUDA(cudaMemcpyAsync(tot, pred_resp + n, sizeof(tot), cudaMemcpyDeviceToHost, s->stream));
+        if (fit->elpd_resp) GP_CUDA(cudaMemcpyAsync(fit->elpd_resp, pred_resp, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+        if (fit->elpd_item) GP_CUDA(cudaMemcpyAsync(fit->elpd_item, pred_stats + 2 * (size_t)m, (size_t)m * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+        // per-cell outputs one at a time, tightly packed into the (now free) running-mean plane
+        double* const outs[3] = {fit->pred, fit->lpd_cell, fit->pwaic_cell};
+        for (int w = 0; w < 3; ++w) {
+            if (!outs[w]) continue;
+            GP_TRY(launch_predictive_cells(s->stream, gd.pred_acc, s->ldn, gd.pred_code, s->ldy8, (int)n, (int)m, S, w, gd.pred_acc + pred_plane));
+            GP_CUDA(cudaStreamSynchronize(s->stream));
+            GP_TRY(chunked_d2h(outs[w], gd.pred_acc + pred_plane, nm, 0, gd.copy));
+        }
+        GP_CUDA(cudaStreamSynchronize(s->stream));
+        const double N = tot[5], sum_e = tot[2], var = (tot[3] - sum_e * sum_e / N) / (N - 1.0);
+        fit->lppd = tot[0];
+        fit->p_waic = tot[1];
+        fit->elpd_waic = tot[0] - tot[1];
+        fit->waic = -2.0 * fit->elpd_waic;
+        fit->se_elpd_waic = std::sqrt(N * (var < 0.0 ? 0.0 : var));   // loo's convention; NaN stays NaN
+        fit->lpd_holdout = sample_iterations ? tot[4] : NAN;   // S = 0: NaN even where no cell is held out
+        fit->n_obs = (int64_t)tot[5];
+        fit->n_holdout = (int64_t)tot[6];
     }
     GP_CUDA(cudaStreamSynchronize(s->stream));
     if (cb) cb(100.0, cb_ctx);

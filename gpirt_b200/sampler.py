@@ -10,7 +10,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import GpirtError, Opts, N_GRID
+from ._lib import Fit, GpirtError, Opts, N_GRID
 from .response_matrix import DEFAULT_CODES, as_response_matrix
 
 
@@ -47,13 +47,18 @@ def nccl_unique_id():
 
 def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_prior_means=None, beta_prior_sds=None,
               beta_proposal_sds=None, theta_init=None, *, seed=None, progress=None, store_f=True, fstar_mode=0,
-              device=-1, shard=None, thin=1, f_summary=False, use_graph=0):
+              device=-1, shard=None, thin=1, f_summary=False, use_graph=0, predictive=False, y_holdout=None):
     """Drop-in for the reference's gpirtMCMC().  Keyword-only extras (not in the reference): seed (Philox key; default
     drawn from numpy's global RNG, as the R shim draws it from R's), progress(percent) -> truthy to interrupt,
     store_f=False to skip the n*m*(S+1) f draws, shard=(rank, world, m_global, item_offset, unique_id) for item
     sharding across GPUs, thin=k to keep every k-th sampling iteration only (outputs then hold 1 + S // k slots; IRFs
     still average over all S), f_summary=True to also return the posterior mean / sd of f over all sampling iterations
-    (accumulated on the device: "f_mean", "f_sd", n x m)."""
+    (accumulated on the device: "f_mean", "f_sd", n x m), predictive=True to also return posterior predictive
+    probabilities, WAIC and held-out scores over all sampling iterations ("predictive": dict with pred, lpd_cell, pwaic_cell
+    (n x m), elpd_item (m), elpd_resp (n) and the scalars lppd, p_waic, elpd_waic, waic, se_elpd_waic, lpd_holdout, n_obs,
+    n_holdout; accumulated on the device, definitions in include/gpirt_b200.h), y_holdout = n x m array of the coded
+    response matrix's shape holding +1 / -1 where a missing response was held out (NaN elsewhere; read where y is NA).
+    With shard, per-cell and per-item outputs cover the local items, elpd_resp and the scalars all items."""
     L = _lib.load()
     y = as_response_matrix(data, vote_codes or DEFAULT_CODES)                        # R/gpirtMCMC.R:93
     y = np.asfortranarray(np.asarray(y, dtype=np.float64))
@@ -82,6 +87,21 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
     f = np.empty((n, m, slots), order="F") if store_f else None
     irf = np.empty((N_GRID, m), order="F")
     f_mean = f_sd = None
+    fit = None
+    if y_holdout is not None and not predictive:
+        raise ValueError("y_holdout is only read with predictive=True")
+    if predictive:
+        fit = Fit()
+        if y_holdout is not None:
+            y_holdout = _F(y_holdout)
+            if y_holdout.shape != (n, m):
+                raise ValueError("y_holdout must have the shape of the coded response matrix %r, got %r" % ((n, m), y_holdout.shape))
+            fit.y_holdout = _lib.ptr(y_holdout)
+        pred = dict(pred=np.empty((n, m), order="F"), lpd_cell=np.empty((n, m), order="F"),
+                    pwaic_cell=np.empty((n, m), order="F"), elpd_item=np.empty(m), elpd_resp=np.empty(n))
+        for k, a in pred.items():
+            setattr(fit, k, _lib.ptr(a))
+        opts.fit = C.pointer(fit)
     if f_summary:
         f_mean = np.empty((n, m), order="F"); f_sd = np.empty((n, m), order="F")
         opts.f_mean_out = _lib.ptr(f_mean); opts.f_sd_out = _lib.ptr(f_sd)
@@ -100,6 +120,10 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
         out["f"] = f
     if f_summary:
         out["f_mean"], out["f_sd"] = f_mean, f_sd
+    if predictive:
+        for k in ("lppd", "p_waic", "elpd_waic", "waic", "se_elpd_waic", "lpd_holdout", "n_obs", "n_holdout"):
+            pred[k] = getattr(fit, k)
+        out["predictive"] = pred
     return out
 
 
@@ -282,6 +306,14 @@ def int8_peak_tops(random_operands=False):
     L = _lib.load()
     _lib.check((L.gpirt_b200_int8_peak_tops_random if random_operands else L.gpirt_b200_int8_peak_tops)(C.byref(a)))
     return a.value
+
+
+def predictive_accumulate_time(n, m, reps=100):
+    """(ms per launch of the posterior predictive accumulation over an n x m state, ms per device-to-device copy of its
+    accumulator planes), CUDA events in one run"""
+    a = C.c_double(0); b = C.c_double(0)
+    _lib.check(_lib.load().gpirt_b200_predictive_accumulate_time(int(n), int(m), int(reps), C.byref(a), C.byref(b)))
+    return a.value, b.value
 
 
 def rng_probe(seed, sweep, purpose, stream, idx0, count):

@@ -32,6 +32,31 @@ enum gpirt_b200_status {
     GPIRT_B200_ERR_NOMEM = -8
 };
 
+/* Posterior predictive summaries accumulated on the device over all S sampling iterations (burn-in excluded, thin has no
+ * effect), each iteration's end-of-sweep state (f, theta, beta).  Per cell g = f_ij + beta0_j + beta1_j theta_i; the
+ * scoring orientation yt_ij is y_ij where observed, y_holdout_ij where y is NA and y_holdout gives +1 / -1, else +1.
+ * Zero-initialise, set the pointers you want; the library fills the scalars.  With items sharded, per-cell and per-item
+ * outputs cover the local item block, elpd_resp and every scalar are global (all-reduced); every rank must set fit.
+ * S = 0: every output is NaN.  S = 1: pwaic_cell, p_waic, elpd_*, waic and se_elpd_waic are NaN. */
+typedef struct gpirt_b200_fit {
+    const double* y_holdout; /* optional n x m {+1, -1, NaN}: held-out responses, read only where y is NA
+                                (any other value: GPIRT_B200_ERR_Y_VALUE) */
+    double* pred;         /* optional n x m: mean_s sigma(g), the posterior predictive P(y_ij = +1), every cell */
+    double* lpd_cell;     /* optional n x m: log(mean_s sigma(yt g)) on observed and held-out cells, NaN elsewhere */
+    double* pwaic_cell;   /* optional n x m: sample variance (denominator S - 1) over s of log sigma(yt g), observed cells
+                             only, NaN elsewhere */
+    double* elpd_item;    /* optional m: sum of lpd_cell - pwaic_cell over the observed cells of the item */
+    double* elpd_resp;    /* optional n: the same sum over the observed cells of the respondent */
+    double lppd;          /* out: sum of lpd_cell over the observed cells */
+    double p_waic;        /* out: sum of pwaic_cell over the observed cells */
+    double elpd_waic;     /* out: lppd - p_waic */
+    double waic;          /* out: -2 elpd_waic */
+    double se_elpd_waic;  /* out: sqrt(n_obs var(lpd_cell - pwaic_cell)) over the observed cells (sample variance) */
+    double lpd_holdout;   /* out: sum of lpd_cell over the held-out cells */
+    int64_t n_obs;        /* out: number of observed cells */
+    int64_t n_holdout;    /* out: number of held-out cells */
+} gpirt_b200_fit;
+
 /* Options beyond the reference's seven arguments.  Zero-initialise, then set what you need. */
 typedef struct gpirt_b200_opts {
     uint64_t seed;        /* Philox4x32-10 key; the R shim derives it from R's RNG so set.seed() reproduces runs */
@@ -56,6 +81,8 @@ typedef struct gpirt_b200_opts {
     int32_t reserved0;
     double* f_mean_out;   /* optional n x m: posterior mean of f over all sampling iterations, accumulated on the device */
     double* f_sd_out;     /* optional n x m: posterior standard deviation of f (denominator S - 1, as R's sd()) */
+    gpirt_b200_fit* fit;  /* optional: posterior predictive probabilities, WAIC and held-out scores (gpirt_b200_fit);
+                             NULL = none.  Costs 25 bytes of device memory per cell for the run */
 } gpirt_b200_opts;
 
 /* Progress / interrupt callback: called once per iteration with percent complete (as the reference's Rprintf,
@@ -181,6 +208,11 @@ int gpirt_b200_int8_peak_tops(double* tops);
  * (tools/umma_i8_shapes.cu), but the switching power pulls the SM clock down, so the sustained operations/s are lower —
  * the practical ceiling of a kernel that multiplies real operand planes */
 int gpirt_b200_int8_peak_tops_random(double* tops);
+/* measurement: mean milliseconds of one launch of the posterior predictive accumulation (opts.fit) over an n x m state
+ * (f, theta, beta standard normal, every cell observed; 57 bytes of HBM traffic per cell), CUDA events over `reps`
+ * launches, and of a device-to-device copy of its 3 accumulator planes (24 (n rounded up to 8) m bytes read and as many
+ * written) in the same run: the copy rate the accumulation is compared with */
+int gpirt_b200_predictive_accumulate_time(int64_t n, int64_t m, int reps, double* ms_accumulate, double* ms_copy);
 /* ---- the host steps either side of the sampler (SURVEY 8 f4) ---- */
 /* Response coding, the producer of y (reference R/response_matrix.R:79-98) for numeric code matrices, on the device:
  * codes n x m (column-major doubles, NaN = NA); yea / nay / missing code lists; cells with a code in none of the lists are
