@@ -7,6 +7,8 @@ compared with the CPU oracle here, through the C ABI.
                     (draw-theta.cpp:12-34): each step runs on the FULL GPU state and >= 32 random items / >= 16 random
                     respondents are checked against the oracle with the same addressed variates (stream maps), with the
                     fixed-point (int8 tensor-core) products on and off, with and without 5 % missing cells
+  C5  16384 x 20000 the same steps on the full C5 state (fixed-point products on, 0 % / 5 % missing): K* solves by blocked
+                    substitution, streaming per-item kernels, the rebuilt factor checked on sampled rows
   n > 4096          the streaming launch shape of the per-item kernels (C5's shape) on small-m problems
 
 Every test asserts WHICH code path ran (gpirt_b200_sampler_uses).  Tolerances as in test_gpu_parity.py: discrete decisions
@@ -47,10 +49,10 @@ def test_c2_one_full_lockstep_sweep(G, O):
     s.close()
 
 
-def _c3_state(G, missing, monkeypatch, int8):
+def _c3_state(G, missing, monkeypatch, int8, workload="c3"):
     from gpirt_b200 import synthetic, _lib
     monkeypatch.setenv("GPIRT_GEMM_INT8", "1" if int8 else "0")
-    c = synthetic.WORKLOADS["c3"]
+    c = synthetic.WORKLOADS[workload]
     d = synthetic.make(c["n"], c["m"], missing=missing)
     s = G.Sampler(d["y"], d["theta_init"], d["pm"], d["psd"], d["pstep"], seed=synthetic.SEED)
     s.set_pipeline(False)          # steps are run one at a time below
@@ -60,12 +62,20 @@ def _c3_state(G, missing, monkeypatch, int8):
     return d, s, _lib
 
 
-@pytest.mark.parametrize("missing,int8", [(0.0, True), (0.0, False), (0.05, True), (0.05, False)])
-def test_c3_sampled_items_and_respondents_against_the_oracle(G, O, monkeypatch, missing, int8):
-    """BASELINE configs[2] (the bench workload): one step at a time on the full 4096 x 10000 state"""
+@pytest.mark.parametrize("workload,missing,int8", [
+    pytest.param("c3", 0.0, True, id="0.0-True"), pytest.param("c3", 0.0, False, id="0.0-False"),
+    pytest.param("c3", 0.05, True, id="0.05-True"), pytest.param("c3", 0.05, False, id="0.05-False"),
+    pytest.param("c5", 0.0, True, id="c5-0.0-True"), pytest.param("c5", 0.05, True, id="c5-0.05-True")])
+def test_c3_sampled_items_and_respondents_against_the_oracle(G, O, monkeypatch, workload, missing, int8):
+    """BASELINE configs[2] (the bench workload): one step at a time on the full 4096 x 10000 state.  The same at C5
+    (BASELINE configs[4], 16384 x 20000): L Z with K = 16384, the f* solves by blocked substitution (route 1), the theta
+    contraction over 20000 items for 16384 rows and the streaming item kernels."""
     from gpirt_b200 import synthetic
-    d, s, _lib = _c3_state(G, missing, monkeypatch, int8)
+    d, s, _lib = _c3_state(G, missing, monkeypatch, int8, workload)
     n, m = d["y"].shape
+    big = n > 4096                 # C5: per-item kernels in the streaming shape, K* solves by substitution
+    item_shape = ITEM_STREAM if big else ITEM_PERSISTENT
+    assert s.uses(4) == (1 if big else 0)
     seed = synthetic.SEED
     rs = np.random.RandomState(42 + int(100 * missing) + int(int8))
     J = np.sort(rs.choice(m, 32, replace=False))
@@ -79,14 +89,16 @@ def test_c3_sampled_items_and_respondents_against_the_oracle(G, O, monkeypatch, 
     f0 = s.get(_lib.F)
     sweep = 11
     s.step(_lib.STEP_DRAW_F, sweep)
-    assert s.uses(2) == ITEM_PERSISTENT
+    assert s.uses(2) == item_shape
     nu = s.get(_lib.NU); f1 = s.get(_lib.F); nprop = s.get(_lib.ESS_NPROP).astype(int)
     rng = O.Rng.keyed(seed); rng.set_sweep(sweep); rng.set_item_map(J)
     mu = O.linear_mean(theta, beta[:, J])
     fo, npo = O.draw_f(f0[:, J], yJ, L, mu, rng)
     for jj, j in enumerate(J[:4]):   # the proposal itself for a few items: nu_j = L z_j
         z = np.array([O.keyed_normal(seed, sweep, O.P_ESS_Z, int(j), i) for i in range(n)])
-        assert np.max(np.abs(nu[:, j] - L @ z)) <= 1e-11
+        # C5: the fixed-point bound K 2^-51 max|L_i| max|z| with L sliced at the fixed scale |L| < 2^L_FIXED_EXP = 2
+        tol = n * 2.0 ** -51 * 2.0 * np.abs(z).max() if big else 1e-11
+        assert np.max(np.abs(nu[:, j] - L @ z)) <= tol
     assert np.array_equal(nprop[J], npo), "ESS proposal counts must match the oracle"
     assert np.max(np.abs(f1[:, J] - fo)) <= 1e-9
 
@@ -113,19 +125,24 @@ def test_c3_sampled_items_and_respondents_against_the_oracle(G, O, monkeypatch, 
     # ---- draw_beta (draw-beta.cpp:16-38) with the NEW theta and the current f ----
     sweep = 14
     s.step(_lib.STEP_DRAW_BETA, sweep)
-    assert s.uses(3) == ITEM_PERSISTENT
+    assert s.uses(3) == item_shape
     b1 = s.get(_lib.BETA)
     rng = O.Rng.keyed(seed); rng.set_sweep(sweep); rng.set_item_map(J)
     bo, _ = O.draw_beta(beta[:, J], theta_new, yJ, f1[:, J], d["pm"][:, J], d["psd"][:, J], d["pstep"][:, J], rng)
     assert np.max(np.abs(b1[:, J] - bo)) <= 1e-12
 
-    # ---- rebuild (gpirtMCMC.cpp:76-78): the Cholesky chain kernels at n = 4096 against the definition ----
+    # ---- rebuild (gpirtMCMC.cpp:76-78): the Cholesky chain kernels against the definition ----
+    del nu, f0, f1, L
     s.step(_lib.STEP_REBUILD, 0)
     L2 = s.get(_lib.CHOL)
+    s.close()
     S = O.K(theta_new, theta_new) + 1e-3 * np.eye(n)
     assert np.array_equal(np.triu(L2, 1), np.zeros_like(L2)), "strict upper triangle must be exactly zero"
-    assert np.max(np.abs(L2 @ L2.T - S)) <= 1e-12 * 12
-    s.close()
+    if not big:
+        assert np.max(np.abs(L2 @ L2.T - S)) <= 1e-12 * 12
+    else:   # 64 sampled rows (and the first and last) against 2 n u max|S|, as test_gpu_large_n.py::_check_factor
+        R = np.unique(np.r_[0, n - 1, rs.choice(n, 64, replace=False)])
+        assert np.max(np.abs(L2[R, :] @ L2.T - S[R, :])) <= 2 * n * 2.0 ** -53 * np.abs(S).max()
 
 
 @pytest.mark.parametrize("n,m,missing", [(4097, 8, 0.0), (6000, 6, 0.1), (8192, 4, 0.0)])

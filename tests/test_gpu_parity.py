@@ -66,28 +66,32 @@ def test_dgemm(G, ta, tb, M, N, K):
 
 @pytest.mark.parametrize("ta,lower,M,N,K", [(0, 0, 1, 1, 1), (0, 0, 128, 64, 64), (1, 0, 100, 37, 50), (1, 0, 300, 200, 257),
                                              (0, 1, 257, 130, 257), (0, 1, 1000, 333, 1000), (1, 0, 1001, 500, 1100),
-                                             (0, 0, 129, 65, 4097)])
+                                             (0, 0, 129, 65, 4097), (0, 1, 16384, 70, 16384), (1, 2, 16384, 70, 16384)])
 def test_dgemm_i8_fixed_point_tensor_core_product(G, ta, lower, M, N, K):
     """op(A) B in 56-bit fixed point on the int8 tensor cores (tcgen05): the kernel behind nu = L Z (draw-f.cpp:20) and the
     f* product.  The plane products are exact integers, so the only error is the dropped digit levels:
-    |err_ij| <= K 2^-51 max|A[i,:]| max|B[:,j]|  (the tolerance stated in include/gpirt_b200.h)"""
+    |err_ij| <= K 2^-51 max|A[i,:]| max|B[:,j]|  (the tolerance stated in include/gpirt_b200.h).  lower = 1: op(A) lower
+    triangular (L Z); lower = 2: op(A) = A^T upper triangular (the L^-T product); K = 16384 is C5's n.  The reference is
+    summed in long double, its own rounding far below K 2^-51; at K = 16384 on 64 sampled rows and the first and last 32."""
     rs = np.random.RandomState(M * 11 + N * 5 + K)
-    A = rs.randn(M, K) * np.exp(2.0 * rs.randn(M, 1))          # rows of very different magnitude
+    tri = {0: lambda X: X, 1: np.tril, 2: np.triu}[lower]
+    A = tri(rs.randn(M, K) * np.exp(2.0 * rs.randn(M, 1)))     # rows of very different magnitude
     B = rs.randn(K, N) * np.exp(2.0 * rs.randn(1, N))
-    if lower:
-        A = np.tril(A)
     if M > 2:
         A[1, :] = 0.0                                            # an all-zero row
     if K > 3:
         A[0, 3] = 0.0
-    got = G.dgemm_i8(np.asfortranarray(A.T) if ta else A, B, ta=bool(ta), a_lower=bool(lower))
-    want = A @ B
-    bound = K * 2.0 ** -51 * np.abs(A).max(axis=1)[:, None] * np.abs(B).max(axis=0)[None, :]
+    rows = np.arange(M) if M <= 4096 else np.unique(np.r_[0:32, M - 32:M, rs.choice(M, 64, replace=False)])
+    got = G.dgemm_i8(np.asfortranarray(A.T) if ta else A, B, ta=bool(ta), a_lower=lower)[rows]
+    want = A[rows].astype(np.longdouble) @ B.astype(np.longdouble)
+    bound = K * 2.0 ** -51 * np.abs(A[rows]).max(axis=1)[:, None] * np.abs(B).max(axis=0)[None, :]
     assert np.all(np.abs(got - want) <= bound + 1e-300)
+    del A
     # against an FP64 product's own error scale: within a few units of K u sum|a||b| when rows are evenly scaled
-    A2 = np.tril(rs.randn(M, K)) if lower else rs.randn(M, K)
+    A2 = tri(rs.randn(M, K))
     B2 = rs.randn(K, N)
-    got2 = G.dgemm_i8(np.asfortranarray(A2.T) if ta else A2, B2, ta=bool(ta), a_lower=bool(lower))
+    got2 = G.dgemm_i8(np.asfortranarray(A2.T) if ta else A2, B2, ta=bool(ta), a_lower=lower)[rows]
+    A2 = A2[rows]
     assert np.max(np.abs(got2 - A2 @ B2)) <= 64 * 2.0 ** -53 * max(1.0, np.max(np.abs(A2) @ np.abs(B2)))
 
 
@@ -351,12 +355,13 @@ def test_chain_fixed_point_products_match_dmma_products(G, monkeypatch):
     assert np.max(np.abs(a["IRFs"] - b["IRFs"])) <= 1e-9
 
 
-@pytest.mark.parametrize("n,m", [(100, 40), (400, 150), (700, 320), (1100, 260), (2304, 260)])
+@pytest.mark.parametrize("n,m", [(100, 40), (400, 150), (700, 320), (1100, 260), (2304, 260), (6145, 260), (9000, 260)])
 def test_chain_blocked_substitution_solves_match_inverse_route(G, O, n, m, monkeypatch):
-    """GPIRT_SOLVE_MODE=1 (the default when items are sharded over GPUs): L^-1 K* and L^-T(.) by blocked substitution
-    with the 128-block inverses, forward steps trailing the Cholesky panels, instead of L^-1 + triangular products
-    (draw-fstar.cpp:19,24).  Same chain as the inverse route, and in lock-step with the oracle.  n >= 1024: the backward
-    pass runs on 512 / 1024-wide diagonal-block inverses (n = 2304: two full 1024-blocks and a ragged one)."""
+    """GPIRT_SOLVE_MODE=1 (the default when items are sharded over GPUs, and for n > 6144): L^-1 K* and L^-T(.) by blocked
+    substitution with the 128-block inverses, forward steps trailing the Cholesky panels, instead of L^-1 + triangular
+    products (draw-fstar.cpp:19,24).  Same chain as the inverse route, and in lock-step with the oracle.  n >= 1024: the
+    backward pass runs on 512 / 1024-wide diagonal-block inverses (n = 2304: two full 1024-blocks and a ragged one;
+    n = 6145: a one-row last panel; n = 9000: ragged pairs at the levels 256 and 512)."""
     from gpirt_b200 import ResponseMatrix
     prob = make_problem(n, m, seed=n + 5, missing=0.04)
     out = {}
@@ -377,14 +382,18 @@ def test_chain_blocked_substitution_solves_match_inverse_route(G, O, n, m, monke
         assert np.max(np.abs(a["IRFs"] - want["IRFs"])) <= 1e-7
 
 
-@pytest.mark.parametrize("n,m,route", [(100, 60, "0"), (640, 300, "0"), (640, 300, "1"), (1152, 260, "1")])
+@pytest.mark.parametrize("n,m,route", [(100, 60, "0"), (640, 300, "0"), (640, 300, "1"), (1152, 260, "1"),
+                                        pytest.param(9000, 300, None, id="9000-300-default")])
 def test_graph_replayed_sweeps_equal_eager_sweeps(G, n, m, route, monkeypatch):
     """With the per-step timers off every sweep after the first is ONE CUDA-graph launch — captured from the very launch
     sequence of the eager sweep, for n > 256 the pipelined one with its five streams forked and joined inside the graph
     (stream priorities carried as per-node launch attributes).  Same kernels, same addressed RNG: the state after 6 sweeps
-    must be bit-identical to 6 eager sweeps, on both K*-solve routes."""
+    must be bit-identical to 6 eager sweeps, on both K*-solve routes (route None: the default, substitution for n > 6144)."""
     from gpirt_b200 import _lib
-    monkeypatch.setenv("GPIRT_SOLVE_MODE", route)
+    if route is None:
+        monkeypatch.delenv("GPIRT_SOLVE_MODE", raising=False)
+    else:
+        monkeypatch.setenv("GPIRT_SOLVE_MODE", route)
     prob = make_problem(n, m, seed=n + 3, missing=0.03)
     state = {}
     for use_graph in (0, -1):
@@ -393,7 +402,7 @@ def test_graph_replayed_sweeps_equal_eager_sweeps(G, n, m, route, monkeypatch):
         s.init_draws()
         s.sweep(4)
         s.sweep(2, accumulate_irf=True)
-        assert s.uses(4) == int(route)
+        assert s.uses(4) == (1 if route is None else int(route))
         replays = s.uses(5)
         assert (replays >= 4) if use_graph == 0 else (replays == 0), "graph replay must be the path that ran (or not)"
         state[use_graph] = {k: s.get(f) for k, f in (("theta", _lib.THETA), ("beta", _lib.BETA), ("f", _lib.F), ("fstar", _lib.FSTAR),

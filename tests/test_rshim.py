@@ -12,13 +12,16 @@ from conftest import make_problem
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 FAKE = os.path.join(HERE, "fake_r")
-HARNESS = os.path.join(FAKE, "fake_r_harness")
 
 
-def build_harness():
+@pytest.fixture(scope="module")
+def harness(tmp_path_factory):
+    """the harness is built outside the source tree, which may be read-only"""
     from gpirt_b200 import _lib
     _lib.load()   # makes sure libgpirt_b200.so exists
-    subprocess.check_call(["make", "-s", "-C", FAKE])
+    out = str(tmp_path_factory.mktemp("fake_r") / "fake_r_harness")
+    subprocess.check_call(["make", "-s", "-C", FAKE, "OUT=" + out])
+    return out
 
 
 def write_input(path, p, S, B, rng_state):
@@ -29,35 +32,32 @@ def write_input(path, p, S, B, rng_state):
             fh.write(np.asfortranarray(a, dtype=np.float64).tobytes(order="F"))
 
 
-def test_shim_registers_the_reference_routine_with_arity_7():
+def test_shim_registers_the_reference_routine_with_arity_7(harness):
     """R_init_gpirt registers _gpirt_gpirtMCMC with 7 arguments exactly as src/RcppExports.cpp:32-40 does (dynamic symbols
     off); the only other routine is the same call with the draw-storage options as three trailing arguments"""
-    build_harness()
-    out = subprocess.run([HARNESS], capture_output=True, text=True)
+    out = subprocess.run([harness], capture_output=True, text=True)
     assert out.returncode == 0, out.stderr
     assert out.stdout.split("\n")[:2] == ["registered _gpirt_gpirtMCMC arity 7", "registered _gpirt_gpirtMCMC_b200 arity 10"]
 
 
-def test_shim_raises_r_error_without_gpu(tmp_path):
+def test_shim_raises_r_error_without_gpu(harness, tmp_path):
     from gpirt_b200 import _lib
     if _lib.load().gpirt_b200_device_count() > 0:
         pytest.skip("GPU present")
-    build_harness()
     p = make_problem(12, 5, seed=1)
     write_input(tmp_path / "in.bin", p, 2, 1, 42)
-    out = subprocess.run([HARNESS, str(tmp_path / "in.bin"), str(tmp_path / "out.bin")], capture_output=True, text=True)
+    out = subprocess.run([harness, str(tmp_path / "in.bin"), str(tmp_path / "out.bin")], capture_output=True, text=True)
     assert out.returncode == 3 and "no CUDA device" in out.stderr      # Rf_error(), i.e. an R-level stop()
 
 
 @pytest.mark.gpu
-def test_shim_call_matches_c_abi(tmp_path):
+def test_shim_call_matches_c_abi(harness, tmp_path):
     import gpirt_b200
     import gpirt_b200.sampler as G
-    build_harness()
     n, m, S, B = 60, 21, 3, 2
     p = make_problem(n, m, seed=9, missing=0.1)
     write_input(tmp_path / "in.bin", p, S, B, 20261018)
-    out = subprocess.run([HARNESS, str(tmp_path / "in.bin"), str(tmp_path / "out.bin")], capture_output=True, text=True)
+    out = subprocess.run([harness, str(tmp_path / "in.bin"), str(tmp_path / "out.bin")], capture_output=True, text=True)
     assert out.returncode == 0, out.stderr
     raw = open(tmp_path / "out.bin", "rb").read()
     seed = struct.unpack("<Q", raw[:8])[0]
@@ -74,15 +74,14 @@ def test_shim_call_matches_c_abi(tmp_path):
 
 
 @pytest.mark.gpu
-def test_shim_extended_call_thins_and_summarises(tmp_path):
+def test_shim_extended_call_thins_and_summarises(harness, tmp_path):
     """.Call(`_gpirt_gpirtMCMC_b200`, ..., thin, store_f, f_summary): list of 6 with 1 + S %/% thin slots"""
     import gpirt_b200
     import gpirt_b200.sampler as G
-    build_harness()
     n, m, S, B, thin = 40, 13, 9, 2, 3
     p = make_problem(n, m, seed=4, missing=0.05)
     write_input(tmp_path / "in.bin", p, S, B, 777)
-    out = subprocess.run([HARNESS, str(tmp_path / "in.bin"), str(tmp_path / "out.bin"), str(thin)], capture_output=True, text=True)
+    out = subprocess.run([harness, str(tmp_path / "in.bin"), str(tmp_path / "out.bin"), str(thin)], capture_output=True, text=True)
     assert out.returncode == 0, out.stderr
     raw = open(tmp_path / "out.bin", "rb").read()
     seed = struct.unpack("<Q", raw[:8])[0]
