@@ -40,6 +40,7 @@ constexpr int DG_STAGES = 196608 / DG_STAGE_BYTES;
 constexpr int DG_SMEM = DG_STAGES * DG_STAGE_BYTES + 1024 /* alignment slack */ + 256 /* barriers */;
 constexpr int DG_TMEM_COLS = 512;
 constexpr int DG_THREADS = 192;   // warp 0: TMA producer, warp 1: MMA issuer (+ TMEM alloc), warps 2..5: epilogue
+constexpr int CN = 2;             // CTAs per cluster (they share the A slab, see k_dgemm_i8)
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 // one lane of a converged warp; ptxas recognises the pattern and emits the tensor-core / TMA instructions of the elected
@@ -144,7 +145,7 @@ __device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
                  ::"r"(bar), "h"(mask) : "memory");
 }
 
-// With a cluster of CN CTAs the scheduler's "column tile" is a group of CN adjacent 64-column tiles (one per CTA of the
+// With clusters of CN CTAs the scheduler's "column tile" is a group of CN adjacent 64-column tiles (one per CTA of the
 // cluster, all on the same row tile): ntiles, group_cols and total count those groups.
 struct TileSched {
     int mtiles, ntiles, group_cols, total, ascending;   // ascending: row tile 0 is the heaviest (upper-triangular A)
@@ -159,12 +160,11 @@ struct TileSched {
     }
 };
 
-// CN > 1: clusters of CN CTAs work on CN adjacent column tiles of the same row tile.  Each CTA loads 128 / CN rows of
+// Clusters of CN CTAs work on CN adjacent column tiles of the same row tile.  Each CTA loads 128 / CN rows of
 // every A plane and MULTICASTS them to the whole cluster, so the A slab crosses the L2 -> SM fabric once per cluster
 // instead of once per CTA (the 128 x 64 tile is exactly balanced between the int8 tensor rate and the L2 feed rate:
 // 96 KB per 2304 tensor-core cycles per SM = 6.2 KB/clk chip-wide; with CN = 2 it is 64 KB).  A stage may be refilled only
 // when every CTA of the cluster has consumed it: the MMA issuer's commit arrives on the stage's empty barrier of ALL CTAs.
-template <int CN>
 __global__ void __launch_bounds__(DG_THREADS, 1)
 k_dgemm_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, TileSched sched,
            int a_rows_pad, int b_rows_pad, int kb_lo, int kb_hi, int a_tri, int M, int N,
@@ -178,7 +178,7 @@ k_dgemm_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
     uint32_t* tmem_slot = (uint32_t*)(bars + 2 * DG_STAGES + 2);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 
-    const uint32_t crank = CN > 1 ? cluster_ctarank() : 0u;
+    const uint32_t crank = cluster_ctarank();
     const int cluster_id = blockIdx.x / CN, n_clusters = gridDim.x / CN;
     constexpr uint16_t CMASK = (uint16_t)((1u << CN) - 1u);
     if (warp == 0 && lane == 0) {
@@ -195,7 +195,7 @@ k_dgemm_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const uint32_t tmem_base = *tmem_slot;
-    if constexpr (CN > 1) cluster_sync_all();   // every CTA's barriers are initialised before a peer signals them
+    cluster_sync_all();   // every CTA's barriers are initialised before a peer signals them
 
     // K-block range of a row tile: a lower-triangular A stops at the diagonal block, an upper-triangular one starts there
     auto kb_end = [&](int r) { return a_tri == 1 ? min(kb_hi, (int)(((int64_t)(r + 1) * DG_BM + DG_KB - 1) / DG_KB)) : kb_hi; };
@@ -218,11 +218,8 @@ k_dgemm_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
                 const uint32_t sa = smem_u32(smem + s * DG_STAGE_BYTES), sb = sa + DG_A_BYTES;
 #pragma unroll
                 for (int p = 0; p < DG_S; ++p) {
-                    if constexpr (CN > 1)
-                        tma_load_2d_mc(sa + p * DG_A_PLANE + crank * A_PART, &tmA, kb * DG_KB,
-                                       p * a_rows_pad + r * DG_BM + (int)crank * A_PART_ROWS, full0 + 8 * s, CMASK);
-                    else
-                        tma_load_2d(sa + p * DG_A_PLANE, &tmA, kb * DG_KB, p * a_rows_pad + r * DG_BM, full0 + 8 * s);
+                    tma_load_2d_mc(sa + p * DG_A_PLANE + crank * A_PART, &tmA, kb * DG_KB,
+                                   p * a_rows_pad + r * DG_BM + (int)crank * A_PART_ROWS, full0 + 8 * s, CMASK);
                     tma_load_2d(sb + p * DG_B_PLANE, &tmB, kb * DG_KB, p * b_rows_pad + c * DG_BN, full0 + 8 * s);
                 }
             }
@@ -246,8 +243,7 @@ k_dgemm_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
 #pragma unroll
                 for (int k2 = 0; k2 < DG_KB / DG_UMMA_K; ++k2)
                     umma_all_planes(tmem_base, sa + k2 * DG_UMMA_K, sb + k2 * DG_UMMA_K, (uint32_t)((kb != kb0) | (k2 != 0)));
-                if constexpr (CN > 1) umma_commit_mc(empty0 + 8 * s, CMASK);   // frees the slot in every CTA of the cluster
-                else umma_commit(empty0 + 8 * s);                              // ... once these MMAs have read it
+                umma_commit_mc(empty0 + 8 * s, CMASK);   // frees the slot in every CTA of the cluster once these MMAs have read it
             }
             umma_commit(tfull);                // all level accumulators of this tile are complete
         }
@@ -302,7 +298,7 @@ k_dgemm_i8(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUte
     }
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
-    if constexpr (CN > 1) cluster_sync_all();   // no CTA leaves while a peer may still signal its barriers
+    cluster_sync_all();   // no CTA leaves while a peer may still signal its barriers
     if (warp == 1) {
         asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(DG_TMEM_COLS) : "memory");
     }
@@ -444,19 +440,9 @@ constexpr int ROWMAX_CHUNKS = 16;
 
 struct DigitPlanes::Map { CUtensorMap m, m_part; };   // m_part: box of box_rows / cluster size rows (multicast parts of an A slab)
 
-// CTAs per cluster of k_dgemm_i8 (GPIRT_I8_CLUSTER = 1, 2 or 4)
-static int cluster_cols() {
-    static const int cn = [] {
-        const char* e = getenv("GPIRT_I8_CLUSTER");
-        const int v = e ? atoi(e) : 2;
-        return (v == 1 || v == 2 || v == 4) ? v : 2;
-    }();
-    return cn;
-}
-
 int DigitPlanes::init(cudaStream_t st, int rows_, int k_, int box_rows_) {
     rows = rows_; k = k_; box_rows = box_rows_;
-    rows_pad = round_up(rows, box_rows == DG_BN ? DG_BN * cluster_cols() : box_rows);   // whole clusters of column tiles
+    rows_pad = round_up(rows, box_rows == DG_BN ? DG_BN * CN : box_rows);   // whole clusters of column tiles
     k_pad = round_up(k, 128);
     const size_t bytes = (size_t)S * rows_pad * k_pad;
     GP_TRY(pool_alloc((void**)&planes, bytes, st));
@@ -467,7 +453,7 @@ int DigitPlanes::init(cudaStream_t st, int rows_, int k_, int box_rows_) {
     GP_CUDA(cudaMemsetAsync(scale, 0, (size_t)rows_pad * sizeof(double), st));
     map = new Map();
     GP_TRY(make_map_sw64(&map->m, planes, (uint64_t)S * rows_pad, (uint64_t)k_pad, (uint32_t)box_rows));
-    GP_TRY(make_map_sw64(&map->m_part, planes, (uint64_t)S * rows_pad, (uint64_t)k_pad, (uint32_t)(box_rows / cluster_cols())));
+    GP_TRY(make_map_sw64(&map->m_part, planes, (uint64_t)S * rows_pad, (uint64_t)k_pad, (uint32_t)(box_rows / CN)));
     return GPIRT_B200_OK;
 }
 
@@ -512,35 +498,30 @@ int dgemm_i8(cudaStream_t st, const DigitPlanes& A, const DigitPlanes& B, double
     int dev = 0;
     GP_CUDA(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64) { set_last_error("dgemm_i8: device ordinal out of range"); return GPIRT_B200_ERR_ARG; }
-    const int cn = cluster_cols();
     {
         DeviceOnce once(attr_set);
         if (once.first) {
             GP_CUDA(cudaDeviceGetAttribute(&sm_count[dev], cudaDevAttrMultiProcessorCount, dev));
-            GP_CUDA(cudaFuncSetAttribute(k_dgemm_i8<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, DG_SMEM));
-            GP_CUDA(cudaFuncSetAttribute(k_dgemm_i8<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, DG_SMEM));
-            GP_CUDA(cudaFuncSetAttribute(k_dgemm_i8<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, DG_SMEM));
+            GP_CUDA(cudaFuncSetAttribute(k_dgemm_i8, cudaFuncAttributeMaxDynamicSharedMemorySize, DG_SMEM));
         }
     }
     const int n_sm = sm_count[dev];
-    if (B.rows_pad % (DG_BN * cn) != 0) { set_last_error("dgemm_i8: B operand is not padded to whole clusters"); return GPIRT_B200_ERR_ARG; }
+    if (B.rows_pad % (DG_BN * CN) != 0) { set_last_error("dgemm_i8: B operand is not padded to whole clusters"); return GPIRT_B200_ERR_ARG; }
     TileSched sched;
     // an accumulating slice of a lower-triangular product adds nothing to the rows above its first column
     sched.mtile0 = (a_tri == DG_TRI_LOWER && accumulate) ? k_lo / DG_BM : 0;
     sched.mtiles = (int)(A.rows_pad / DG_BM) - sched.mtile0;
     if (sched.mtiles <= 0) return GPIRT_B200_OK;
-    sched.ntiles = (int)(B.rows_pad / (DG_BN * cn));
-    const int gc = group_cols > 0 ? (int)ceil_div(group_cols, cn) : 0;
+    sched.ntiles = (int)(B.rows_pad / (DG_BN * CN));
+    const int gc = group_cols > 0 ? (int)ceil_div(group_cols, CN) : 0;
     sched.group_cols = gc > 0 ? min(gc, sched.ntiles) : sched.ntiles;
     sched.total = sched.mtiles * sched.ntiles;
     sched.ascending = a_tri == DG_TRI_UPPER ? 1 : 0;
     // persistent (one CTA per SM walks the tile list) when the kernel owns the GPU; one tile per CTA when it shares the
     // GPU with a latency-critical chain on a higher-priority stream, so that the chain's CTAs get SMs as tiles retire
-    static const int force = getenv("GPIRT_I8_PERSISTENT") ? atoi(getenv("GPIRT_I8_PERSISTENT")) : -1;
-    const bool pers = force >= 0 ? force != 0 : persistent;
-    const int clusters = pers ? min(sched.total, n_sm / cn) : sched.total;
+    const int clusters = persistent ? min(sched.total, n_sm / CN) : sched.total;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(clusters * cn));
+    cfg.gridDim = dim3((unsigned)(clusters * CN));
     cfg.blockDim = dim3(DG_THREADS);
     cfg.dynamicSmemBytes = DG_SMEM;
     cfg.stream = st;
@@ -551,18 +532,14 @@ int dgemm_i8(cudaStream_t st, const DigitPlanes& A, const DigitPlanes& B, double
         attr[na].val.priority = prio;
         ++na;
     }
-    if (cn > 1) {
-        attr[na].id = cudaLaunchAttributeClusterDimension;
-        attr[na].val.clusterDim.x = (unsigned)cn; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
-        ++na;
-    }
+    attr[na].id = cudaLaunchAttributeClusterDimension;
+    attr[na].val.clusterDim.x = (unsigned)CN; attr[na].val.clusterDim.y = 1; attr[na].val.clusterDim.z = 1;
+    ++na;
     cfg.attrs = attr;
     cfg.numAttrs = na;
-    const CUtensorMap& ma = cn > 1 ? A.map->m_part : A.map->m;
     const int a_rows_pad = (int)A.rows_pad, b_rows_pad = (int)B.rows_pad, kb_lo = k_lo / DG_KB, kb_hi = (int)ceil_div(k_hi, DG_KB);
     const int acc = accumulate ? 1 : 0;
-    auto kern = cn == 4 ? k_dgemm_i8<4> : (cn == 2 ? k_dgemm_i8<2> : k_dgemm_i8<1>);
-    GP_CUDA(cudaLaunchKernelEx(&cfg, kern, ma, B.map->m, sched, a_rows_pad, b_rows_pad, kb_lo, kb_hi, a_tri, A.rows, B.rows,
+    GP_CUDA(cudaLaunchKernelEx(&cfg, k_dgemm_i8, A.map->m_part, B.map->m, sched, a_rows_pad, b_rows_pad, kb_lo, kb_hi, a_tri, A.rows, B.rows,
                                (const double*)A.scale, (const double*)B.scale, C, ldc, acc));
     ++g_launch_count;
     GP_CUDA(cudaGetLastError());

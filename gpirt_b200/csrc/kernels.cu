@@ -264,8 +264,8 @@ template <int EPT> struct ItemRegs {
     }
 };
 
-template <int EPT, int MAXT>
-__global__ void __launch_bounds__(MAXT) k_ess(double* __restrict__ f, const double* __restrict__ nu, int64_t ld, const int8_t* __restrict__ y8,
+template <int EPT>
+__global__ void __launch_bounds__(512) k_ess(double* __restrict__ f, const double* __restrict__ nu, int64_t ld, const int8_t* __restrict__ y8,
                       int64_t ldy, const double* __restrict__ theta, const double* __restrict__ beta, int n, RngKey key,
                       uint32_t item_offset, int* __restrict__ nprop, int* __restrict__ status,
                       const double* __restrict__ sp) {
@@ -341,8 +341,8 @@ __device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
-template <int EPT, int MAXT>
-__global__ void __launch_bounds__(MAXT) k_ess_persist(double* __restrict__ f, const double* __restrict__ nu, int64_t ld,
+template <int EPT>
+__global__ void __launch_bounds__(512) k_ess_persist(double* __restrict__ f, const double* __restrict__ nu, int64_t ld,
                                                       const int8_t* __restrict__ y8, int64_t ldy, const double* __restrict__ theta,
                                                       const double* __restrict__ beta, int n, int m, RngKey key,
                                                       uint32_t item_offset, int* __restrict__ nprop, int* __restrict__ status,
@@ -430,29 +430,23 @@ static int persistent_grid(K kernel, int threads, size_t smem, int m, int* grid)
     *grid = m > it->second ? it->second : 0;
     return GPIRT_B200_OK;
 }
-static bool item_kernels_persistent() {
-    static const int v = getenv("GPIRT_ITEM_PERSIST") ? atoi(getenv("GPIRT_ITEM_PERSIST")) : 1;
-    return v != 0;
-}
-
 // block size / elements-per-thread for a per-item CTA holding n <= 4096 respondents in registers (ept = 0: stream)
 static void item_cta_shape(int n, int& ept, int& threads) {
-    // 2048 < n <= 4096: 512 threads x 8 values.  GPIRT_ITEM_THREADS=1024 selects 1024 x 4 (32 warps per SM instead of
-    // 16): measured 10% SLOWER at n = 4096 — the kernels are bound by the L1 gather of table rows, not by latency.
-    static const int wide = getenv("GPIRT_ITEM_THREADS") ? atoi(getenv("GPIRT_ITEM_THREADS")) : 512;
-    if (n <= 256) ept = 1; else if (n <= 1024) ept = 2; else if (n <= 2048) ept = 4; else if (n <= 4096) ept = (wide > 512 ? 4 : 8); else ept = 0;
+    // 2048 < n <= 4096: 512 threads x 8 values.  1024 x 4 (32 warps per SM instead of 16) was measured 10% SLOWER at
+    // n = 4096 — the kernels are bound by the L1 gather of table rows, not by latency.
+    if (n <= 256) ept = 1; else if (n <= 1024) ept = 2; else if (n <= 2048) ept = 4; else if (n <= 4096) ept = 8; else ept = 0;
     threads = ept ? (int)round_up(ceil_div(n, ept), 32) : 1024;
     if (threads < 32) threads = 32;
 }
 
-#define ESS_PERSIST_CASE(E, MT)                                                                                              \
+#define ESS_PERSIST_CASE(E)                                                                                                  \
     {                                                                                                                            \
         const size_t smem = (size_t)2 * (E) * threads * 17;                                                                      \
         int grid = 0;                                                                                                            \
-        GP_TRY(persistent_grid(k_ess_persist<E, MT>, threads, smem, m, &grid));                                                  \
+        GP_TRY(persistent_grid(k_ess_persist<E>, threads, smem, m, &grid));                                                  \
         if (grid > 0) {                                                                                                          \
             GP_CUDA(cudaMemsetAsync(work, 0, sizeof(int), st));                                                                  \
-            GP_LAUNCH((k_ess_persist<E, MT>), grid, threads, smem, st, f, nu, ld, y8, ldy, theta, beta, n, m, key, item_offset,  \
+            GP_LAUNCH((k_ess_persist<E>), grid, threads, smem, st, f, nu, ld, y8, ldy, theta, beta, n, m, key, item_offset,  \
                       nprop, status, sp, work);                                                                                  \
             launched = true;                                                                                                     \
         }                                                                                                                        \
@@ -466,26 +460,23 @@ int launch_ess(cudaStream_t st, double* f, const double* nu, int64_t ld, const i
     item_cta_shape(n, ept, threads);
     const double* sp = nullptr;
     GP_TRY(softplus_table(&sp));
-    if (work && ept && item_kernels_persistent()) {
+    if (work && ept) {
         bool launched = false;
         switch (ept) {
-            case 1: ESS_PERSIST_CASE(1, 512) break;
-            case 2: ESS_PERSIST_CASE(2, 512) break;
-            case 4: if (threads > 512) ESS_PERSIST_CASE(4, 1024) else ESS_PERSIST_CASE(4, 512) break;
-            default: ESS_PERSIST_CASE(8, 512) break;
+            case 1: ESS_PERSIST_CASE(1) break;
+            case 2: ESS_PERSIST_CASE(2) break;
+            case 4: ESS_PERSIST_CASE(4) break;
+            default: ESS_PERSIST_CASE(8) break;
         }
         GP_CUDA(cudaGetLastError());
         if (launched) { if (shape) *shape = ITEM_SHAPE_PERSISTENT; return GPIRT_B200_OK; }
     }
     if (shape) *shape = ept ? ITEM_SHAPE_CTA : ITEM_SHAPE_STREAM;
     switch (ept) {
-        case 1: GP_LAUNCH((k_ess<1, 512>), m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp); break;
-        case 2: GP_LAUNCH((k_ess<2, 512>), m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp); break;
-        case 4:
-            if (threads > 512) GP_LAUNCH((k_ess<4, 1024>), m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp);
-            else GP_LAUNCH((k_ess<4, 512>), m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp);
-            break;
-        case 8: GP_LAUNCH((k_ess<8, 512>), m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp); break;
+        case 1: GP_LAUNCH(k_ess<1>, m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp); break;
+        case 2: GP_LAUNCH(k_ess<2>, m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp); break;
+        case 4: GP_LAUNCH(k_ess<4>, m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp); break;
+        case 8: GP_LAUNCH(k_ess<8>, m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp); break;
         default: GP_LAUNCH(k_ess_stream, m, threads, 0, st, f, nu, ld, y8, ldy, theta, beta, n, key, item_offset, nprop, status, sp); break;
     }
     GP_CUDA(cudaGetLastError());
@@ -731,8 +722,8 @@ template <int EPT> struct BetaRegs {
     }
 };
 
-template <int EPT, int MAXT>
-__global__ void __launch_bounds__(MAXT) k_beta(double* __restrict__ beta, const double* __restrict__ f, int64_t ld, const int8_t* __restrict__ y8,
+template <int EPT>
+__global__ void __launch_bounds__(512) k_beta(double* __restrict__ beta, const double* __restrict__ f, int64_t ld, const int8_t* __restrict__ y8,
                        int64_t ldy, const double* __restrict__ theta, const double* __restrict__ pm,
                        const double* __restrict__ psd, const double* __restrict__ pstep, int n, RngKey key,
                        uint32_t item_offset, const double* __restrict__ sp) {
@@ -750,8 +741,8 @@ __global__ void __launch_bounds__(MAXT) k_beta(double* __restrict__ beta, const 
 }
 
 // persistent shape of the beta step (see k_ess_persist): next item's f and y columns prefetched, theta read once
-template <int EPT, int MAXT>
-__global__ void __launch_bounds__(MAXT) k_beta_persist(double* __restrict__ beta, const double* __restrict__ f, int64_t ld,
+template <int EPT>
+__global__ void __launch_bounds__(512) k_beta_persist(double* __restrict__ beta, const double* __restrict__ f, int64_t ld,
                                                        const int8_t* __restrict__ y8, int64_t ldy, const double* __restrict__ theta,
                                                        const double* __restrict__ pm, const double* __restrict__ psd,
                                                        const double* __restrict__ pstep, int n, int m, RngKey key,
@@ -814,14 +805,14 @@ __global__ void __launch_bounds__(1024) k_beta_stream(double* __restrict__ beta,
               });
 }
 
-#define BETA_PERSIST_CASE(E, MT)                                                                                             \
+#define BETA_PERSIST_CASE(E)                                                                                                 \
     {                                                                                                                            \
         const size_t smem = (size_t)2 * (E) * threads * 9;                                                                       \
         int grid = 0;                                                                                                            \
-        GP_TRY(persistent_grid(k_beta_persist<E, MT>, threads, smem, m, &grid));                                                 \
+        GP_TRY(persistent_grid(k_beta_persist<E>, threads, smem, m, &grid));                                                 \
         if (grid > 0) {                                                                                                          \
             GP_CUDA(cudaMemsetAsync(work, 0, sizeof(int), st));                                                                  \
-            GP_LAUNCH((k_beta_persist<E, MT>), grid, threads, smem, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, m, key,  \
+            GP_LAUNCH((k_beta_persist<E>), grid, threads, smem, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, m, key,  \
                       item_offset, sp, work);                                                                                    \
             launched = true;                                                                                                     \
         }                                                                                                                        \
@@ -836,26 +827,23 @@ int launch_beta(cudaStream_t st, double* beta, const double* f, int64_t ld, cons
     item_cta_shape(n, ept, threads);
     const double* sp = nullptr;
     GP_TRY(softplus_table(&sp));
-    if (work && ept && item_kernels_persistent()) {
+    if (work && ept) {
         bool launched = false;
         switch (ept) {
-            case 1: BETA_PERSIST_CASE(1, 512) break;
-            case 2: BETA_PERSIST_CASE(2, 512) break;
-            case 4: if (threads > 512) BETA_PERSIST_CASE(4, 1024) else BETA_PERSIST_CASE(4, 512) break;
-            default: BETA_PERSIST_CASE(8, 512) break;
+            case 1: BETA_PERSIST_CASE(1) break;
+            case 2: BETA_PERSIST_CASE(2) break;
+            case 4: BETA_PERSIST_CASE(4) break;
+            default: BETA_PERSIST_CASE(8) break;
         }
         GP_CUDA(cudaGetLastError());
         if (launched) { if (shape) *shape = ITEM_SHAPE_PERSISTENT; return GPIRT_B200_OK; }
     }
     if (shape) *shape = ept ? ITEM_SHAPE_CTA : ITEM_SHAPE_STREAM;
     switch (ept) {
-        case 1: GP_LAUNCH((k_beta<1, 512>), m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp); break;
-        case 2: GP_LAUNCH((k_beta<2, 512>), m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp); break;
-        case 4:
-            if (threads > 512) GP_LAUNCH((k_beta<4, 1024>), m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp);
-            else GP_LAUNCH((k_beta<4, 512>), m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp);
-            break;
-        case 8: GP_LAUNCH((k_beta<8, 512>), m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp); break;
+        case 1: GP_LAUNCH(k_beta<1>, m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp); break;
+        case 2: GP_LAUNCH(k_beta<2>, m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp); break;
+        case 4: GP_LAUNCH(k_beta<4>, m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp); break;
+        case 8: GP_LAUNCH(k_beta<8>, m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp); break;
         default: GP_LAUNCH(k_beta_stream, m, threads, 0, st, beta, f, ld, y8, ldy, theta, pm, psd, pstep, n, key, item_offset, sp); break;
     }
     GP_CUDA(cudaGetLastError());

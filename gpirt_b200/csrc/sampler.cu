@@ -147,27 +147,40 @@ struct gpirt_b200_sampler {
     bool pipeline = true;
     cudaStream_t st_beta = nullptr, st_lz = nullptr;
     cudaEvent_t ev_theta = nullptr, ev_z = nullptr, ev_beta = nullptr, ev_lz = nullptr;
-    bool nu_ready = false;       // nu already holds L z for sweep nu_sweep
-    uint32_t nu_sweep = 0;
-    bool solve_ready = false;    // kstar already holds S^-1 K* and s the predictive sd for the current theta (ev_solve)
     cudaEvent_t ev_linv = nullptr, ev_solve = nullptr, ev_fwd = nullptr;
-    // The K* solves of the NEXT sweep depend on theta and the factor only.  rebuild_pipelined leaves them pending and the
-    // next sweep starts them on a side stream right before its ESS, so that they run beside it — and so that every side
-    // stream is joined at the end of a sweep, which is what lets the whole pipelined sweep be captured as a CUDA graph.
-    //   1: backward substitution of this rank's grid columns (the forward steps trailed the panels)   2: through L^-1
-    int deferred = 0;
+    // What a pipelined sweep leaves for the next one.  The K* solves of the NEXT sweep depend on theta and the factor
+    // only: rebuild_pipelined leaves them pending and the next sweep starts them on a side stream right before its ESS,
+    // so that they run beside it — and so that every side stream is joined at the end of a sweep, which is what lets the
+    // whole pipelined sweep be captured as a CUDA graph.
+    struct Carry {
+        enum class Start { NONE, BWD, LINV_SOLVES };   // backward substitution of this rank's grid columns (the forward
+                                                       // steps trailed the panels), or the solves through L^-1
+        enum class Solved { NONE, LOCAL, ALL };        // in flight behind ev_solve: this rank's slice of S^-1 K* and s (not
+                                                       // yet gathered), or S^-1 K* and s complete for the current theta
+        bool nu_ready = false;       // nu already holds L z for sweep nu_sweep
+        uint32_t nu_sweep = 0;
+        Start start = Start::NONE;   // K* work the next sweep starts before its ESS
+        Solved solved = Solved::NONE;
+        bool ess_yields = false;     // the backward pass was just started: the ESS that follows must leave it SMs
+    } carry;
+    // discards the carried state (the sampler's state was changed from outside the sweep, or the sweep's shape changes)
+    void drop_carry() {
+        if (carry.solved != Carry::Solved::NONE) cudaStreamWaitEvent(stream, ev_solve, 0);
+        carry = Carry{};
+    }
     int prio_second = 0;            // one notch below the top stream priority
-    bool tail_beside_ess = false;   // the backward pass was just started: the ESS that follows must leave it SMs
-    int pipe_mask = 7;           // GPIRT_PIPE_MASK (debugging): 1 LZ, 2 beta / fill, 4 solves on their own streams
     int launch_deferred_solves();
     int fstar_solves(cudaStream_t st);
-    // solve_mode 1 (default with items sharded over GPUs): the two triangular solves for this rank's slice of the grid
-    // columns as blocked substitutions with the 128-block inverses of the factorisation — no L^-1.  The forward steps
-    // trail the Cholesky panels on st_trsm; only the backward pass (32 short steps) follows the factorisation.  With
-    // few right-hand sides per rank this replaces the replicated 1.3 ms L^-1 + products by a ~0.4 ms chain.
-    int solve_mode = 0;
+    // Route of the K* solves, chosen once in create():
+    //   LINV     (default on one GPU for n <= 6144) through L^-1
+    //   SUBST    (default with items sharded over GPUs, and for n > 6144) the two triangular solves for this rank's slice
+    //            of the grid columns as blocked substitutions with the 128-block inverses of the factorisation — no L^-1.
+    //            The forward steps trail the Cholesky panels on st_trsm; only the backward pass (32 short steps) follows
+    //            the factorisation.  With few right-hand sides per rank this replaces the replicated 1.3 ms L^-1 +
+    //            products by a ~0.4 ms chain.
+    //   LITERAL  opts.fstar_mode = 1: the reference's per-item solves, through L^-1
+    enum class Route { LINV, SUBST, LITERAL } route = Route::LINV;
     cudaStream_t st_trsm = nullptr;
-    bool local_solve_ready = false;   // this rank's slice of S^-1 K* and s is complete on st_trsm (ev_solve), not yet gathered
     void grid_slice(int& c0, int& nc) const {
         const int per = (int)ceil_div(N_GRID, comm.world);
         c0 = std::min(N_GRID, comm.rank * per);
@@ -248,19 +261,8 @@ struct gpirt_b200_sampler {
         if (!pool.empty()) { cudaEvent_t e = pool.back(); pool.pop_back(); return e; }
         cudaEvent_t e; cudaEventCreate(&e); return e;
     }
-    void tic(int timer) {
-        if (stamping()) { cur = tic_on(timer, stream); return; }
-        cur.slot = -1;
-        if (!timing || capturing) return;
-        cur.timer = timer; cur.a = get_event(); cur.b = get_event();
-        cudaEventRecord(cur.a, stream);
-    }
-    void toc() {
-        if (cur.slot >= 0) { toc_on(cur, stream); cur.slot = -1; return; }
-        if (!timing || capturing) return;
-        cudaEventRecord(cur.b, stream);
-        pending.push_back(cur);
-    }
+    void tic(int timer) { cur = tic_on(timer, stream); }
+    void toc() { toc_on(cur, stream); }
     // GPIRT_TRACE=<file>: every timed segment is also written as "timer start_ms end_ms" relative to the sampler's
     // creation (segments of different streams overlap: this is the timeline the per-timer sums cannot show)
     cudaEvent_t trace_ref = nullptr;
@@ -290,14 +292,13 @@ struct gpirt_b200_sampler {
     }
     // ---- CUDA graph of a sweep (small n: ~20 short kernels, pure launch latency; n > 256: the pipelined sweep, whose
     // Cholesky chain takes ~15 host API calls per panel — with items sharded the host is the limit otherwise) ----
-    bool graph_enabled = true, capturing = false, warmed = false;
+    bool graph_enabled = true, capturing = false, warmed = false;   // graph_enabled: opts.use_graph >= 0 and capturable
     uint32_t capture_base = 0;
     uint32_t* d_sweep = nullptr;          // device copy of the sweep counter read by the captured kernels
     uint32_t d_sweep_value = 0xffffffffu; // what *d_sweep holds (host mirror)
     cudaGraphExec_t gexec[2] = {nullptr, nullptr};   // [accumulate_irf]
     int64_t graph_replays = 0;            // sweeps run as a graph launch (gpirt_b200_sampler_uses(s, 5))
-    bool graph_pipelined = false;         // the captured sweep is the pipelined one (side streams forked and joined inside the graph)
-    int graph_deferred = 0;
+    Carry graph_carry[2];                 // what the captured sweep left, nu_sweep relative to the captured sweep
     void drop_graphs() { for (auto& g : gexec) if (g) { cudaGraphExecDestroy(g); g = nullptr; } }
     int64_t graph_kernels = 0;            // kernels per sweep (counted on the eager path; a graph replay launches the same ones)
     int sweep_eager(uint32_t t, int accumulate);
@@ -363,10 +364,7 @@ int gpirt_b200_sampler::create(const double* y, int64_t n_, int64_t m_, const do
     }
     if (o && opts.device >= 0) GP_CUDA(cudaSetDevice(opts.device));
     key.k0 = (uint32_t)opts.seed; key.k1 = (uint32_t)(opts.seed >> 32); key.sweep = 0; key.sweep_dev = nullptr;
-    {
-        const char* ge = getenv("GPIRT_GRAPH");
-        graph_enabled = ge ? atoi(ge) != 0 : opts.use_graph >= 0;
-    }
+    graph_enabled = opts.use_graph >= 0;
     if (opts.world_size > 1) {
         item_offset = (uint32_t)opts.item_offset;
         GP_TRY(comm_init(comm, opts.rank, opts.world_size, opts.nccl_unique_id));
@@ -387,19 +385,18 @@ int gpirt_b200_sampler::create(const double* y, int64_t n_, int64_t m_, const do
         // the substitution steps that trail the panels yield to the chain itself
         GP_CUDA(cudaStreamCreateWithPriority(&st_trsm, cudaStreamNonBlocking, greatest < least ? greatest + 1 : greatest));
         for (cudaEvent_t* e : {&ev_theta, &ev_z, &ev_beta, &ev_lz, &ev_linv, &ev_solve, &ev_fwd}) GP_CUDA(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
-        if (const char* pm = getenv("GPIRT_PIPE_MASK")) pipe_mask = atoi(pm);
         if (trace_file) {
             GP_CUDA(cudaEventCreate(&trace_ref)); GP_CUDA(cudaEventRecord(trace_ref, stream));
             GP_CUDA(cudaMalloc((void**)&d_stamps, MAX_STAMPS * sizeof(unsigned long long)));
             GP_CUDA(cudaMemset(d_stamps, 0, MAX_STAMPS * sizeof(unsigned long long)));
         }
+        // GPIRT_SOLVE_MODE = 0 / 1 forces the route through L^-1 / by substitution.  Through L^-1 costs n^3/3 for the
+        // inverse + two triangular products, blocked substitution behind the Cholesky panels 2 n^2 x 1001: substitution
+        // wins when few right-hand sides are left per rank, and on one GPU once n/3 > 2 x 1001
         const char* sm = getenv("GPIRT_SOLVE_MODE");
-        // through L^-1 (n^3/3 for the inverse + two triangular products) or by blocked substitution behind the Cholesky panels
-        // (2 n^2 x 1001): substitution wins when few right-hand sides are left per rank, and on one GPU once n/3 > 2 x 1001
-        solve_mode = sm ? atoi(sm) : ((comm.world > 1 || n > 6144) ? 1 : 0);
-        if (opts.fstar_mode != 0) solve_mode = 0;   // the literal per-item form needs L^-1
-        const char* pe = getenv("GPIRT_PIPELINE");
-        if (pe) pipeline = atoi(pe) != 0;
+        const bool subst = sm ? atoi(sm) == 1 : (comm.world > 1 || n > 6144);
+        if (opts.fstar_mode != 0) route = Route::LITERAL;   // the literal per-item form needs L^-1
+        else route = subst ? Route::SUBST : Route::LINV;
     }
 
     const size_t nm = (size_t)ldn * m, Nm = (size_t)ldN * m;
@@ -421,7 +418,7 @@ int gpirt_b200_sampler::create(const double* y, int64_t n_, int64_t m_, const do
     GP_TRY(alloc(f, nm)); GP_TRY(alloc(Z, nm)); GP_TRY(alloc(nu, nm));
     GP_TRY(alloc(fstar, Nm)); GP_TRY(alloc(Dmat, Nm)); GP_TRY(alloc(irf_sum, Nm));
     GP_TRY(alloc(kstar, (size_t)ldn * kcols)); GP_TRY(alloc(s, std::max((size_t)ldN, kcols)));
-    if (solve_mode == 1) {
+    if (route == Route::SUBST) {
         // split-K workspace: the thin products of the backward pass (M <= 4096 rows x this rank's grid columns, 8 splits) and
         // the batched late levels of the block inverses (n / 1024 pairs of 512 x 512 tiles, 4 splits)
         const size_t per = (size_t)ceil_div(N_GRID, comm.world);
@@ -472,16 +469,15 @@ int gpirt_b200_sampler::create(const double* y, int64_t n_, int64_t m_, const do
             GP_TRY(dp_L.init(stream, n, n, 128));
             GP_TRY(dp_A.init(stream, N_GRID, n, 128));
             GP_TRY(dp_B.init(stream, m, n, 64));
-            if (opts.fstar_mode == 0 && solve_mode == 0) {
-                const int per = (int)ceil_div(N_GRID, comm.world), c0 = min(N_GRID, comm.rank * per), nc = min(N_GRID, c0 + per) - c0;
+            if (route == Route::LINV) {
+                int c0, nc;
+                grid_slice(c0, nc);
                 GP_TRY(dp_Linv.init(stream, n, n, 128));
                 GP_TRY(dp_LinvT.init(stream, n, n, 128));
                 if (nc > 0) GP_TRY(dp_K.init(stream, nc, n, 64));
             }
             lz_group = 16;
         }
-        const char* g = getenv("GPIRT_LZ_GROUP");
-        if (g && atoi(g) > 0) lz_group = atoi(g);
     }
     GP_TRY(step_rebuild());                                                         // gpirtMCMC.cpp:15-17
     GP_CUDA(cudaStreamSynchronize(stream));
@@ -509,7 +505,7 @@ int gpirt_b200_sampler::step_rebuild() {
     tic(GPIRT_B200_T_CHOL);
     GP_TRY(potrf_lower_rl(stream, L, ldn, n, Dinv, ldn, status, chol_flags, &lookahead));
     toc();
-    if (solve_mode == 0) {
+    if (route != Route::SUBST) {
         tic(GPIRT_B200_T_TRTRI);   // L^-1 once per sweep: every triangular solve of draw_fstar becomes a triangular GEMM
         GP_TRY(trtri_lower(stream, L, ldn, n, Dinv, ldn, Linv, ldn, Tmp, ldn));
         toc();
@@ -583,17 +579,11 @@ int gpirt_b200_sampler::trsm_fwd_step(cudaStream_t st, int k) {
 // grid columns per rank those products are thin (126 columns at 8 GPUs: 32 output tiles, K = 1024), so they are split
 // over K (deterministic split-K, gemm_f64.cuh); and every diagonal-block inverse but the last is computed behind the
 // factorisation (invert_bwd_block from the panel hook), which leaves one block inverse and seven short products in the tail.
-int gpirt_b200_sampler::bwd_block() const {
-    static const int forced = getenv("GPIRT_BWD_BLOCK") ? atoi(getenv("GPIRT_BWD_BLOCK")) : 0;
-    int blk = forced > 0 ? forced : (n >= 2048 ? 1024 : (n >= 1024 ? 512 : CHOL_NB));
-    if (blk % CHOL_NB != 0 || (blk & (blk - 1)) != 0) blk = CHOL_NB;
-    return blk;
-}
+int gpirt_b200_sampler::bwd_block() const { return n >= 2048 ? 1024 : (n >= 1024 ? 512 : CHOL_NB); }
 // the split factor depends on the shape of the product's A operand only — never on the number of right-hand sides, i.e.
 // on how many ranks share the grid columns: a sharded run stays bit-identical to the unsharded one
 GemmArgs gpirt_b200_sampler::thin(GemmArgs a) const {
-    static const bool off = getenv("GPIRT_SPLITK") && atoi(getenv("GPIRT_SPLITK")) == 0;
-    if (!off && splitk_ws && a.K >= 512 && a.M <= 4096) {
+    if (splitk_ws && a.K >= 512 && a.M <= 4096) {
         a.splitk = (int)std::min<int64_t>(8, a.K / 128);
         a.ws = splitk_ws;
         a.ws_count = splitk_count;
@@ -643,31 +633,23 @@ int gpirt_b200_sampler::gather_solves(cudaStream_t st) {
     return GPIRT_B200_OK;
 }
 
+// With items sharded over GPUs this part would be replicated: instead every rank solves for its slice of the 1001 grid
+// columns and the slices are all-gathered (n x 1001 doubles) — through L^-1 the caller passes the main stream then
 int gpirt_b200_sampler::fstar_solves(cudaStream_t st) {
-    const int N = N_GRID;
-    if (solve_mode == 1) {
-        Seg a = tic_on(GPIRT_B200_T_KSTAR, st);
-        GP_TRY(trsm_kstar(st));
-        toc_on(a, st);
-        Seg b = tic_on(GPIRT_B200_T_TRSM, st);
+    Seg a = tic_on(GPIRT_B200_T_KSTAR, st);
+    GP_TRY(trsm_kstar(st));
+    toc_on(a, st);
+    Seg b = tic_on(GPIRT_B200_T_TRSM, st);
+    int c0, nc;
+    grid_slice(c0, nc);
+    double* Kc = kstar + (int64_t)c0 * ldn;
+    double* K2c = kstar2 + (int64_t)c0 * ldn;
+    if (route == Route::SUBST) {
         const int nblk = (int)ceil_div(n, CHOL_NB);
         for (int k = 0; k < nblk; ++k) GP_TRY(trsm_fwd_step(st, k));
         GP_TRY(trsm_bwd(st));
-        GP_TRY(gather_solves(st));
-        toc_on(b, st);
-        return GPIRT_B200_OK;
-    }
-    // with items sharded over GPUs this part would be replicated: instead every rank solves for its slice of the 1001
-    // grid columns and the slices are all-gathered (n x 1001 doubles) — the caller passes the main stream then
-    const int per = (int)ceil_div(N, comm.world), c0 = min(N, comm.rank * per), nc = min(N, c0 + per) - c0;
-    Seg a = tic_on(GPIRT_B200_T_KSTAR, st);
-    GP_TRY(launch_se_cov(st, theta, n, theta_star + c0, nc, 0.0, false, kstar + (int64_t)c0 * ldn, ldn));   // :17
-    toc_on(a, st);
-    Seg b = tic_on(GPIRT_B200_T_TRSM, st);
-    if (nc > 0 && use_i8gemm) {
+    } else if (nc > 0 && use_i8gemm) {
         // the two triangular products with L^-1 in fixed point as well (L^-1 has zeros above the diagonal: trtri_lower)
-        double* Kc = kstar + (int64_t)c0 * ldn;
-        double* K2c = kstar2 + (int64_t)c0 * ldn;
         GP_TRY(dp_Linv.slice_mcontig(st, Linv, ldn, true, 0, n, INT_MIN));
         GP_TRY(dp_LinvT.slice_kcontig(st, Linv, ldn));
         GP_TRY(dp_K.slice_kcontig(st, Kc, ldn));
@@ -676,15 +658,11 @@ int gpirt_b200_sampler::fstar_solves(cudaStream_t st) {
         GP_TRY(dp_K.slice_kcontig(st, K2c, ldn));
         GP_TRY(dgemm_i8(st, dp_LinvT, dp_K, Kc, ldn, DG_TRI_UPPER, 0, n, false, 0));
     } else if (nc > 0) {
-        GP_TRY(gemm_f64(st, false, false, G(n, nc, n, Linv, ldn, kstar + (int64_t)c0 * ldn, ldn, kstar2 + (int64_t)c0 * ldn, ldn, 1.0, 0.0, TRI_A_LOWER)));   // :19
-        GP_TRY(launch_fstar_sd(st, kstar2 + (int64_t)c0 * ldn, ldn, n, nc, s + c0));           // :20
-        GP_TRY(gemm_f64(st, true, false, G(n, nc, n, Linv, ldn, kstar2 + (int64_t)c0 * ldn, ldn, kstar + (int64_t)c0 * ldn, ldn, 1.0, 0.0, TRI_A_UPPER)));
+        GP_TRY(gemm_f64(st, false, false, G(n, nc, n, Linv, ldn, Kc, ldn, K2c, ldn, 1.0, 0.0, TRI_A_LOWER)));   // :19
+        GP_TRY(launch_fstar_sd(st, K2c, ldn, n, nc, s + c0));                                                   // :20
+        GP_TRY(gemm_f64(st, true, false, G(n, nc, n, Linv, ldn, K2c, ldn, Kc, ldn, 1.0, 0.0, TRI_A_UPPER)));
     }
-    if (comm.world > 1) {
-        GP_TRY(comm_allgather_f64(comm, kstar, (size_t)per * ldn, st));
-        GP_TRY(comm_allgather_f64(comm, s, (size_t)per, st));
-    }
-    if (use_i8gemm) GP_TRY(dp_A.slice_kcontig(st, kstar, ldn));   // row k of A^T = column k of S^-1 K*
+    GP_TRY(gather_solves(st));
     toc_on(b, st);
     return GPIRT_B200_OK;
 }
@@ -693,16 +671,15 @@ int gpirt_b200_sampler::fstar_solves(cudaStream_t st) {
 int gpirt_b200_sampler::step_draw_fstar(uint32_t sweep, int accumulate) {
     const RngKey k = key_at(sweep);
     const int N = N_GRID;
-    if (opts.fstar_mode == 0) {
-        if (solve_ready) GP_CUDA(cudaStreamWaitEvent(stream, ev_solve, 0));   // done under the previous sweep's tail / this sweep's ESS
-        else if (local_solve_ready) {   // this rank's slice was solved behind the factorisation: gather it now
+    if (route != Route::LITERAL) {
+        if (carry.solved == Carry::Solved::ALL) GP_CUDA(cudaStreamWaitEvent(stream, ev_solve, 0));   // done under the previous sweep's tail / this sweep's ESS
+        else if (carry.solved == Carry::Solved::LOCAL) {   // this rank's slice was solved behind the factorisation: gather it now
             GP_CUDA(cudaStreamWaitEvent(stream, ev_solve, 0));
             tic(GPIRT_B200_T_TRSM);
             GP_TRY(gather_solves(stream));
             toc();
         } else GP_TRY(fstar_solves(stream));
-        solve_ready = false;
-        local_solve_ready = false;
+        carry.solved = Carry::Solved::NONE;
         tic(GPIRT_B200_T_FSTAR_GEMM);
         if (use_i8gemm) {
             GP_TRY(dp_B.slice_kcontig(stream, f, ldn));
@@ -712,8 +689,6 @@ int gpirt_b200_sampler::step_draw_fstar(uint32_t sweep, int accumulate) {
         }
         toc();
     } else {
-        solve_ready = false;
-        local_solve_ready = false;
         tic(GPIRT_B200_T_KSTAR);
         GP_TRY(launch_se_cov(stream, theta, n, theta_star, N, 0.0, false, kstar, ldn));          // :17
         toc();
@@ -799,9 +774,9 @@ int gpirt_b200_sampler::ess_only(uint32_t sweep) {
     // queue is empty), so that the short kernels of the pass get SMs as item CTAs retire
     // and one notch below the pass in priority: an item CTA takes the whole register file of its SM, and at equal priority
     // the block scheduler drains the grid that was launched first — the pass would start when the ESS has ended
-    int* queue = tail_beside_ess ? nullptr : work;
-    LaunchPriority yield(tail_beside_ess ? prio_second : INT_MIN);
-    tail_beside_ess = false;
+    int* queue = carry.ess_yields ? nullptr : work;
+    LaunchPriority yield(carry.ess_yields ? prio_second : INT_MIN);
+    carry.ess_yields = false;
     GP_TRY(launch_ess(stream, f, nu, ldn, y8, ldy8, theta, beta, n, m, key_at(sweep), item_offset, nprop, status + 1, queue, &ess_shape));
     toc();
     return GPIRT_B200_OK;
@@ -812,9 +787,6 @@ int gpirt_b200_sampler::ess_only(uint32_t sweep) {
 //   stream  : K(theta,theta)+1e-3 I, right-looking Cholesky chain (+ its bulk stream), L^-1
 //   st_lz   : after every lz_group finished block columns  nu[r0:, :] (+)= L[r0:, r0:r1] Z[r0:r1, :]
 int gpirt_b200_sampler::rebuild_pipelined(uint32_t sweep, uint32_t next_sweep) {
-    const int mask = pipe_mask;
-    cudaStream_t st_beta = (mask & 2) ? this->st_beta : stream;
-    cudaStream_t st_lz = (mask & 1) ? this->st_lz : stream;
     GP_CUDA(cudaEventRecord(ev_theta, stream));
     GP_CUDA(cudaStreamWaitEvent(st_beta, ev_theta, 0));
     {
@@ -835,8 +807,8 @@ int gpirt_b200_sampler::rebuild_pipelined(uint32_t sweep, uint32_t next_sweep) {
     tic(GPIRT_B200_T_KBUILD);
     GP_TRY(launch_se_cov(stream, theta, n, theta, n, 0.001, true, L, ldn));
     toc();
-    const bool trsm_route = solve_mode == 1 && opts.fstar_mode == 0;
-    if (trsm_route) {   // K* for this rank's grid columns as soon as theta is known
+    const bool subst = route == Route::SUBST;
+    if (subst) {   // K* for this rank's grid columns as soon as theta is known
         GP_CUDA(cudaStreamWaitEvent(st_trsm, ev_theta, 0));
         Seg a = tic_on(GPIRT_B200_T_KSTAR, st_trsm);
         GP_TRY(trsm_kstar(st_trsm));
@@ -852,16 +824,15 @@ int gpirt_b200_sampler::rebuild_pipelined(uint32_t sweep, uint32_t next_sweep) {
     // The schedule may depend on the route but never on the sharding itself: the slices are added in FP64, so their
     // boundaries are part of the rounding of nu, and a sharded run must reproduce the unsharded one bit for bit.
     const int nblk_all = (int)ceil_div(n, CHOL_NB);
-    static const bool lz_forced = getenv("GPIRT_LZ_GROUP") != nullptr;   // developer override: slices of lz_group panels on every route
     auto next_end = [&](int e) {
-        if (lz_forced || !use_i8gemm || !trsm_route) return min(nblk_all, e + lz_group);
+        if (!use_i8gemm || !subst) return min(nblk_all, e + lz_group);
         if (e < nblk_all / 2) return max(1, nblk_all / 2);
         const int tail_start = nblk_all - max(1, nblk_all / 8);
         return e < tail_start ? tail_start : nblk_all;
     };
     int lz_slice = 0, lz_prev_end = 0, lz_next_end = next_end(0);
     lookahead.after_panel = [&](int k, int nblk, cudaEvent_t done) -> int {
-        if (trsm_route) {   // forward substitution step k trails panel k
+        if (subst) {   // forward substitution step k trails panel k
             GP_CUDA(cudaStreamWaitEvent(st_trsm, done, 0));
             Seg sg = tic_on(GPIRT_B200_T_TRSM, st_trsm);
             GP_TRY(trsm_fwd_step(st_trsm, k));
@@ -901,27 +872,28 @@ int gpirt_b200_sampler::rebuild_pipelined(uint32_t sweep, uint32_t next_sweep) {
     lookahead.after_panel = nullptr;
     GP_TRY(rc);
     toc();
-    if (!trsm_route) {
+    if (!subst) {
         tic(GPIRT_B200_T_TRTRI);
         GP_TRY(trtri_lower(stream, L, ldn, n, Dinv, ldn, Linv, ldn, Tmp, ldn));
         toc();
     } else {   // the forward steps join here; the backward substitution starts with the next sweep, beside its ESS
         GP_CUDA(cudaEventRecord(ev_fwd, st_trsm));
         GP_CUDA(cudaStreamWaitEvent(stream, ev_fwd, 0));
-        deferred = 1;
     }
     GP_CUDA(cudaStreamWaitEvent(stream, ev_lz, 0));
     GP_CUDA(cudaStreamWaitEvent(stream, ev_beta, 0));
-    nu_ready = true;
-    nu_sweep = next_sweep;
-    if (opts.fstar_mode == 0 && comm.world <= 1 && !trsm_route) deferred = 2;   // K* solves through L^-1, beside the next ESS
+    carry.nu_ready = true;
+    carry.nu_sweep = next_sweep;
+    // sharded, the solves through L^-1 run in the next sweep's draw_fstar: all ranks gather their slices there
+    carry.start = subst ? Carry::Start::BWD
+                : (route == Route::LINV && comm.world <= 1) ? Carry::Start::LINV_SOLVES : Carry::Start::NONE;
     return GPIRT_B200_OK;
 }
 
 int gpirt_b200_sampler::launch_deferred_solves() {
-    const int what = deferred;
-    deferred = 0;
-    if (what == 1) {
+    const Carry::Start what = carry.start;
+    carry.start = Carry::Start::NONE;
+    if (what == Carry::Start::BWD) {
         // on the factorisation's bulk stream (idle now, same top priority as the ESS on the main stream: on the trailing
         // stream, one notch lower, the first kernel of the pass did not get an SM before the ESS had dispatched all of its
         // CTAs — 0.37 ms into the sweep on 4 GPUs)
@@ -932,15 +904,14 @@ int gpirt_b200_sampler::launch_deferred_solves() {
         GP_TRY(trsm_bwd(st_tail, true));
         toc_on(sg, st_tail);
         GP_CUDA(cudaEventRecord(ev_solve, st_tail));
-        local_solve_ready = true;
-        tail_beside_ess = true;
-    } else if (what == 2) {
-        cudaStream_t st_solve = (pipe_mask & 4) ? st_lz : stream;
+        carry.solved = Carry::Solved::LOCAL;
+        carry.ess_yields = true;
+    } else if (what == Carry::Start::LINV_SOLVES) {
         GP_CUDA(cudaEventRecord(ev_linv, stream));
-        GP_CUDA(cudaStreamWaitEvent(st_solve, ev_linv, 0));
-        GP_TRY(fstar_solves(st_solve));
-        GP_CUDA(cudaEventRecord(ev_solve, st_solve));
-        solve_ready = true;
+        GP_CUDA(cudaStreamWaitEvent(st_lz, ev_linv, 0));
+        GP_TRY(fstar_solves(st_lz));
+        GP_CUDA(cudaEventRecord(ev_solve, st_lz));
+        carry.solved = Carry::Solved::ALL;
     }
     return GPIRT_B200_OK;
 }
@@ -949,10 +920,10 @@ __global__ void k_bump_sweep(uint32_t* sweep) { *sweep += 1u; }
 
 int gpirt_b200_sampler::sweep_eager(uint32_t t, int accumulate) {
     const bool can_pipe = pipeline && ceil_div(n, CHOL_NB) > 2;   // the look-ahead factorisation needs > 2 panels
-    if (deferred) GP_TRY(launch_deferred_solves());
-    if (can_pipe && nu_ready && nu_sweep == t) GP_TRY(ess_only(t));
-    else { tail_beside_ess = false; GP_TRY(step_draw_f(t)); }
-    nu_ready = false;
+    GP_TRY(launch_deferred_solves());
+    if (can_pipe && carry.nu_ready && carry.nu_sweep == t) GP_TRY(ess_only(t));
+    else { carry.ess_yields = false; GP_TRY(step_draw_f(t)); }
+    carry.nu_ready = false;
     GP_TRY(step_draw_fstar(t, accumulate));
     GP_TRY(step_draw_theta(t));
     if (can_pipe) return rebuild_pipelined(t, t + 1);
@@ -980,8 +951,8 @@ int gpirt_b200_sampler::sweep_graph(uint32_t t, int accumulate) {
             GP_LAUNCH(k_bump_sweep, 1, 1, 0, stream, d_sweep);
             rc = sweep_eager(t, accumulate);
             e = cudaStreamEndCapture(stream, &graph);
-            graph_pipelined = pipeline && ceil_div(n, CHOL_NB) > 2;
-            graph_deferred = deferred;
+            graph_carry[a] = carry;
+            graph_carry[a].nu_sweep -= t;
         }
         capturing = false;
         g_launch_count = counted;
@@ -1002,11 +973,8 @@ int gpirt_b200_sampler::sweep_graph(uint32_t t, int accumulate) {
     g_launch_count += graph_kernels;   // the kernels inside the graph still launch
     graph_replays += 1;
     d_sweep_value = t;
-    if (graph_pipelined) {             // the host-side state a pipelined sweep leaves behind
-        nu_ready = true; nu_sweep = t + 1;
-        deferred = graph_deferred;
-        solve_ready = local_solve_ready = false;
-    }
+    carry = graph_carry[a];            // the host-side state the sweep leaves behind
+    carry.nu_sweep += t;
     return GPIRT_B200_OK;
 }
 
@@ -1016,8 +984,8 @@ int gpirt_b200_sampler::sweep(int accumulate) {
     // graph replay without per-step timers, after one eager sweep has done every lazy first-use initialisation (function
     // attributes, occupancy queries, the softplus table); the pipelined sweep only in its steady state (proposals and
     // solves prepared by the previous sweep), which is the state the captured launch sequence assumes
-    const bool steady = !can_pipe || (nu_ready && nu_sweep == t && deferred != 0);
-    if (graph_enabled && !timing && warmed && opts.fstar_mode == 0 && steady) return sweep_graph(t, accumulate);
+    const bool steady = !can_pipe || (carry.nu_ready && carry.nu_sweep == t && carry.start != Carry::Start::NONE);
+    if (graph_enabled && !timing && warmed && route != Route::LITERAL && steady) return sweep_graph(t, accumulate);
     const int64_t before = g_launch_count;
     GP_TRY(sweep_eager(t, accumulate));
     graph_kernels = g_launch_count - before;
@@ -1257,9 +1225,7 @@ int gpirt_b200_sampler_sweep(gpirt_b200_sampler* s, int n_sweeps, int accumulate
 
 int gpirt_b200_sampler_step(gpirt_b200_sampler* s, int step, uint32_t sweep) {
     if (!s) return GPIRT_B200_ERR_ARG;
-    s->nu_ready = false;
-    s->deferred = 0;
-    if (s->solve_ready || s->local_solve_ready) { cudaStreamWaitEvent(s->stream, s->ev_solve, 0); s->solve_ready = s->local_solve_ready = false; }
+    s->drop_carry();
     int rc;
     switch (step) {
         case GPIRT_B200_STEP_DRAW_F: rc = s->step_draw_f(sweep); break;
@@ -1322,9 +1288,7 @@ int gpirt_b200_sampler_set(gpirt_b200_sampler* s, int field, const double* host_
     if (!s || !host_in) return GPIRT_B200_ERR_ARG;
     double* dev; int64_t ld; int rows, cols;
     if (field_shape(s, field, &dev, &ld, &rows, &cols)) return GPIRT_B200_ERR_ARG;
-    s->nu_ready = false;
-    s->deferred = 0;
-    if (s->solve_ready || s->local_solve_ready) { cudaStreamWaitEvent(s->stream, s->ev_solve, 0); s->solve_ready = s->local_solve_ready = false; }
+    s->drop_carry();
     GP_TRY(upload_padded(dev, ld, host_in, rows, cols, s->stream));
     GP_CUDA(cudaStreamSynchronize(s->stream));
     return GPIRT_B200_OK;
@@ -1350,9 +1314,7 @@ int gpirt_b200_sampler_set_pipeline(gpirt_b200_sampler* s, int enabled) {
     if (!s) return GPIRT_B200_ERR_ARG;
     s->pipeline = enabled != 0;
     s->drop_graphs();
-    s->nu_ready = false;
-    s->deferred = 0;
-    if (s->solve_ready || s->local_solve_ready) { cudaStreamWaitEvent(s->stream, s->ev_solve, 0); s->solve_ready = s->local_solve_ready = false; }
+    s->drop_carry();
     return GPIRT_B200_OK;
 }
 
@@ -1362,9 +1324,7 @@ int gpirt_b200_sampler_set_pipeline(gpirt_b200_sampler* s, int enabled) {
 int gpirt_b200_sampler_time_factorisation(gpirt_b200_sampler* s, int reps, int as_graph, float* ms_per_rep) {
     if (!s || reps <= 0 || !ms_per_rep) return GPIRT_B200_ERR_ARG;
     GP_TRY(s->check_status());                              // drains every stream of the sampler
-    s->nu_ready = false;
-    s->deferred = 0;
-    s->solve_ready = s->local_solve_ready = false;
+    s->drop_carry();
     const bool timing_was = s->timing;
     s->timing = false;
     struct Restore { gpirt_b200_sampler* s; bool t; ~Restore() { s->timing = t; } } restore{s, timing_was};
@@ -1415,7 +1375,7 @@ int gpirt_b200_sampler_uses(gpirt_b200_sampler* s, int feature) {
     if (feature == 1) return s->use_i8gemm ? 1 : 0;
     if (feature == 2) return s->ess_shape;
     if (feature == 3) return s->beta_shape;
-    if (feature == 4) return s->solve_mode;
+    if (feature == 4) return s->route == gpirt_b200_sampler::Route::SUBST ? 1 : 0;
     if (feature == 5) return (int)std::min<int64_t>(s->graph_replays, INT_MAX);
     return -1;
 }

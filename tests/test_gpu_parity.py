@@ -382,34 +382,62 @@ def test_chain_blocked_substitution_solves_match_inverse_route(G, O, n, m, monke
         assert np.max(np.abs(a["IRFs"] - want["IRFs"])) <= 1e-7
 
 
-@pytest.mark.parametrize("n,m,route", [(100, 60, "0"), (640, 300, "0"), (640, 300, "1"), (1152, 260, "1"),
-                                        pytest.param(9000, 300, None, id="9000-300-default")])
-def test_graph_replayed_sweeps_equal_eager_sweeps(G, n, m, route, monkeypatch):
+# calls that change or re-time the sampler's state between sweeps: each drops what a pipelined sweep leaves for the next
+_INTERRUPTS = {
+    "set": lambda s, lib: s.set(lib.BETA, s.get(lib.BETA)),
+    "step": lambda s, lib: s.step(lib.STEP_REBUILD, 0),
+    "set_pipeline": lambda s, lib: s.set_pipeline(True),
+    "time_factorisation": lambda s, lib: s.time_factorisation(1),
+}
+
+
+@pytest.mark.parametrize("n,m,route,interrupt",
+                         [pytest.param(100, 60, "0", None, id="100-60-0"), pytest.param(640, 300, "0", None, id="640-300-0")]
+                         + [pytest.param(640, 300, "0", i, id="640-300-0-" + i) for i in _INTERRUPTS]
+                         + [pytest.param(640, 300, "1", None, id="640-300-1"), pytest.param(1152, 260, "1", None, id="1152-260-1")]
+                         + [pytest.param(1152, 260, "1", i, id="1152-260-1-" + i) for i in _INTERRUPTS]
+                         + [pytest.param(9000, 300, None, None, id="9000-300-default")])
+def test_graph_replayed_sweeps_equal_eager_sweeps(G, n, m, route, interrupt, monkeypatch):
     """With the per-step timers off every sweep after the first is ONE CUDA-graph launch — captured from the very launch
     sequence of the eager sweep, for n > 256 the pipelined one with its five streams forked and joined inside the graph
     (stream priorities carried as per-node launch attributes).  Same kernels, same addressed RNG: the state after 6 sweeps
-    must be bit-identical to 6 eager sweeps, on both K*-solve routes (route None: the default, substitution for n > 6144)."""
+    must be bit-identical to 6 eager sweeps, on both K*-solve routes (route None: the default, substitution for n > 6144).
+    With `interrupt`, both samplers make that call after the 4th sweep: the chain must resume — as a graph replay on the
+    graph sampler — and agree with a chain that had no call (nu is then formed in one product instead of in slices)."""
     from gpirt_b200 import _lib
     if route is None:
         monkeypatch.delenv("GPIRT_SOLVE_MODE", raising=False)
     else:
         monkeypatch.setenv("GPIRT_SOLVE_MODE", route)
     prob = make_problem(n, m, seed=n + 3, missing=0.03)
-    state = {}
-    for use_graph in (0, -1):
+
+    def run(use_graph, call):
         s = G.Sampler(prob["y"], prob["theta"], prob["pm"], prob["psd"], prob["pstep"], seed=77, use_graph=use_graph)
         s.set_timing(False)
         s.init_draws()
         s.sweep(4)
+        if call is not None:
+            _INTERRUPTS[call](s, _lib)
+        at_call = s.uses(5)
         s.sweep(2, accumulate_irf=True)
         assert s.uses(4) == (1 if route is None else int(route))
         replays = s.uses(5)
         assert (replays >= 4) if use_graph == 0 else (replays == 0), "graph replay must be the path that ran (or not)"
-        state[use_graph] = {k: s.get(f) for k, f in (("theta", _lib.THETA), ("beta", _lib.BETA), ("f", _lib.F), ("fstar", _lib.FSTAR),
-                                                      ("irf", _lib.IRF_SUM), ("L", _lib.CHOL))}
+        if use_graph == 0 and call is not None:
+            assert replays > at_call, "graph replay must resume after the call"
+        out = {k: s.get(f) for k, f in (("theta", _lib.THETA), ("beta", _lib.BETA), ("f", _lib.F), ("fstar", _lib.FSTAR),
+                                        ("irf", _lib.IRF_SUM), ("L", _lib.CHOL))}
         s.close()
+        return out
+
+    state = {use_graph: run(use_graph, interrupt) for use_graph in (0, -1)}
     for k in state[0]:
         assert np.array_equal(state[0][k], state[-1][k]), k
+    if interrupt is not None:
+        plain = run(0, None)
+        assert np.array_equal(state[0]["theta"], plain["theta"])
+        assert np.max(np.abs(state[0]["beta"] - plain["beta"])) <= 1e-10
+        assert np.max(np.abs(state[0]["f"] - plain["f"])) <= 1e-9
 
 
 def test_senate116_short_chain(G, O):
