@@ -370,6 +370,54 @@ int gpirt_b200_predictive_accumulate_time(int64_t n, int64_t m, int reps, double
     return GPIRT_B200_OK;
 }
 
+int gpirt_b200_irf_bands(const double* draws, int64_t cols, int64_t S, double band, double* lower, double* upper, int reps,
+                         double* ms) {
+    if (!draws || !lower || !upper || cols <= 0 || cols > INT_MAX || S <= 0 || S > INT_MAX || !std::isfinite(band) || !(band > 0.0 && band < 1.0) ||
+        reps < 0 || (reps > 0 && !ms)) {
+        set_last_error("bad argument: irf_bands needs draws, 1 <= cols <= INT_MAX, 1 <= S <= INT_MAX, 0 < band < 1, outputs, reps >= 0");
+        return GPIRT_B200_ERR_ARG;
+    }
+    GP_TRY(have_device());
+    const IrfBandPlan plan = irf_band_plan((int)S, band);
+    DevBuf x, acc, lo, hi, out;
+    GP_TRY(x.alloc((size_t)cols * S)); GP_TRY(acc.alloc(2 * (size_t)cols));
+    GP_TRY(lo.alloc((size_t)cols * plan.klo)); GP_TRY(hi.alloc((size_t)cols * plan.khi)); GP_TRY(out.alloc(2 * (size_t)cols));
+    GP_CUDA(cudaMemcpy(x.p, draws, (size_t)cols * S * sizeof(double), cudaMemcpyHostToDevice));
+    cudaEvent_t e[3];
+    for (auto& v : e) GP_CUDA(cudaEventCreate(&v));
+    int rc = GPIRT_B200_OK;
+    float t_upd = 0.f, t_fin = 0.f;
+    for (int pass = 0; pass < std::max(reps, 1) && rc == GPIRT_B200_OK; ++pass) {   // every pass starts the stream afresh
+        cudaEventRecord(e[0], 0);
+        for (int64_t s = 0; s < S && rc == GPIRT_B200_OK; ++s)
+            rc = launch_irf_accumulate(0, x.p + (size_t)s * cols, cols, (int)cols, cols, (int)s + 1,
+                                       acc.p, acc.p + cols, lo.p, plan.klo, hi.p, plan.khi);
+        cudaEventRecord(e[1], 0);
+        if (rc == GPIRT_B200_OK)
+            rc = launch_irf_finish_bands(0, cols, (int)S, acc.p + cols, nullptr, lo.p, hi.p, plan, false, out.p, out.p + cols);
+        cudaEventRecord(e[2], 0);
+        if (rc == GPIRT_B200_OK && cudaEventSynchronize(e[2]) != cudaSuccess) {
+            set_last_error("irf band computation failed: %s", cudaGetErrorString(cudaGetLastError()));
+            rc = GPIRT_B200_ERR_CUDA;
+        }
+        if (rc == GPIRT_B200_OK) {
+            float a = 0.f, b = 0.f;
+            cudaEventElapsedTime(&a, e[0], e[1]);
+            cudaEventElapsedTime(&b, e[1], e[2]);
+            t_upd += a; t_fin += b;
+        }
+    }
+    for (auto& v : e) cudaEventDestroy(v);
+    if (rc) return rc;
+    GP_CUDA(cudaMemcpy(lower, out.p, (size_t)cols * sizeof(double), cudaMemcpyDeviceToHost));
+    GP_CUDA(cudaMemcpy(upper, out.p + cols, (size_t)cols * sizeof(double), cudaMemcpyDeviceToHost));
+    if (reps > 0) {
+        ms[0] = t_upd / ((double)reps * (double)S);
+        ms[1] = t_fin / reps;
+    }
+    return GPIRT_B200_OK;
+}
+
 int gpirt_b200_rng_probe(uint64_t seed, uint32_t sweep, uint32_t purpose, uint32_t stream, uint32_t idx0, int count,
                          double* uniforms, double* normals) {
     if (count < 0 || !uniforms || !normals) return GPIRT_B200_ERR_ARG;

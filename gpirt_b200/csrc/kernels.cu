@@ -1,5 +1,7 @@
 // Non-GEMM kernels of the Gibbs sweep: covariance builder, response ingest, Philox fills, the batched elliptical
 // slice sampler with the fused logistic log-likelihood, f* finishing draw, theta grid sampler, beta Metropolis step.
+#include <algorithm>
+#include <cmath>
 #include <map>
 #include <mutex>
 #include <tuple>
@@ -1112,6 +1114,134 @@ int launch_predictive_reduce(cudaStream_t st, const double* acc, int64_t ld, con
     GP_LAUNCH(k_predictive_resp, grid, 128, 0, st, acc, ld, plane, code, ldc, n, m, S, partial, n_chunks);
     GP_LAUNCH(k_reduce_partials, (unsigned)ceil_div(n, 128), 128, 0, st, partial, n, n_chunks, resp_totals);
     GP_LAUNCH(k_predictive_totals, (unsigned)PRED_STATS, 256, 0, st, stats, m, resp_totals + n);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------------
+// IRF posterior summaries (opts.irf).  One thread per grid cell, cells contiguous in k.  Per draw: the Welford mean / M2
+// of P = plogis(f*) and two bounded heaps per cell that end up holding exactly the order statistics the bands need — a
+// max-heap of the K_lo smallest f* and a min-heap of the K_hi largest, stored slot-major so that a warp's root reads are
+// one coalesced load.  Once a heap is full most draws only compare against its root; the rare insertion sifts down.
+// ------------------------------------------------------------------------------------------------------------------
+IrfBandPlan irf_band_plan(int S, double band) {
+    IrfBandPlan p;
+    if (S <= 0) return p;
+    const double q_lo = (1.0 - band) / 2.0, q_hi = (1.0 + band) / 2.0;
+    const double h_lo = (double)(S - 1) * q_lo, h_hi = (double)(S - 1) * q_hi;
+    const int r_lo = std::min(S - 1, (int)std::floor(h_lo)), r_hi = std::min(S - 1, (int)std::floor(h_hi));
+    p.tlo = h_lo - (double)r_lo;
+    p.thi = h_hi - (double)r_hi;
+    p.lo_last = r_lo == S - 1;
+    p.hi_last = r_hi == S - 1;
+    p.klo = std::min(S, r_lo + 2);
+    p.khi = S - r_hi;
+    return p;
+}
+
+// MAXH: max-heap (root = largest kept value); `above(a, b)`: a belongs nearer the root than b
+template <bool MAXH>
+__device__ __forceinline__ bool heap_above(double a, double b) { return MAXH ? a > b : a < b; }
+// adds v to the heap of cell c, which holds `size` values (capacity K): while not full every value goes in (sift up);
+// once full v replaces the root only if it belongs strictly below it in the kept tail (sift down)
+template <bool MAXH>
+__device__ __forceinline__ void heap_add(double* h, int64_t cells, int64_t c, int K, int size, double v) {
+    auto at = [&](int i) -> double& { return h[(int64_t)i * cells + c]; };
+    if (size < K) {
+        int i = size;
+        while (i > 0) {
+            const int p = (i - 1) >> 1;
+            const double pv = at(p);
+            if (!heap_above<MAXH>(v, pv)) break;
+            at(i) = pv;
+            i = p;
+        }
+        at(i) = v;
+        return;
+    }
+    if (!heap_above<MAXH>(at(0), v)) return;   // v is not inside the kept tail (ties keep the value already there)
+    int i = 0;
+    for (;;) {
+        const int l = 2 * i + 1;
+        if (l >= K) break;
+        int ci = l;
+        double cv = at(l);
+        if (l + 1 < K) {
+            const double rv = at(l + 1);
+            if (heap_above<MAXH>(rv, cv)) { ci = l + 1; cv = rv; }
+        }
+        if (!heap_above<MAXH>(cv, v)) break;
+        at(i) = cv;
+        i = ci;
+    }
+    at(i) = v;
+}
+
+__global__ void __launch_bounds__(256) k_irf_accumulate(const double* __restrict__ x, int64_t ld, int rows, int64_t cells,
+                                                        int s, double* __restrict__ mean, double* __restrict__ m2,
+                                                        double* __restrict__ lo, int klo, double* __restrict__ hi, int khi) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= cells) return;
+    const int64_t j = c / rows, k = c - j * rows;
+    const double v = x[k + j * ld];
+    const double p = 1.0 / (1.0 + exp(-v));                    // as k_irf_finish
+    if (s == 1) {                                              // first draw: no memset of the accumulators
+        mean[c] = p;
+        m2[c] = 0.0;
+    } else {
+        const double mu = mean[c], d = p - mu, mu2 = mu + d / (double)s;
+        mean[c] = mu2;
+        m2[c] = fma(d, p - mu2, m2[c]);
+    }
+    if (klo > 0) {
+        heap_add<true>(lo, cells, c, klo, min(s - 1, klo), v);
+        heap_add<false>(hi, cells, c, khi, min(s - 1, khi), v);
+    }
+}
+int launch_irf_accumulate(cudaStream_t st, const double* x, int64_t ld, int rows, int64_t cells, int s, double* mean,
+                          double* m2, double* lo, int klo, double* hi, int khi) {
+    if (cells <= 0) return GPIRT_B200_OK;
+    GP_LAUNCH(k_irf_accumulate, (unsigned)ceil_div(cells, 256), 256, 0, st, x, ld, rows, cells, s, mean, m2, lo, klo, hi, khi);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+
+// type-7 quantile from the two order statistics next to it, without contraction (a numpy reference matches it bit for bit)
+__device__ __forceinline__ double irf_lerp(double x0, double x1, double t) { return __dadd_rn(x0, __dmul_rn(t, __dsub_rn(x1, x0))); }
+// lower, upper and sd_out may alias the inputs of their own cell (each thread reads its cell before it writes it)
+__global__ void __launch_bounds__(256) k_irf_finish_bands(int64_t cells, double S, const double* m2, double* sd_out,
+                                                          const double* lo, const double* hi, int klo, int khi, int lo_last,
+                                                          int hi_last, double tlo, double thi, int plogis, double* lower,
+                                                          double* upper) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= cells) return;
+    if (sd_out) sd_out[c] = sqrt(m2[c] / (S - 1.0));          // S = 1: 0 / 0 = NaN, as R's sd() of one value
+    if (!lo) return;
+    // lo: max-heap of x_(0..r_lo+1): root = x_(r_lo+1), the larger child = x_(r_lo); hi: min-heap of x_(r_hi..S-1)
+    const double l0 = lo[c], h0 = hi[c];
+    double ql = l0, qh = h0;
+    if (!lo_last) {
+        const double l1 = lo[cells + c];
+        const double below = klo > 2 ? fmax(l1, lo[2 * cells + c]) : l1;
+        ql = irf_lerp(below, l0, tlo);
+    }
+    if (!hi_last) {
+        const double h1 = hi[cells + c];
+        const double above = khi > 2 ? fmin(h1, hi[2 * cells + c]) : h1;
+        qh = irf_lerp(h0, above, thi);
+    }
+    if (plogis) {
+        ql = 1.0 / (1.0 + exp(-ql));
+        qh = 1.0 / (1.0 + exp(-qh));
+    }
+    lower[c] = ql;
+    upper[c] = qh;
+}
+int launch_irf_finish_bands(cudaStream_t st, int64_t cells, int S, const double* m2, double* sd_out, const double* lo,
+                            const double* hi, const IrfBandPlan& p, bool plogis, double* lower, double* upper) {
+    if (cells <= 0 || S <= 0) return GPIRT_B200_OK;
+    GP_LAUNCH(k_irf_finish_bands, (unsigned)ceil_div(cells, 256), 256, 0, st, cells, (double)S, m2, sd_out, lo, hi, p.klo,
+              p.khi, (int)p.lo_last, (int)p.hi_last, p.tlo, p.thi, (int)plogis, lower, upper);
     GP_CUDA(cudaGetLastError());
     return GPIRT_B200_OK;
 }

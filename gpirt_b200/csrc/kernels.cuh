@@ -78,5 +78,24 @@ int launch_predictive_cells(cudaStream_t st, const double* acc, int64_t ld, cons
 int launch_predictive_reduce(cudaStream_t st, const double* acc, int64_t ld, const int8_t* code, int64_t ldc, int n, int m,
                              double S, double* stats, double* partial, int n_chunks, double* resp_totals);
 
+// ---- IRF posterior summaries (opts.irf, definitions in include/gpirt_b200.h) ----
+// Which order statistics a band at level `band` over S draws needs (type 7 quantiles at q_lo = (1 - b)/2, q_hi = (1 + b)/2)
+// and how many values per cell the two tail heaps keep: K_lo = r_lo + 2 (at most S) smallest, K_hi = S - r_hi largest.
+struct IrfBandPlan {
+    int klo = 0, khi = 0;
+    bool lo_last = false, hi_last = false;   // r = S - 1: Q = x_(S-1)
+    double tlo = 0.0, thi = 0.0;
+};
+IrfBandPlan irf_band_plan(int S, double band);
+// draw s (1-based) of `cells` grid cells, cell c = k + j rows read from x[k + j ld]: Welford mean / M2 of plogis(x) and,
+// with klo > 0, the tail heaps (slot-major: heap[slot * cells + c]; lo a max-heap of the klo smallest, hi a min-heap of
+// the khi largest)
+int launch_irf_accumulate(cudaStream_t st, const double* x, int64_t ld, int rows, int64_t cells, int s, double* mean,
+                          double* m2, double* lo, int klo, double* hi, int khi);
+// after S >= 1 draws: sd_out = sqrt(m2 / (S - 1)) (sd_out may be m2; NULL: skipped) and, with lo != NULL, the band ends
+// Q(q_lo) -> lower, Q(q_hi) -> upper (plogis applied if asked; lower may alias heap slot 0 of lo, upper of hi)
+int launch_irf_finish_bands(cudaStream_t st, int64_t cells, int S, const double* m2, double* sd_out, const double* lo,
+                            const double* hi, const IrfBandPlan& plan, bool plogis, double* lower, double* upper);
+
 
 }  // namespace gpirt

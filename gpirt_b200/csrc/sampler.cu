@@ -4,6 +4,7 @@
 #include <sys/mman.h>
 
 #include <cstdarg>
+#include <cmath>
 #include <algorithm>
 #include <atomic>
 #include <cstring>
@@ -1520,6 +1521,11 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
     double* f_sd_out = opts ? opts->f_sd_out : nullptr;
     const bool summarise_f = f_mean_out || f_sd_out;
     gpirt_b200_fit* const fit = opts ? opts->fit : nullptr;
+    gpirt_b200_irf* const irf = opts ? opts->irf : nullptr;
+    if (irf && (irf->lower || irf->upper) && !(std::isfinite(irf->band) && irf->band > 0.0 && irf->band < 1.0)) {
+        set_last_error("bad argument: the IRF band level must lie in (0, 1), got %g", irf->band);
+        return GPIRT_B200_ERR_ARG;
+    }
     const bool trace = getenv("GPIRT_TIMING") != nullptr;
     auto now = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; };
     g_last_degenerate_theta = 0;
@@ -1547,6 +1553,7 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         double* h_small[2]; cudaEvent_t ev_small[2];
         bool trace = false;
         double* pred_acc = nullptr; int8_t* pred_code = nullptr; double* pred_aux = nullptr;   // opts.fit
+        double* irf_buf = nullptr; double* snap_fs[2] = {nullptr, nullptr};                     // opts.irf
         ~Guard() {
             auto now = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; };
             const double t0 = now();
@@ -1557,6 +1564,8 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
             for (int i = 0; i < 2; ++i) { if (ev[i]) cudaEventDestroy(ev[i]); pool_free(snap_f[i], s->stream); pool_free(snap_small[i], s->stream); }
             pool_free(f_mean, s->stream); pool_free(f_m2, s->stream); pool_free(agree_dev, s->stream);
             pool_free(pred_acc, s->stream); pool_free(pred_code, s->stream); pool_free(pred_aux, s->stream);
+            for (int i = 0; i < 2; ++i) pool_free(snap_fs[i], s->stream);
+            if (irf_buf) { cudaStreamSynchronize(s->stream); cudaFree(irf_buf); }   // not the pool: GBs of tail buffers must not stay reserved after the call
             const double t2 = now();
             gpirt_b200_sampler_destroy(s);
             if (trace) fprintf(stderr, "gpirt_b200_mcmc: teardown worker/copy stream %.3fs, host + pool frees %.3fs, sampler %.3fs\n", t1 - t0, t2 - t1, now() - t2);
@@ -1632,6 +1641,61 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
             return GPIRT_B200_ERR_Y_VALUE;
         }
     }
+    // IRF summaries: the Welford mean / M2 of P (2 planes of 1001 x m) and the tail heaps (K_lo + K_hi planes) in one
+    // cudaMalloc, checked against the free device memory by arithmetic before the first sweep
+    const int64_t irf_cells = (int64_t)N_GRID * m;
+    const size_t irf_plane = (size_t)irf_cells;
+    double* const fs_out = irf ? irf->fstar_draws : nullptr;
+    const bool irf_bands = irf && (irf->lower || irf->upper) && sample_iterations > 0;
+    const IrfBandPlan irf_plan = irf_bands ? irf_band_plan(sample_iterations, irf->band) : IrfBandPlan{};
+    double *irf_lo = nullptr, *irf_hi = nullptr;
+    if (irf) {
+        irf->band_bytes = 0;
+        const double tail_bytes = 8.0 * (double)irf_cells * ((double)irf_plan.klo + (double)irf_plan.khi);
+        const double need = tail_bytes + 16.0 * (double)irf_cells;
+        size_t free_b = 0, total_b = 0;
+        GP_CUDA(cudaMemGetInfo(&free_b, &total_b));
+        if (need > (double)free_b) {   // memory the pool holds unused is free for this purpose: hand it back first
+            int dev = 0;
+            cudaMemPool_t pool;
+            GP_CUDA(cudaStreamSynchronize(s->stream));
+            GP_CUDA(cudaGetDevice(&dev));
+            GP_CUDA(cudaDeviceGetDefaultMemPool(&pool, dev));
+            GP_CUDA(cudaMemPoolTrimTo(pool, 0));
+            GP_CUDA(cudaMemGetInfo(&free_b, &total_b));
+        }
+        double short_all = need > (double)free_b ? 1.0 : 0.0;
+        if (sharded) {   // every rank refuses together, as for y_holdout
+            GP_CUDA(cudaMemcpyAsync(gd.agree_dev, &short_all, sizeof(double), cudaMemcpyHostToDevice, s->stream));
+            GP_TRY(comm_allreduce_sum_f64(s->comm, gd.agree_dev, 1, s->stream));
+            GP_CUDA(cudaMemcpyAsync(&short_all, gd.agree_dev, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+            GP_CUDA(cudaStreamSynchronize(s->stream));
+        }
+        if (short_all != 0.0) {
+            set_last_error("IRF bands at level %g over %d sampling iterations need %.0f bytes of device memory for their tail "
+                           "buffers (%.0f in all); %zu bytes are free on this device%s", irf->band, sample_iterations, tail_bytes,
+                           need, free_b, need > (double)free_b ? "" : " (another rank lacks them)");
+            return GPIRT_B200_ERR_NOMEM;
+        }
+        const cudaError_t e = cudaMalloc((void**)&gd.irf_buf, (size_t)need);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            gd.irf_buf = nullptr;
+            set_last_error("device allocation of %.0f bytes for the IRF summaries failed: %s", need, cudaGetErrorString(e));
+            return GPIRT_B200_ERR_NOMEM;
+        }
+        irf->band_bytes = (int64_t)tail_bytes;
+        if (irf_bands) {
+            irf_lo = gd.irf_buf + 2 * irf_plane;
+            irf_hi = irf_lo + (size_t)irf_plan.klo * irf_plane;
+        }
+        if (fs_out) {
+            for (int i = 0; i < 2; ++i) GP_TRY(pool_alloc((void**)&gd.snap_fs[i], irf_plane * sizeof(double), s->stream));
+            // pinned bounce buffers large enough for an f* plane now: the storage worker must never reallocate them while
+            // the other buffer's transfer is in flight (without pinned memory the plane goes by a plain copy)
+            g_bounce.ensure(std::max(keep_f ? nm : (size_t)0, irf_plane));
+        }
+    }
     double t_c = now();
     GP_TRY(s->init_draws());
     double t_d = now();
@@ -1642,6 +1706,9 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         GP_CUDA(cudaMemcpyAsync(gd.snap_small[b] + n, s->beta, 2 * (size_t)m * sizeof(double), cudaMemcpyDeviceToDevice, s->stream));
         if (keep_f)
             GP_CUDA(cudaMemcpy2DAsync(gd.snap_f[b], (size_t)n * sizeof(double), s->f, s->ldn * sizeof(double), (size_t)n * sizeof(double),
+                                      (size_t)m, cudaMemcpyDeviceToDevice, s->stream));
+        if (fs_out)
+            GP_CUDA(cudaMemcpy2DAsync(gd.snap_fs[b], N_GRID * sizeof(double), s->fstar, s->ldN * sizeof(double), N_GRID * sizeof(double),
                                       (size_t)m, cudaMemcpyDeviceToDevice, s->stream));
         GP_CUDA(cudaEventRecord(gd.ev[b], s->stream));
         return GPIRT_B200_OK;
@@ -1674,6 +1741,14 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         const double* small = gd.h_small[b];
         for (int64_t i = 0; i < n; ++i) theta_out[(size_t)i * n_slots + slot] = small[i];
         std::memcpy(beta_out + (size_t)slot * 2 * m, small + n, 2 * (size_t)m * sizeof(double));
+        if (fs_out) {   // the f* plane after this slot's f slice, through the same bounce buffer (its DMA has landed)
+            double* dst = fs_out + (size_t)slot * irf_plane;
+            if (irf_plane <= g_bounce.cap) GP_TRY(chunked_d2h(dst, gd.snap_fs[b], irf_plane, b, gd.copy));
+            else {
+                GP_CUDA(cudaMemcpyAsync(dst, gd.snap_fs[b], irf_plane * sizeof(double), cudaMemcpyDeviceToHost, gd.copy));
+                GP_CUDA(cudaStreamSynchronize(gd.copy));
+            }
+        }
         worker.busy_s += now() - ts0;
         return GPIRT_B200_OK;
     };
@@ -1744,6 +1819,9 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         if (sampling && fit)
             GP_TRY(launch_predictive_accumulate(s->stream, s->f, s->ldn, gd.pred_code, s->ldy8, s->theta, s->beta, (int)n, (int)m,
                                                 (double)si, gd.pred_acc));
+        if (sampling && irf)   // the f* this sweep drew (fstar, not the means in Dmat); nothing on a side stream writes it
+            GP_TRY(launch_irf_accumulate(s->stream, s->fstar, s->ldN, N_GRID, irf_cells, si, gd.irf_buf, gd.irf_buf + irf_plane,
+                                         irf_lo, irf_plan.klo, irf_hi, irf_plan.khi));
         if (store) {
             const int slot = si / thin;                                             // :99-103
             worker.wait_buffer_free(slot & 1);                                      // slot - 2 has left this snapshot buffer
@@ -1820,6 +1898,21 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         fit->lpd_holdout = sample_iterations ? tot[4] : NAN;   // S = 0: NaN even where no cell is held out
         fit->n_obs = (int64_t)tot[5];
         fit->n_holdout = (int64_t)tot[6];
+    }
+    if (irf) {
+        double* const mean = gd.irf_buf;
+        double* const m2 = mean + irf_plane;
+        if (sample_iterations == 0) {   // all-ones bit pattern = NaN: no sampling iterations
+            GP_CUDA(cudaMemsetAsync(mean, 0xff, 2 * irf_plane * sizeof(double), s->stream));
+        } else {   // sd over M2 in place; the band ends over heap slot 0 of each heap (read before written, per cell)
+            GP_TRY(launch_irf_finish_bands(s->stream, irf_cells, sample_iterations, m2, m2, irf_lo, irf_hi, irf_plan, true,
+                                           irf_lo, irf_hi));
+        }
+        GP_CUDA(cudaStreamSynchronize(s->stream));
+        if (irf->prob_mean) GP_TRY(chunked_d2h(irf->prob_mean, mean, irf_plane, 0, gd.copy));
+        if (irf->prob_sd) GP_TRY(chunked_d2h(irf->prob_sd, m2, irf_plane, 1, gd.copy));
+        if (irf->lower) GP_TRY(chunked_d2h(irf->lower, irf_bands ? irf_lo : m2, irf_plane, 0, gd.copy));   // S = 0: the NaN plane
+        if (irf->upper) GP_TRY(chunked_d2h(irf->upper, irf_bands ? irf_hi : m2, irf_plane, 1, gd.copy));
     }
     GP_CUDA(cudaStreamSynchronize(s->stream));
     if (cb) cb(100.0, cb_ctx);

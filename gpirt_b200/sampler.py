@@ -10,7 +10,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import Fit, GpirtError, Opts, N_GRID
+from ._lib import Fit, GpirtError, Irf, Opts, N_GRID
 from .response_matrix import DEFAULT_CODES, as_response_matrix
 
 
@@ -47,7 +47,8 @@ def nccl_unique_id():
 
 def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_prior_means=None, beta_prior_sds=None,
               beta_proposal_sds=None, theta_init=None, *, seed=None, progress=None, store_f=True, fstar_mode=0,
-              device=-1, shard=None, thin=1, f_summary=False, use_graph=0, predictive=False, y_holdout=None):
+              device=-1, shard=None, thin=1, f_summary=False, use_graph=0, predictive=False, y_holdout=None,
+              irf_band=None, store_fstar=False):
     """Drop-in for the reference's gpirtMCMC().  Keyword-only extras (not in the reference): seed (Philox key; default
     drawn from numpy's global RNG, as the R shim draws it from R's), progress(percent) -> truthy to interrupt,
     store_f=False to skip the n*m*(S+1) f draws, shard=(rank, world, m_global, item_offset, unique_id) for item
@@ -58,7 +59,15 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
     (n x m), elpd_item (m), elpd_resp (n) and the scalars lppd, p_waic, elpd_waic, waic, se_elpd_waic, lpd_holdout, n_obs,
     n_holdout; accumulated on the device, definitions in include/gpirt_b200.h), y_holdout = n x m array of the coded
     response matrix's shape holding +1 / -1 where a missing response was held out (NaN elsewhere; read where y is NA).
-    With shard, per-cell and per-item outputs cover the local items, elpd_resp and the scalars all items."""
+    With shard, per-cell and per-item outputs cover the local items, elpd_resp and the scalars all items.
+    irf_band=b (0 < b < 1) to also return "IRF_summary": dict(mean, sd, lower, upper) of P(y = +1 | theta*) on the grid
+    (1001 x m, over all sampling iterations; lower / upper are the exact pointwise type-7 quantiles at (1 -+ b) / 2 of f*
+    mapped through plogis), band = b and band_bytes = the device memory of its tail buffers; store_fstar=True to also return
+    the f* draws "fstar" (1001 x m x slots, the slots of theta / beta).  With shard both cover the local items."""
+    if irf_band is not None:
+        irf_band = float(irf_band)
+        if not 0.0 < irf_band < 1.0:   # NaN fails too
+            raise ValueError("irf_band must lie in (0, 1), got %r" % irf_band)
     L = _lib.load()
     y = as_response_matrix(data, vote_codes or DEFAULT_CODES)                        # R/gpirtMCMC.R:93
     y = np.asfortranarray(np.asarray(y, dtype=np.float64))
@@ -105,6 +114,17 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
     if f_summary:
         f_mean = np.empty((n, m), order="F"); f_sd = np.empty((n, m), order="F")
         opts.f_mean_out = _lib.ptr(f_mean); opts.f_sd_out = _lib.ptr(f_sd)
+    irf_s = None
+    fstar = np.empty((N_GRID, m, slots), order="F") if store_fstar else None
+    if irf_band is not None or store_fstar:
+        irf_s = Irf()
+        irf_s.fstar_draws = _lib.ptr(fstar)
+        if irf_band is not None:
+            summ = {k: np.empty((N_GRID, m), order="F") for k in ("mean", "sd", "lower", "upper")}
+            irf_s.band = irf_band
+            irf_s.prob_mean, irf_s.prob_sd = _lib.ptr(summ["mean"]), _lib.ptr(summ["sd"])
+            irf_s.lower, irf_s.upper = _lib.ptr(summ["lower"]), _lib.ptr(summ["upper"])
+        opts.irf = C.pointer(irf_s)
 
     def _cb(pct, _ctx):
         try:
@@ -124,6 +144,10 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
         for k in ("lppd", "p_waic", "elpd_waic", "waic", "se_elpd_waic", "lpd_holdout", "n_obs", "n_holdout"):
             pred[k] = getattr(fit, k)
         out["predictive"] = pred
+    if irf_band is not None:
+        out["IRF_summary"] = dict(summ, band=irf_band, band_bytes=int(irf_s.band_bytes))
+    if store_fstar:
+        out["fstar"] = fstar
     return out
 
 
@@ -314,6 +338,20 @@ def predictive_accumulate_time(n, m, reps=100):
     a = C.c_double(0); b = C.c_double(0)
     _lib.check(_lib.load().gpirt_b200_predictive_accumulate_time(int(n), int(m), int(reps), C.byref(a), C.byref(b)))
     return a.value, b.value
+
+
+def irf_bands(draws, band, reps=0):
+    """The IRF band ends of gpirtMCMC(irf_band=band) in f* space, computed on the device by the same update and finish
+    kernels: draws is cols x S (one column per draw, e.g. out["fstar"][:, :, 1:].reshape(-1, S, order="F")); returns
+    (Q(q_lo), Q(q_hi)), each of length cols, and with reps > 0 also (ms per update launch, ms per finish) over reps passes"""
+    d = _F(draws)
+    if d.ndim != 2:
+        raise ValueError("draws must be a cols x S matrix")
+    cols, S = d.shape
+    lo = np.empty(cols); hi = np.empty(cols); ms = np.zeros(2)
+    _lib.check(_lib.load().gpirt_b200_irf_bands(_lib.ptr(d), cols, S, float(band), _lib.ptr(lo), _lib.ptr(hi), int(reps),
+                                                _lib.ptr(ms)))
+    return (lo, hi, (float(ms[0]), float(ms[1]))) if reps > 0 else (lo, hi)
 
 
 def rng_probe(seed, sweep, purpose, stream, idx0, count):

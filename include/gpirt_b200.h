@@ -57,6 +57,33 @@ typedef struct gpirt_b200_fit {
     int64_t n_holdout;    /* out: number of held-out cells */
 } gpirt_b200_fit;
 
+/* Posterior summaries of the item response functions on the grid theta* (1001 points), accumulated on the device.
+ * S = sample_iterations.  For grid point k and local item j, x_s is the f*_kj that sampling iteration s (s = 1..S) draws
+ * (the value the IRF sum accumulates) and P_s = 1 / (1 + exp(-x_s)), as in irf_out.
+ *   prob_mean = mean_s P_s, prob_sd = sd_s P_s (denominator S - 1): FP64 Welford over ALL S iterations (thin has no effect).
+ *   Bands at level b (0 < b < 1): q_lo = (1 - b) / 2, q_hi = (1 + b) / 2 (FP64, on the host); for each q
+ *     h = (S - 1) q, r = floor(h), t = h - r,
+ *     Q = x_(r) + t (x_(r+1) - x_(r))  (0-based ascending order statistics of x_1..x_S: R's type 7, numpy's "linear";
+ *         computed as __dadd_rn(x_(r), __dmul_rn(t, __dsub_rn(x_(r+1), x_(r)))), no contraction), Q = x_(S-1) if r = S - 1;
+ *     lower = plogis(Q(q_lo)), upper = plogis(Q(q_hi)): the band is taken in f* space and mapped to P.
+ *   The order statistics are exact: per grid cell the device keeps the K_lo = r_lo + 2 smallest and the K_hi = S - r_hi
+ *   largest f* seen (two heaps, 8 (K_lo + K_hi) bytes per cell, reported in band_bytes) instead of every draw.
+ *   fstar_draws: 1001 x m x (1 + S / thin), slot 0 = the initial f*, slot k = f* after sampling iteration k * thin.
+ *   S = 0: prob_mean, prob_sd, lower, upper are NaN.  S = 1: prob_sd is NaN, lower = upper = prob_mean = P_1.
+ * Zero-initialise and set the pointers you want (each 1001 x m over the local items; with items sharded each rank's
+ * outputs cover its own item block and no collective is involved).  lower / upper need 0 < band < 1 (else
+ * GPIRT_B200_ERR_ARG); a run whose tail buffers do not fit in free device memory is refused with GPIRT_B200_ERR_NOMEM
+ * before its first sweep.  The buffers are allocated for the call and returned to the device when it ends. */
+typedef struct gpirt_b200_irf {
+    double band;          /* level b of the pointwise credible band (lower / upper only) */
+    double* prob_mean;    /* optional 1001 x m */
+    double* prob_sd;      /* optional 1001 x m */
+    double* lower;        /* optional 1001 x m */
+    double* upper;        /* optional 1001 x m */
+    double* fstar_draws;  /* optional 1001 x m x (1 + S / thin) */
+    int64_t band_bytes;   /* out: device bytes of the tail buffers, 8 * 1001 * m * (K_lo + K_hi) (0 without bands) */
+} gpirt_b200_irf;
+
 /* Options beyond the reference's seven arguments.  Zero-initialise, then set what you need. */
 typedef struct gpirt_b200_opts {
     uint64_t seed;        /* Philox4x32-10 key; the R shim derives it from R's RNG so set.seed() reproduces runs */
@@ -83,6 +110,8 @@ typedef struct gpirt_b200_opts {
     double* f_sd_out;     /* optional n x m: posterior standard deviation of f (denominator S - 1, as R's sd()) */
     gpirt_b200_fit* fit;  /* optional: posterior predictive probabilities, WAIC and held-out scores (gpirt_b200_fit);
                              NULL = none.  Costs 25 bytes of device memory per cell for the run */
+    gpirt_b200_irf* irf;  /* optional: posterior mean, sd, pointwise credible bands and draws of f* on the grid
+                             (gpirt_b200_irf); NULL = none */
 } gpirt_b200_opts;
 
 /* Progress / interrupt callback: called once per iteration with percent complete (as the reference's Rprintf,
@@ -213,6 +242,13 @@ int gpirt_b200_int8_peak_tops_random(double* tops);
  * launches, and of a device-to-device copy of its 3 accumulator planes (24 (n rounded up to 8) m bytes read and as many
  * written) in the same run: the copy rate the accumulation is compared with */
 int gpirt_b200_predictive_accumulate_time(int64_t n, int64_t m, int reps, double* ms_accumulate, double* ms_copy);
+/* The band computation of gpirt_b200_irf on arbitrary draws (tests, measurement): draws is cols x S, column-major, on the
+ * host (for example fstar_draws without slot 0, reshaped to (1001 m) x S).  The draws are uploaded once (8 cols S bytes of
+ * device memory), streamed one at a time through the update kernel gpirt_b200_mcmc uses, then finished as there.
+ * Returns the f*-space Q(q_lo) in lower and Q(q_hi) in upper (cols each, no plogis).  reps > 0: the whole pass is repeated
+ * reps times, timed with CUDA events: ms[0] = mean time of one update launch, ms[1] = mean time of the finish. */
+int gpirt_b200_irf_bands(const double* draws, int64_t cols, int64_t S, double band, double* lower, double* upper, int reps,
+                         double* ms);
 /* ---- the host steps either side of the sampler (SURVEY 8 f4) ---- */
 /* Response coding, the producer of y (reference R/response_matrix.R:79-98) for numeric code matrices, on the device:
  * codes n x m (column-major doubles, NaN = NA); yea / nay / missing code lists; cells with a code in none of the lists are
