@@ -52,12 +52,20 @@ class Irf(C.Structure):
                 ("fstar_draws", C.POINTER(C.c_double)), ("band_bytes", C.c_int64)]
 
 
+class Chains(C.Structure):
+    """gpirt_b200_chains: several chains in one call and their convergence diagnostics (include/gpirt_b200.h)"""
+    _fields_ = [("chains", C.c_int32), ("reserved0", C.c_int32), ("seeds", C.POINTER(C.c_uint64)),
+                ("theta_rhat", C.POINTER(C.c_double)), ("theta_ess", C.POINTER(C.c_double)),
+                ("beta_rhat", C.POINTER(C.c_double)), ("beta_ess", C.POINTER(C.c_double)),
+                ("irf_rhat", C.POINTER(C.c_double)), ("diag_bytes", C.c_int64)]
+
+
 class Opts(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("device", C.c_int32), ("fstar_mode", C.c_int32), ("skip_f_draws", C.c_int32),
                 ("use_graph", C.c_int32), ("rank", C.c_int32), ("world_size", C.c_int32), ("m_global", C.c_int64),
                 ("item_offset", C.c_int64), ("nccl_unique_id", C.c_void_p), ("thin", C.c_int32), ("reserved0", C.c_int32),
                 ("f_mean_out", C.POINTER(C.c_double)), ("f_sd_out", C.POINTER(C.c_double)), ("fit", C.POINTER(Fit)),
-                ("irf", C.POINTER(Irf))]
+                ("irf", C.POINTER(Irf)), ("chains", C.POINTER(Chains))]
 
 
 PROGRESS_CB = C.CFUNCTYPE(C.c_int, C.c_double, C.c_void_p)

@@ -1246,4 +1246,220 @@ int launch_irf_finish_bands(cudaStream_t st, int64_t cells, int S, const double*
     return GPIRT_B200_OK;
 }
 
+// ---- convergence diagnostics of several chains (opts.chains) ----
+// Sampling iteration t = s - 1 of S belongs to the first half (t < half), the second (t >= S - half) or, for odd S, to
+// neither (the middle one); half = S / 2.  Returns the half (-1: none) and the 1-based count within it.
+__device__ __forceinline__ int chain_half(int s, int S, int* count) {
+    const int t = s - 1, half = S / 2;
+    if (t < half) { *count = t + 1; return 0; }
+    if (t >= S - half) { *count = t - (S - half) + 1; return 1; }
+    return -1;
+}
+// One thread per grid cell (halves != NULL) and per traced parameter (trace != NULL).  Cells: the Welford mean / M2 of
+// P = plogis(f*) of the half this iteration belongs to, planes [mean_0, m2_0, mean_1, m2_1] of `cells`.  Parameters:
+// trace[p S + s - 1] = (theta | beta)[p], parameter-major so that the diagnostics read each chain contiguously.
+__global__ void __launch_bounds__(256) k_chain_irf_halves(const double* __restrict__ x, int64_t ld, int rows, int64_t cells,
+                                                          int s, int S, double* __restrict__ halves,
+                                                          const double* __restrict__ theta, int n,
+                                                          const double* __restrict__ beta, int nbeta,
+                                                          double* __restrict__ trace) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (trace && c < n + nbeta) trace[c * S + (s - 1)] = c < n ? theta[c] : beta[c - n];
+    if (!halves || c >= cells) return;
+    int cnt = 0;
+    const int h = chain_half(s, S, &cnt);
+    if (h < 0) return;
+    double* mean = halves + (int64_t)(2 * h) * cells;
+    double* m2 = mean + cells;
+    const int64_t j = c / rows, k = c - j * rows;
+    const double p = 1.0 / (1.0 + exp(-x[k + j * ld]));        // as k_irf_accumulate
+    if (cnt == 1) {
+        mean[c] = p;
+        m2[c] = 0.0;
+    } else {
+        const double mu = mean[c], d = p - mu, mu2 = mu + d / (double)cnt;
+        mean[c] = mu2;
+        m2[c] = fma(d, p - mu2, m2[c]);
+    }
+}
+int launch_chain_halves(cudaStream_t st, const double* x, int64_t ld, int rows, int64_t cells, int s, int S, double* halves,
+                        const double* theta, int n, const double* beta, int nbeta, double* trace) {
+    const int64_t work = std::max(halves ? cells : 0, trace ? (int64_t)n + nbeta : 0);
+    if (work <= 0) return GPIRT_B200_OK;
+    GP_LAUNCH(k_chain_irf_halves, (unsigned)ceil_div(work, 256), 256, 0, st, x, ld, rows, cells, s, S, halves, theta, n, beta,
+              nbeta, trace);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+
+constexpr int DIAG_THREADS = 256, DIAG_WARPS = DIAG_THREADS / 32;
+// sum over the CTA of one value per thread, in a fixed order (thread-strided partial sums, shuffle tree, warp partials in
+// warp order): bit-identical run to run.  Every thread gets the total.
+__device__ __forceinline__ double diag_block_sum(double v, double* red) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    const int warp = threadIdx.x >> 5;
+    __syncthreads();                                           // red[] free (previous sum read by every thread)
+    if ((threadIdx.x & 31) == 0) red[warp] = v;
+    __syncthreads();
+    double t = 0.0;
+#pragma unroll
+    for (int w = 0; w < DIAG_WARPS; ++w) t += red[w];
+    return t;
+}
+// One CTA per parameter p, chains in order.  Per chain (S draws at trace + (c P + p) S): the means and sums of squared
+// deviations of its two halves, and Geyer's initial monotone sequence ESS over all S draws with autocovariances of
+// denominator S.  Warp w computes lag pair k = base + w (lags 2k, 2k + 1), eight pairs per block of lags; thread 0 walks
+// them in order and stops at the first non-positive pair.  The formulas of gpirt_b200_theta_diagnostics.
+// use_smem: the chain is staged (centred) in S doubles of dynamic shared memory; else it is read from global memory.
+__global__ void __launch_bounds__(DIAG_THREADS) k_chain_diag(const double* __restrict__ trace, int P, int S, int C,
+                                                             int use_smem, double* __restrict__ rhat, double* __restrict__ ess) {
+    extern __shared__ double xs[];
+    __shared__ double red[DIAG_WARPS], acv[2 * DIAG_WARPS], means[64];
+    __shared__ int done;
+    const int p = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int half = S / 2;
+    const double T = (double)S;
+    double W = 0.0, grand = 0.0, ess_sum = 0.0;               // thread 0's running values
+    for (int c = 0; c < C; ++c) {
+        const double* x = trace + ((int64_t)c * P + p) * S;
+        if (use_smem) {
+            __syncthreads();                                   // previous chain's readers are done with xs
+            for (int t = tid; t < S; t += DIAG_THREADS) xs[t] = x[t];
+            __syncthreads();
+        }
+        const double* src = use_smem ? xs : x;
+        // Every sum runs over values shifted by the first value of their segment: the same statistics as the host's, and
+        // exactly zero spread for a constant segment (a sum of S equal values over S need not give the value back).
+        for (int h = 0; h < 2; ++h) {
+            const double* seg = src + (h ? S - half : 0);
+            const double x0 = seg[0];
+            double a = 0.0;
+            for (int t = tid; t < half; t += DIAG_THREADS) a += seg[t] - x0;
+            const double dmu = diag_block_sum(a, red) / (double)half;
+            double q = 0.0;
+            for (int t = tid; t < half; t += DIAG_THREADS) { const double d = (seg[t] - x0) - dmu; q += d * d; }
+            const double v = diag_block_sum(q, red);
+            if (tid == 0) {
+                const double mu = x0 + dmu;
+                W += v / (double)(half - 1);
+                means[2 * c + h] = mu;
+                grand += mu;
+            }
+        }
+        const double x0 = src[0];
+        double a = 0.0;
+        for (int t = tid; t < S; t += DIAG_THREADS) a += src[t] - x0;
+        const double dmean = diag_block_sum(a, red) / T;
+        double sub1 = x0, sub2 = dmean;                        // y_t = (x_t - x0) - dmean
+        if (use_smem) {                                        // centre in place
+            for (int t = tid; t < S; t += DIAG_THREADS) xs[t] = (xs[t] - x0) - dmean;
+            __syncthreads();
+            sub1 = sub2 = 0.0;
+        }
+        double c0 = 0.0, sum = 0.0, prev = INFINITY;
+        if (tid == 0) done = 0;
+        for (int base = 0;; base += DIAG_WARPS) {
+            const int k = base + warp;
+            double s0 = 0.0, s1 = 0.0;                         // lags 2k and 2k + 1
+            if (2 * k + 1 < S) {
+                const int lag = 2 * k;
+                for (int t = lane; t + lag < S; t += 32) {
+                    const double yt = (src[t] - sub1) - sub2;
+                    s0 += yt * ((src[t + lag] - sub1) - sub2);
+                    if (t + lag + 1 < S) s1 += yt * ((src[t + lag + 1] - sub1) - sub2);
+                }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) {
+                    s0 += __shfl_xor_sync(0xffffffffu, s0, o);
+                    s1 += __shfl_xor_sync(0xffffffffu, s1, o);
+                }
+            }
+            __syncthreads();                                   // acv[] of the previous block has been read
+            if (lane == 0) { acv[2 * warp] = s0 / T; acv[2 * warp + 1] = s1 / T; }
+            __syncthreads();
+            if (tid == 0) {
+                for (int w = 0; w < DIAG_WARPS && !done; ++w) {
+                    const int kk = base + w;
+                    if (kk == 0) {
+                        c0 = acv[0];
+                        if (!(c0 > 0.0)) { done = 2; break; }  // constant chain
+                    }
+                    if (!(2 * kk + 1 < S)) { done = 1; break; }
+                    double pair = (acv[2 * w] + acv[2 * w + 1]) / c0;
+                    if (pair <= 0.0) { done = 1; break; }
+                    pair = fmin(pair, prev);                   // initial monotone sequence
+                    prev = pair;
+                    sum += pair;
+                }
+            }
+            __syncthreads();
+            if (done) break;
+        }
+        if (tid == 0) {
+            const double tau = -1.0 + 2.0 * sum;
+            ess_sum += done == 2 ? NAN : T / fmax(tau, 1e-12);
+        }
+    }
+    if (tid == 0) {
+        const double M = 2.0 * C;
+        W /= M; grand /= M;
+        double Bv = 0.0;
+        for (int i = 0; i < 2 * C; ++i) Bv += (means[i] - grand) * (means[i] - grand);
+        Bv *= (double)half / (M - 1.0);
+        const double var_plus = ((double)(half - 1) / (double)half) * W + Bv / (double)half;
+        if (rhat) rhat[p] = W > 0.0 ? sqrt(var_plus / W) : NAN;
+        if (ess) ess[p] = ess_sum;
+    }
+}
+int chain_diag_smem_bytes(int S) {
+    int dev = 0, optin = 0;
+    GP_CUDA(cudaGetDevice(&dev));
+    GP_CUDA(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    const size_t fixed = 1024;                                 // the kernel's static shared memory, rounded up
+    const size_t want = (size_t)S * sizeof(double);
+    return want + fixed <= (size_t)optin ? (int)want : 0;
+}
+int launch_chain_diag(cudaStream_t st, const double* trace, int P, int S, int C, double* rhat, double* ess) {
+    if (P <= 0) return GPIRT_B200_OK;
+    if (S < 4 || C < 1 || C > 32) return GPIRT_B200_ERR_ARG;
+    const int smem = chain_diag_smem_bytes(S);
+    if (smem > 0) GP_CUDA(cudaFuncSetAttribute(k_chain_diag, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    GP_LAUNCH(k_chain_diag, (unsigned)P, DIAG_THREADS, (size_t)smem, st, trace, P, S, C, smem > 0 ? 1 : 0, rhat, ess);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+// one thread per cell: split-R-hat of P over the 2C half-chain Welford states (chain c's planes at halves + 4 c cells)
+__global__ void __launch_bounds__(256) k_chain_irf_rhat(const double* __restrict__ halves, int64_t cells, int S, int C,
+                                                        double* __restrict__ rhat) {
+    const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= cells) return;
+    const int half = S / 2;
+    double W = 0.0, grand = 0.0;
+    for (int ch = 0; ch < C; ++ch)
+        for (int h = 0; h < 2; ++h) {
+            const double* mean = halves + (int64_t)(4 * ch + 2 * h) * cells;
+            W += mean[cells + c] / (double)(half - 1);
+            grand += mean[c];
+        }
+    const double M = 2.0 * C;
+    W /= M; grand /= M;
+    double Bv = 0.0;
+    for (int ch = 0; ch < C; ++ch)
+        for (int h = 0; h < 2; ++h) {
+            const double mu = halves[(int64_t)(4 * ch + 2 * h) * cells + c];
+            Bv += (mu - grand) * (mu - grand);
+        }
+    Bv *= (double)half / (M - 1.0);
+    const double var_plus = ((double)(half - 1) / (double)half) * W + Bv / (double)half;
+    rhat[c] = W > 0.0 ? sqrt(var_plus / W) : NAN;
+}
+int launch_chain_irf_rhat(cudaStream_t st, const double* halves, int64_t cells, int S, int C, double* rhat) {
+    if (cells <= 0) return GPIRT_B200_OK;
+    if (S < 4) return GPIRT_B200_ERR_ARG;
+    GP_LAUNCH(k_chain_irf_rhat, (unsigned)ceil_div(cells, 256), 256, 0, st, halves, cells, S, C, rhat);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+
 }  // namespace gpirt

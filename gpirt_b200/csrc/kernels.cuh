@@ -97,5 +97,19 @@ int launch_irf_accumulate(cudaStream_t st, const double* x, int64_t ld, int rows
 int launch_irf_finish_bands(cudaStream_t st, int64_t cells, int S, const double* m2, double* sd_out, const double* lo,
                             const double* hi, const IrfBandPlan& plan, bool plogis, double* lower, double* upper);
 
+// ---- convergence diagnostics of several chains (opts.chains, definitions in include/gpirt_b200.h) ----
+// sampling iteration s (1-based) of S of one chain: with halves != NULL the Welford mean / M2 of plogis(x) of the half the
+// iteration belongs to (planes mean_0, m2_0, mean_1, m2_1 of `cells`; the middle iteration of an odd S is skipped); with
+// trace != NULL trace[p S + s - 1] = theta[p] (p < n) or beta[p - n] (n <= p < n + nbeta)
+int launch_chain_halves(cudaStream_t st, const double* x, int64_t ld, int rows, int64_t cells, int s, int S, double* halves,
+                        const double* theta, int n, const double* beta, int nbeta, double* trace);
+// after S >= 4 iterations of C chains (trace: C blocks of P x S, parameter-major): split-R-hat and summed Geyer ESS per
+// parameter (rhat / ess: P, either may be NULL); fixed-order reductions, no atomics
+int launch_chain_diag(cudaStream_t st, const double* trace, int P, int S, int C, double* rhat, double* ess);
+// dynamic shared memory k_chain_diag stages one chain in (0: the chain is read from global memory)
+int chain_diag_smem_bytes(int S);
+// split-R-hat of P per cell over the 2C half-chain states (chain c's four planes at halves + 4 c cells), S >= 4
+int launch_chain_irf_rhat(cudaStream_t st, const double* halves, int64_t cells, int S, int C, double* rhat);
+
 
 }  // namespace gpirt

@@ -12,6 +12,7 @@
 #include <condition_variable>
 #include <deque>
 #include <functional>
+#include <memory>
 #include <string>
 #include <thread>
 #include <vector>
@@ -124,6 +125,9 @@ __global__ void k_stamp(unsigned long long* slot) {
     asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
     *slot = t;
 }
+
+// set around gpirt_b200_sampler_create by a several-chain call: chains after the first ignore GPIRT_TRACE
+static thread_local bool t_untraced_create = false;
 
 struct gpirt_b200_sampler {
     int n = 0, m = 0;
@@ -371,7 +375,7 @@ int gpirt_b200_sampler::create(const double* y, int64_t n_, int64_t m_, const do
         GP_TRY(comm_init(comm, opts.rank, opts.world_size, opts.nccl_unique_id));
     }
     launches_at_create = g_launch_count;
-    if (const char* tf = getenv("GPIRT_TRACE")) {
+    if (const char* tf = t_untraced_create ? nullptr : getenv("GPIRT_TRACE")) {
         if (opts.rank == 0 || opts.world_size <= 1) trace_file = fopen(tf, "a");
         if (trace_file) fprintf(trace_file, "# sampler %d x %d world %d\n", n, m, opts.world_size > 1 ? opts.world_size : 1);
     }
@@ -1070,12 +1074,13 @@ struct Bounce {
 Bounce g_bounce;        // process-wide, reused across calls (2 x n*m*8 bytes of pinned memory once f draws are stored)
 std::mutex g_bounce_mu; // held by a gpirt_b200_mcmc call for its whole duration (concurrent calls in one process take turns)
 
-int host_threads_for_copy() {
+// host copy threads of one storage worker: one process per GPU on the same host, and the chains of one call, share the cores
+int host_threads_for_copy(int chains) {
     const char* e = getenv("GPIRT_COPY_THREADS");
     int t = e ? atoi(e) : (int)std::min(12u, std::max(1u, std::thread::hardware_concurrency() * 3 / 4));
-    const char* ws = getenv("WORLD_SIZE");   // one process per GPU on the same host: share the cores
-    const int world = ws ? atoi(ws) : 1;
-    if (!e && world > 1) t = std::max(2, t / world);
+    const char* ws = getenv("WORLD_SIZE");
+    const int share = (ws ? std::max(1, atoi(ws)) : 1) * chains;
+    if (!e && share > 1) t = std::max(2, t / share);
     return t < 1 ? 1 : (t > 32 ? 32 : t);
 }
 
@@ -1087,15 +1092,17 @@ int host_threads_for_copy() {
 // piece — the only part that cannot overlap the DMA — is 4 MiB by one thread (with 32 MiB pieces one thread spent 8-20 ms
 // on the last one after the DMA had finished: first-touch copies run at 1.5 GB/s per thread on 4 KiB pages, ~4 GB/s on
 // huge pages; tools/host_store_probe.cpp), and a huge page of the destination is first touched by exactly one thread.
-// The caller holds g_bounce_mu.
+// `bo` is g_bounce (its caller holds g_bounce_mu) or bounce buffers a call owns; `threads` host threads copy.
 struct BounceXfer {
     std::vector<size_t> cut;   // piece boundaries in doubles
     double* dst = nullptr;
     bool staged = false;       // false: no pinned memory, the copy was done by the driver in bounce_issue
+    Bounce* bo = nullptr;
+    int threads = 1;
 };
-int bounce_issue(double* dst, const double* src, size_t count, int b, cudaStream_t stream, BounceXfer& x) {
-    x.dst = dst; x.cut.clear(); x.staged = false;
-    if (g_bounce.ensure(count) != GPIRT_B200_OK) {   // no pinned memory: plain (driver-staged) copy
+int bounce_issue(Bounce& bo, int threads, double* dst, const double* src, size_t count, int b, cudaStream_t stream, BounceXfer& x) {
+    x.dst = dst; x.cut.clear(); x.staged = false; x.bo = &bo; x.threads = threads;
+    if (bo.ensure(count) != GPIRT_B200_OK) {   // no pinned memory: plain (driver-staged) copy
         GP_CUDA(cudaMemcpyAsync(dst, src, count * sizeof(double), cudaMemcpyDeviceToHost, stream));
         GP_CUDA(cudaStreamSynchronize(stream));
         return GPIRT_B200_OK;
@@ -1108,15 +1115,15 @@ int bounce_issue(double* dst, const double* src, size_t count, int b, cudaStream
     while (next < d1) { x.cut.push_back((next - d0) / sizeof(double)); next += piece; }
     x.cut.push_back(count);
     const int npieces = (int)x.cut.size() - 1;
-    while ((int)g_bounce.ev[b].size() < npieces) {
+    while ((int)bo.ev[b].size() < npieces) {
         cudaEvent_t e;
         GP_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        g_bounce.ev[b].push_back(e);
+        bo.ev[b].push_back(e);
     }
-    double* bb = g_bounce.buf[b];
+    double* bb = bo.buf[b];
     for (int c = 0; c < npieces; ++c) {
         GP_CUDA(cudaMemcpyAsync(bb + x.cut[c], src + x.cut[c], (x.cut[c + 1] - x.cut[c]) * sizeof(double), cudaMemcpyDeviceToHost, stream));
-        GP_CUDA(cudaEventRecord(g_bounce.ev[b][c], stream));
+        GP_CUDA(cudaEventRecord(bo.ev[b][c], stream));
     }
     x.staged = true;
     return GPIRT_B200_OK;
@@ -1124,15 +1131,15 @@ int bounce_issue(double* dst, const double* src, size_t count, int b, cudaStream
 int bounce_finish(int b, BounceXfer& x) {
     if (!x.staged) return GPIRT_B200_OK;
     const int npieces = (int)x.cut.size() - 1;
-    const double* bb = g_bounce.buf[b];
-    const int T = std::min(host_threads_for_copy(), npieces);
+    const double* bb = x.bo->buf[b];
+    const int T = std::min(x.threads, npieces);
     std::atomic<int> next{0};
     std::atomic<int> failed{0};
     auto work = [&]() {
         for (;;) {
             const int c = next.fetch_add(1);
             if (c >= npieces) break;
-            if (cudaEventSynchronize(g_bounce.ev[b][c]) != cudaSuccess) { failed = 1; break; }
+            if (cudaEventSynchronize(x.bo->ev[b][c]) != cudaSuccess) { failed = 1; break; }
             std::memcpy(x.dst + x.cut[c], bb + x.cut[c], (x.cut[c + 1] - x.cut[c]) * sizeof(double));
         }
     };
@@ -1144,9 +1151,9 @@ int bounce_finish(int b, BounceXfer& x) {
     if (failed) { set_last_error("device-to-host copy of a draw slice failed"); return GPIRT_B200_ERR_CUDA; }
     return GPIRT_B200_OK;
 }
-int chunked_d2h(double* dst, const double* src, size_t count, int b, cudaStream_t stream) {
+int chunked_d2h(Bounce& bo, int threads, double* dst, const double* src, size_t count, int b, cudaStream_t stream) {
     BounceXfer x;
-    GP_TRY(bounce_issue(dst, src, count, b, stream, x));
+    GP_TRY(bounce_issue(bo, threads, dst, src, count, b, stream, x));
     return bounce_finish(b, x);
 }
 }  // namespace
@@ -1505,76 +1512,145 @@ __global__ void __launch_bounds__(256) k_f_sd(double* __restrict__ m2, size_t co
     if (i < count_elems) m2[i] = sqrt(m2[i] / denom);   // denom = S - 1 (R's sd); S = 1 gives NaN like sd() of one value
 }
 
-int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_init, int sample_iterations,
-                    int burn_iterations, const double* pm, const double* psd, const double* pstep,
-                    const gpirt_b200_opts* opts, double* theta_out, double* beta_out, double* f_out, double* irf_out,
-                    gpirt_b200_progress_cb cb, void* cb_ctx) {
-    if (sample_iterations < 0 || burn_iterations < 0 || !theta_out || !beta_out || !irf_out) {
-        set_last_error("bad argument: negative iteration count or null output");
-        return GPIRT_B200_ERR_ARG;
-    }
-    const bool keep_f = !(opts && opts->skip_f_draws);
-    if (keep_f && !f_out) { set_last_error("f_out is NULL but f draws were requested"); return GPIRT_B200_ERR_ARG; }
-    if (opts && opts->thin < 0) { set_last_error("bad argument: thin < 0"); return GPIRT_B200_ERR_ARG; }
-    const int thin = (opts && opts->thin > 1) ? opts->thin : 1;
-    double* f_mean_out = opts ? opts->f_mean_out : nullptr;
-    double* f_sd_out = opts ? opts->f_sd_out : nullptr;
-    const bool summarise_f = f_mean_out || f_sd_out;
-    gpirt_b200_fit* const fit = opts ? opts->fit : nullptr;
-    gpirt_b200_irf* const irf = opts ? opts->irf : nullptr;
-    if (irf && (irf->lower || irf->upper) && !(std::isfinite(irf->band) && irf->band > 0.0 && irf->band < 1.0)) {
-        set_last_error("bad argument: the IRF band level must lie in (0, 1), got %g", irf->band);
-        return GPIRT_B200_ERR_ARG;
-    }
-    const bool trace = getenv("GPIRT_TIMING") != nullptr;
-    auto now = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; };
-    g_last_degenerate_theta = 0;
-    double t_a = now();
-    struct ExitTrace {   // first local: destroyed last
-        bool on; double t_enter; double t_body_end = 0.0;
-        ~ExitTrace() {
-            if (!on) return;
-            timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts);
-            const double t = ts.tv_sec + 1e-9 * ts.tv_nsec;
-            fprintf(stderr, "gpirt_b200_mcmc: total %.3fs in the call, %.3fs after the body\n", t - t_enter, t_body_end > 0.0 ? t - t_body_end : 0.0);
+namespace {
+// One chain of gpirtMCMC(): the sampler, its draw storage (snapshot buffers, copy stream, StoreWorker), the status polling
+// and the on-device accumulators, driven by setup(), one iterate() per sweep and finish().  gpirt_b200_mcmc drives one;
+// with opts.chains it drives several on one device, round-robin from the calling thread.  The progress callback belongs
+// to the driver: a chain only learns of an interrupt through want_stop.
+struct ChainRun {
+    // arguments of the call (outputs already offset to this chain's block)
+    const double* y; int64_t n, m; const double* theta_init; int S, B; const double *pm, *psd, *pstep;
+    const gpirt_b200_opts* opts; double *theta_out, *beta_out, *f_out, *irf_out;
+    Bounce* bo;                       // pinned staging: g_bounce, or a set the call owns
+    int copy_threads;                 // host copy threads of the storage worker
+    bool trace;                       // GPIRT_TIMING
+    bool untraced = false;            // create() ignores GPIRT_TRACE (chains after the first)
+    // several chains: this chain's trace of theta | beta (P x S, parameter-major) and its IRF half-chain states
+    double* diag_trace = nullptr;
+    double* diag_halves = nullptr;
+
+    bool keep_f = true; int thin = 1;
+    double *f_mean_out = nullptr, *f_sd_out = nullptr; bool summarise_f = false;
+    gpirt_b200_fit* fit = nullptr; gpirt_b200_irf* irf = nullptr;
+    int n_slots = 0; size_t nm = 0, n_small = 0; bool sharded = false;
+    // resources, released by the destructor
+    gpirt_b200_sampler* s = nullptr; cudaStream_t copy = nullptr; cudaEvent_t ev[2] = {nullptr, nullptr};
+    double* snap_f[2] = {nullptr, nullptr}; double* snap_small[2] = {nullptr, nullptr};
+    double *f_mean = nullptr, *f_m2 = nullptr, *agree_dev = nullptr; int* h_poll = nullptr; StoreWorker* worker = nullptr;
+    double* h_small[2] = {nullptr, nullptr}; cudaEvent_t ev_small[2] = {nullptr, nullptr};
+    double* pred_acc = nullptr; int8_t* pred_code = nullptr; double* pred_aux = nullptr;   // opts.fit
+    double* irf_buf = nullptr; double* snap_fs[2] = {nullptr, nullptr};                     // opts.irf
+    // state of the run
+    double* h_ring = nullptr; volatile int* w_poll = nullptr; int agree_count = 0;
+    static constexpr int PRED_CHUNKS = 64;
+    size_t pred_plane = 0;
+    double *pred_stats = nullptr, *pred_partial = nullptr, *pred_resp = nullptr;
+    int64_t irf_cells = 0; size_t irf_plane = 0; double* fs_out = nullptr; bool irf_bands = false; IrfBandPlan irf_plan{};
+    double *irf_lo = nullptr, *irf_hi = nullptr;
+    BounceXfer xfer[2];
+    bool want_stop = false; int stop_code = GPIRT_B200_OK; int n_summarised = 0;
+    int64_t degenerate = 0;           // theta draws with a degenerate grid CDF (finish)
+    double t_a = 0.0, t_b = 0.0, t_c = 0.0, t_d = 0.0;
+
+    static double now() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; }
+
+    ~ChainRun() {
+        const double t0 = now();
+        if (worker) {   // before anything it uses goes away
+            worker->stop();
+            if (trace) fprintf(stderr, "gpirt_b200_mcmc: storage thread joined in %.3fs\n", now() - t0);
+            delete worker;
         }
-    } exit_trace{trace, t_a};
-    // the pinned bounce buffers are process-wide: a call that moves f through them owns them until it returns
-    std::unique_lock<std::mutex> bounce_lock(g_bounce_mu);
-    gpirt_b200_sampler* s = nullptr;
-    GP_TRY(gpirt_b200_sampler_create(&s, y, n, m, theta_init, pm, psd, pstep, opts));
+        if (!s) return;
+        if (copy) { cudaStreamSynchronize(copy); cudaStreamDestroy(copy); }
+        const double t1 = now();
+        for (int i = 0; i < 2; ++i) if (ev_small[i]) cudaEventDestroy(ev_small[i]);   // h_small / h_poll belong to bo
+        for (int i = 0; i < 2; ++i) { if (ev[i]) cudaEventDestroy(ev[i]); pool_free(snap_f[i], s->stream); pool_free(snap_small[i], s->stream); }
+        pool_free(f_mean, s->stream); pool_free(f_m2, s->stream); pool_free(agree_dev, s->stream);
+        pool_free(pred_acc, s->stream); pool_free(pred_code, s->stream); pool_free(pred_aux, s->stream);
+        for (int i = 0; i < 2; ++i) pool_free(snap_fs[i], s->stream);
+        if (irf_buf) { cudaStreamSynchronize(s->stream); cudaFree(irf_buf); }   // not the pool: GBs of tail buffers must not stay reserved after the call
+        const double t2 = now();
+        gpirt_b200_sampler_destroy(s);
+        if (trace) fprintf(stderr, "gpirt_b200_mcmc: teardown worker/copy stream %.3fs, host + pool frees %.3fs, sampler %.3fs\n", t1 - t0, t2 - t1, now() - t2);
+    }
+
+    int d2h(double* dst, const double* src, size_t count, int b) { return chunked_d2h(*bo, copy_threads, dst, src, count, b, copy); }
+
+    // snapshot(slot): main stream copies theta | beta (and f, tightly packed) into buffer slot & 1 and records the event
+    int snapshot(int slot) {
+        const int b = slot & 1;
+        GP_CUDA(cudaMemcpyAsync(snap_small[b], s->theta, (size_t)n * sizeof(double), cudaMemcpyDeviceToDevice, s->stream));
+        GP_CUDA(cudaMemcpyAsync(snap_small[b] + n, s->beta, 2 * (size_t)m * sizeof(double), cudaMemcpyDeviceToDevice, s->stream));
+        if (keep_f)
+            GP_CUDA(cudaMemcpy2DAsync(snap_f[b], (size_t)n * sizeof(double), s->f, s->ldn * sizeof(double), (size_t)n * sizeof(double),
+                                      (size_t)m, cudaMemcpyDeviceToDevice, s->stream));
+        if (fs_out)
+            GP_CUDA(cudaMemcpy2DAsync(snap_fs[b], N_GRID * sizeof(double), s->fstar, s->ldN * sizeof(double), N_GRID * sizeof(double),
+                                      (size_t)m, cudaMemcpyDeviceToDevice, s->stream));
+        GP_CUDA(cudaEventRecord(ev[b], s->stream));
+        return GPIRT_B200_OK;
+    }
+
+    // Stopping early (interrupt from the progress callback, failed Cholesky / ESS seen in the polled status words, a failed
+    // store) must be a COMMON decision when items are sharded: a rank that returned alone would leave its peers blocked in
+    // the next sweep's collectives.  Every rank therefore enqueues, every 8th iteration, a one-word all-reduce of its local
+    // stop request on the sampler's stream and acts on the agreed value after the host sync that follows it — the same
+    // program point on every rank.  An unsharded chain stops as soon as it sees a reason.
+    int local_stop_code() {
+        std::string msg;
+        const int wrc = worker->status(&msg);
+        if (wrc != GPIRT_B200_OK) { set_last_error("%s", msg.c_str()); return wrc; }
+        if (h_poll[0] || w_poll[0]) { set_last_error("chol(): decomposition failed"); return GPIRT_B200_ERR_NOT_PD; }
+        if (h_poll[1] || w_poll[1]) { set_last_error("elliptical slice sampler did not terminate (NaN log-likelihood?)"); return GPIRT_B200_ERR_ESS; }
+        if (want_stop) { set_last_error("interrupted by the progress callback"); return GPIRT_B200_ERR_INTERRUPT; }
+        return GPIRT_B200_OK;
+    }
+    int enqueue_agreement() {
+        if (!sharded) return GPIRT_B200_OK;
+        const double mine = local_stop_code() != GPIRT_B200_OK ? 1.0 : 0.0;   // pageable source: staged at call time
+        GP_CUDA(cudaMemcpyAsync(agree_dev, &mine, sizeof(double), cudaMemcpyHostToDevice, s->stream));
+        GP_TRY(comm_allreduce_sum_f64(s->comm, agree_dev, 1, s->stream));
+        GP_CUDA(cudaMemcpyAsync(h_ring + (agree_count & 7), agree_dev, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+        agree_count += 1;
+        return GPIRT_B200_OK;
+    }
+    bool stop_now(int agreement) {   // after a host sync that covers agreement number `agreement`
+        stop_code = local_stop_code();
+        if (sharded) {
+            if (agreement < 0 || h_ring[agreement & 7] == 0.0) return false;
+            if (stop_code == GPIRT_B200_OK) { set_last_error("stopped: another rank was interrupted or failed"); stop_code = GPIRT_B200_ERR_INTERRUPT; }
+            return true;
+        }
+        return stop_code != GPIRT_B200_OK;
+    }
+    // before each iteration: interrupt, failed store, failed chain seen by the worker (unsharded: sharded ranks agree later)
+    bool stopped() { return !sharded && stop_now(-1); }
+
+    int setup();
+    int iterate(int iter);
+    int finish();
+};
+
+int ChainRun::setup() {
+    keep_f = !(opts && opts->skip_f_draws);
+    thin = (opts && opts->thin > 1) ? opts->thin : 1;
+    f_mean_out = opts ? opts->f_mean_out : nullptr;
+    f_sd_out = opts ? opts->f_sd_out : nullptr;
+    summarise_f = f_mean_out || f_sd_out;
+    fit = opts ? opts->fit : nullptr;
+    irf = opts ? opts->irf : nullptr;
+    t_a = now();
+    t_untraced_create = untraced;
+    const int crc = gpirt_b200_sampler_create(&s, y, n, m, theta_init, pm, psd, pstep, opts);
+    t_untraced_create = false;
+    GP_TRY(crc);
     s->timing = false;
-    double t_b = now();
+    t_b = now();
     // Draw storage overlaps the next sweep: after sweep t the state is snapshotted device-to-device (cheap), the host
     // enqueues sweep t+1, and only then blocks in the device-to-host copy of snapshot t on a second stream.
-    struct Guard {
-        gpirt_b200_sampler* s; cudaStream_t copy; cudaEvent_t ev[2]; double* snap_f[2]; double* snap_small[2];
-        double *f_mean, *f_m2, *agree_dev; int* h_poll; StoreWorker* worker;
-        double* h_small[2]; cudaEvent_t ev_small[2];
-        bool trace = false;
-        double* pred_acc = nullptr; int8_t* pred_code = nullptr; double* pred_aux = nullptr;   // opts.fit
-        double* irf_buf = nullptr; double* snap_fs[2] = {nullptr, nullptr};                     // opts.irf
-        ~Guard() {
-            auto now = [] { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec + 1e-9 * ts.tv_nsec; };
-            const double t0 = now();
-            if (worker) { worker->stop(); delete worker; }   // before anything it uses goes away
-            if (copy) { cudaStreamSynchronize(copy); cudaStreamDestroy(copy); }
-            const double t1 = now();
-            for (int i = 0; i < 2; ++i) if (ev_small[i]) cudaEventDestroy(ev_small[i]);   // h_small / h_poll belong to g_bounce
-            for (int i = 0; i < 2; ++i) { if (ev[i]) cudaEventDestroy(ev[i]); pool_free(snap_f[i], s->stream); pool_free(snap_small[i], s->stream); }
-            pool_free(f_mean, s->stream); pool_free(f_m2, s->stream); pool_free(agree_dev, s->stream);
-            pool_free(pred_acc, s->stream); pool_free(pred_code, s->stream); pool_free(pred_aux, s->stream);
-            for (int i = 0; i < 2; ++i) pool_free(snap_fs[i], s->stream);
-            if (irf_buf) { cudaStreamSynchronize(s->stream); cudaFree(irf_buf); }   // not the pool: GBs of tail buffers must not stay reserved after the call
-            const double t2 = now();
-            gpirt_b200_sampler_destroy(s);
-            if (trace) fprintf(stderr, "gpirt_b200_mcmc: teardown worker/copy stream %.3fs, host + pool frees %.3fs, sampler %.3fs\n", t1 - t0, t2 - t1, now() - t2);
-        }
-    } gd{s, nullptr, {nullptr, nullptr}, {nullptr, nullptr}, {nullptr, nullptr}, nullptr, nullptr, nullptr, nullptr, nullptr,
-         {nullptr, nullptr}, {nullptr, nullptr}};
-    gd.trace = trace;
-    const int n_slots = sample_iterations / thin + 1;         // slot 0 = initial values, slot k = sampling iteration k * thin
-    const size_t nm = (size_t)n * m;
+    n_slots = S / thin + 1;         // slot 0 = initial values, slot k = sampling iteration k * thin
+    nm = (size_t)n * m;
     if (keep_f && !getenv("GPIRT_NO_HUGEPAGE_HINT")) {
         // the caller's f array is fresh pageable memory: ask for transparent huge pages on its interior so that the
         // first-touch faults of the draw stores are 2 MiB each instead of 4 KiB (advisory; ignored where THP is off).
@@ -1584,56 +1660,53 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         const uintptr_t b = ((uintptr_t)f_out + (size_t)n_slots * nm * sizeof(double)) & ~(((uintptr_t)2 << 20) - 1);
         if (b > a) madvise((void*)a, b - a, MADV_HUGEPAGE);
     }
-    const size_t n_small = (size_t)n + 2 * (size_t)m;     // theta | beta of one slot
-    GP_CUDA(cudaStreamCreateWithFlags(&gd.copy, cudaStreamNonBlocking));
-    if (g_bounce.ensure_small(n_small) != GPIRT_B200_OK) { set_last_error("pinned host staging could not be allocated"); return GPIRT_B200_ERR_NOMEM; }
+    n_small = (size_t)n + 2 * (size_t)m;     // theta | beta of one slot
+    GP_CUDA(cudaStreamCreateWithFlags(&copy, cudaStreamNonBlocking));
+    if (bo->ensure_small(n_small) != GPIRT_B200_OK) { set_last_error("pinned host staging could not be allocated"); return GPIRT_B200_ERR_NOMEM; }
     for (int i = 0; i < 2; ++i) {
-        gd.h_small[i] = g_bounce.small[i];
-        GP_CUDA(cudaEventCreateWithFlags(&gd.ev_small[i], cudaEventDisableTiming));
+        h_small[i] = bo->small[i];
+        GP_CUDA(cudaEventCreateWithFlags(&ev_small[i], cudaEventDisableTiming));
     }
-    gd.h_poll = g_bounce.poll;
-    std::memset(gd.h_poll, 0, Bounce::POLL_BYTES);   // [0..3] status words polled by this thread, [4..7] by the
-    double* h_ring = reinterpret_cast<double*>(gd.h_poll + 8);         // storage worker, then a ring of 8 agreed stop flags
-    volatile int* w_poll = gd.h_poll + 4;
-    int agree_count = 0;
+    h_poll = bo->poll;
+    std::memset(h_poll, 0, Bounce::POLL_BYTES);   // [0..3] status words polled by this thread, [4..7] by the
+    h_ring = reinterpret_cast<double*>(h_poll + 8);      // storage worker, then a ring of 8 agreed stop flags
+    w_poll = h_poll + 4;
     for (int i = 0; i < 2; ++i) {
-        GP_CUDA(cudaEventCreateWithFlags(&gd.ev[i], cudaEventDisableTiming));
-        GP_TRY(pool_alloc((void**)&gd.snap_small[i], n_small * sizeof(double), s->stream));
-        if (keep_f) GP_TRY(pool_alloc((void**)&gd.snap_f[i], nm * sizeof(double), s->stream));
+        GP_CUDA(cudaEventCreateWithFlags(&ev[i], cudaEventDisableTiming));
+        GP_TRY(pool_alloc((void**)&snap_small[i], n_small * sizeof(double), s->stream));
+        if (keep_f) GP_TRY(pool_alloc((void**)&snap_f[i], nm * sizeof(double), s->stream));
     }
     if (summarise_f) {
-        GP_TRY(pool_alloc((void**)&gd.f_mean, nm * sizeof(double), s->stream));
-        GP_TRY(pool_alloc((void**)&gd.f_m2, nm * sizeof(double), s->stream));
+        GP_TRY(pool_alloc((void**)&f_mean, nm * sizeof(double), s->stream));
+        GP_TRY(pool_alloc((void**)&f_m2, nm * sizeof(double), s->stream));
     }
-    const bool sharded = s->comm.world > 1;
-    if (sharded) GP_TRY(pool_alloc((void**)&gd.agree_dev, sizeof(double), s->stream));
+    sharded = s->comm.world > 1;
+    if (sharded) GP_TRY(pool_alloc((void**)&agree_dev, sizeof(double), s->stream));
     // posterior predictive summaries: 3 accumulator planes (ldn x m), the cell code, per-item statistics, the per-respondent
     // partial sums, elpd per respondent + totals, and the illegal-value counter of y_holdout
-    constexpr int PRED_CHUNKS = 64;
-    const size_t pred_plane = (size_t)s->ldn * m;
-    double *pred_stats = nullptr, *pred_partial = nullptr, *pred_resp = nullptr;
+    pred_plane = (size_t)s->ldn * m;
     if (fit) {
-        GP_TRY(pool_alloc((void**)&gd.pred_acc, 3 * pred_plane * sizeof(double), s->stream));
-        GP_TRY(pool_alloc((void**)&gd.pred_code, (size_t)s->ldy8 * m, s->stream));
+        GP_TRY(pool_alloc((void**)&pred_acc, 3 * pred_plane * sizeof(double), s->stream));
+        GP_TRY(pool_alloc((void**)&pred_code, (size_t)s->ldy8 * m, s->stream));
         const size_t aux = (size_t)PRED_STATS * m + (size_t)PRED_CHUNKS * n + (size_t)n + PRED_STATS + 1;
-        GP_TRY(pool_alloc((void**)&gd.pred_aux, aux * sizeof(double), s->stream));
-        pred_stats = gd.pred_aux;
+        GP_TRY(pool_alloc((void**)&pred_aux, aux * sizeof(double), s->stream));
+        pred_stats = pred_aux;
         pred_partial = pred_stats + (size_t)PRED_STATS * m;
         pred_resp = pred_partial + (size_t)PRED_CHUNKS * n;
         unsigned long long* n_bad = reinterpret_cast<unsigned long long*>(pred_resp + n + PRED_STATS);
         GP_CUDA(cudaMemsetAsync(n_bad, 0, sizeof(unsigned long long), s->stream));
         // y_holdout goes up through the first accumulator plane (not in use before the first sampling iteration)
-        if (fit->y_holdout) GP_TRY(upload_pageable(gd.pred_acc, fit->y_holdout, nm * sizeof(double), s->stream));
-        GP_TRY(launch_predictive_code(s->stream, s->y8, s->ldy8, fit->y_holdout ? gd.pred_acc : nullptr, (int)n, (int)m,
-                                      gd.pred_code, n_bad));
+        if (fit->y_holdout) GP_TRY(upload_pageable(pred_acc, fit->y_holdout, nm * sizeof(double), s->stream));
+        GP_TRY(launch_predictive_code(s->stream, s->y8, s->ldy8, fit->y_holdout ? pred_acc : nullptr, (int)n, (int)m,
+                                      pred_code, n_bad));
         unsigned long long bad = 0;
         GP_CUDA(cudaMemcpyAsync(&bad, n_bad, sizeof(bad), cudaMemcpyDeviceToHost, s->stream));
         GP_CUDA(cudaStreamSynchronize(s->stream));
         double bad_all = (double)bad;
         if (sharded) {   // every rank refuses together: one that returned alone would leave its peers in the first collective
-            GP_CUDA(cudaMemcpyAsync(gd.agree_dev, &bad_all, sizeof(double), cudaMemcpyHostToDevice, s->stream));
-            GP_TRY(comm_allreduce_sum_f64(s->comm, gd.agree_dev, 1, s->stream));
-            GP_CUDA(cudaMemcpyAsync(&bad_all, gd.agree_dev, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+            GP_CUDA(cudaMemcpyAsync(agree_dev, &bad_all, sizeof(double), cudaMemcpyHostToDevice, s->stream));
+            GP_TRY(comm_allreduce_sum_f64(s->comm, agree_dev, 1, s->stream));
+            GP_CUDA(cudaMemcpyAsync(&bad_all, agree_dev, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
             GP_CUDA(cudaStreamSynchronize(s->stream));
         }
         if (bad_all != 0.0) {
@@ -1643,12 +1716,11 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
     }
     // IRF summaries: the Welford mean / M2 of P (2 planes of 1001 x m) and the tail heaps (K_lo + K_hi planes) in one
     // cudaMalloc, checked against the free device memory by arithmetic before the first sweep
-    const int64_t irf_cells = (int64_t)N_GRID * m;
-    const size_t irf_plane = (size_t)irf_cells;
-    double* const fs_out = irf ? irf->fstar_draws : nullptr;
-    const bool irf_bands = irf && (irf->lower || irf->upper) && sample_iterations > 0;
-    const IrfBandPlan irf_plan = irf_bands ? irf_band_plan(sample_iterations, irf->band) : IrfBandPlan{};
-    double *irf_lo = nullptr, *irf_hi = nullptr;
+    irf_cells = (int64_t)N_GRID * m;
+    irf_plane = (size_t)irf_cells;
+    fs_out = irf ? irf->fstar_draws : nullptr;
+    irf_bands = irf && (irf->lower || irf->upper) && S > 0;
+    irf_plan = irf_bands ? irf_band_plan(S, irf->band) : IrfBandPlan{};
     if (irf) {
         irf->band_bytes = 0;
         const double tail_bytes = 8.0 * (double)irf_cells * ((double)irf_plan.klo + (double)irf_plan.khi);
@@ -1666,214 +1738,155 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         }
         double short_all = need > (double)free_b ? 1.0 : 0.0;
         if (sharded) {   // every rank refuses together, as for y_holdout
-            GP_CUDA(cudaMemcpyAsync(gd.agree_dev, &short_all, sizeof(double), cudaMemcpyHostToDevice, s->stream));
-            GP_TRY(comm_allreduce_sum_f64(s->comm, gd.agree_dev, 1, s->stream));
-            GP_CUDA(cudaMemcpyAsync(&short_all, gd.agree_dev, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+            GP_CUDA(cudaMemcpyAsync(agree_dev, &short_all, sizeof(double), cudaMemcpyHostToDevice, s->stream));
+            GP_TRY(comm_allreduce_sum_f64(s->comm, agree_dev, 1, s->stream));
+            GP_CUDA(cudaMemcpyAsync(&short_all, agree_dev, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
             GP_CUDA(cudaStreamSynchronize(s->stream));
         }
         if (short_all != 0.0) {
             set_last_error("IRF bands at level %g over %d sampling iterations need %.0f bytes of device memory for their tail "
-                           "buffers (%.0f in all); %zu bytes are free on this device%s", irf->band, sample_iterations, tail_bytes,
+                           "buffers (%.0f in all); %zu bytes are free on this device%s", irf->band, S, tail_bytes,
                            need, free_b, need > (double)free_b ? "" : " (another rank lacks them)");
             return GPIRT_B200_ERR_NOMEM;
         }
-        const cudaError_t e = cudaMalloc((void**)&gd.irf_buf, (size_t)need);
+        const cudaError_t e = cudaMalloc((void**)&irf_buf, (size_t)need);
         if (e != cudaSuccess) {
             cudaGetLastError();
-            gd.irf_buf = nullptr;
+            irf_buf = nullptr;
             set_last_error("device allocation of %.0f bytes for the IRF summaries failed: %s", need, cudaGetErrorString(e));
             return GPIRT_B200_ERR_NOMEM;
         }
         irf->band_bytes = (int64_t)tail_bytes;
         if (irf_bands) {
-            irf_lo = gd.irf_buf + 2 * irf_plane;
+            irf_lo = irf_buf + 2 * irf_plane;
             irf_hi = irf_lo + (size_t)irf_plan.klo * irf_plane;
         }
         if (fs_out) {
-            for (int i = 0; i < 2; ++i) GP_TRY(pool_alloc((void**)&gd.snap_fs[i], irf_plane * sizeof(double), s->stream));
+            for (int i = 0; i < 2; ++i) GP_TRY(pool_alloc((void**)&snap_fs[i], irf_plane * sizeof(double), s->stream));
             // pinned bounce buffers large enough for an f* plane now: the storage worker must never reallocate them while
             // the other buffer's transfer is in flight (without pinned memory the plane goes by a plain copy)
-            g_bounce.ensure(std::max(keep_f ? nm : (size_t)0, irf_plane));
+            bo->ensure(std::max(keep_f ? nm : (size_t)0, irf_plane));
         }
     }
-    double t_c = now();
+    t_c = now();
     GP_TRY(s->init_draws());
-    double t_d = now();
-    // snapshot(slot): main stream copies theta | beta (and f, tightly packed) into buffer slot & 1 and records the event
-    auto snapshot = [&](int slot) -> int {
-        const int b = slot & 1;
-        GP_CUDA(cudaMemcpyAsync(gd.snap_small[b], s->theta, (size_t)n * sizeof(double), cudaMemcpyDeviceToDevice, s->stream));
-        GP_CUDA(cudaMemcpyAsync(gd.snap_small[b] + n, s->beta, 2 * (size_t)m * sizeof(double), cudaMemcpyDeviceToDevice, s->stream));
-        if (keep_f)
-            GP_CUDA(cudaMemcpy2DAsync(gd.snap_f[b], (size_t)n * sizeof(double), s->f, s->ldn * sizeof(double), (size_t)n * sizeof(double),
-                                      (size_t)m, cudaMemcpyDeviceToDevice, s->stream));
-        if (fs_out)
-            GP_CUDA(cudaMemcpy2DAsync(gd.snap_fs[b], N_GRID * sizeof(double), s->fstar, s->ldN * sizeof(double), N_GRID * sizeof(double),
-                                      (size_t)m, cudaMemcpyDeviceToDevice, s->stream));
-        GP_CUDA(cudaEventRecord(gd.ev[b], s->stream));
-        return GPIRT_B200_OK;
-    };
+    t_d = now();
     // drain(slot), on the storage worker: the copy stream waits for the snapshot, then the worker blocks in the
     // device-to-host copies.  The sampler's status words (Cholesky / ESS failure) ride along, so a failed chain is noticed
     // at the next stored slot instead of spinning every item through the ESS iteration cap for the rest of the run.
-    gd.worker = new StoreWorker();
-    StoreWorker& worker = *gd.worker;
-    GP_CUDA(cudaGetDevice(&worker.device));
+    worker = new StoreWorker();
+    GP_CUDA(cudaGetDevice(&worker->device));
     // issue(slot): the copy stream waits for the snapshot and gets every device-to-host transfer of the slot (status words,
     // theta | beta into pinned staging, f in pieces into the pinned bounce buffer); finish(slot): the host copies.
     // The worker issues slot k+1 (other snapshot / bounce / staging buffers) before it finishes slot k, so the PCIe transfer
     // of one slice runs under the host copies of the previous one.
-    BounceXfer xfer[2];
-    worker.issue = [&](int slot) -> int {            // theta_draws.row(slot), beta_draws.slice(slot), f_draws.slice(slot)
+    worker->issue = [this](int slot) -> int {            // theta_draws.row(slot), beta_draws.slice(slot), f_draws.slice(slot)
         const int b = slot & 1;
-        GP_CUDA(cudaStreamWaitEvent(gd.copy, gd.ev[b], 0));
-        GP_CUDA(cudaMemcpyAsync((void*)w_poll, s->status, 4 * sizeof(int), cudaMemcpyDeviceToHost, gd.copy));
-        GP_CUDA(cudaMemcpyAsync(gd.h_small[b], gd.snap_small[b], n_small * sizeof(double), cudaMemcpyDeviceToHost, gd.copy));
-        GP_CUDA(cudaEventRecord(gd.ev_small[b], gd.copy));
-        if (keep_f) GP_TRY(bounce_issue(f_out + (size_t)slot * nm, gd.snap_f[b], nm, b, gd.copy, xfer[b]));
+        GP_CUDA(cudaStreamWaitEvent(copy, ev[b], 0));
+        GP_CUDA(cudaMemcpyAsync((void*)w_poll, s->status, 4 * sizeof(int), cudaMemcpyDeviceToHost, copy));
+        GP_CUDA(cudaMemcpyAsync(h_small[b], snap_small[b], n_small * sizeof(double), cudaMemcpyDeviceToHost, copy));
+        GP_CUDA(cudaEventRecord(ev_small[b], copy));
+        if (keep_f) GP_TRY(bounce_issue(*bo, copy_threads, f_out + (size_t)slot * nm, snap_f[b], nm, b, copy, xfer[b]));
         return GPIRT_B200_OK;
     };
-    worker.finish = [&, n_slots](int slot) -> int {
+    worker->finish = [this](int slot) -> int {
         const double ts0 = now();
         const int b = slot & 1;
         if (keep_f) GP_TRY(bounce_finish(b, xfer[b]));
-        GP_CUDA(cudaEventSynchronize(gd.ev_small[b]));
-        const double* small = gd.h_small[b];
+        GP_CUDA(cudaEventSynchronize(ev_small[b]));
+        const double* small = h_small[b];
         for (int64_t i = 0; i < n; ++i) theta_out[(size_t)i * n_slots + slot] = small[i];
         std::memcpy(beta_out + (size_t)slot * 2 * m, small + n, 2 * (size_t)m * sizeof(double));
         if (fs_out) {   // the f* plane after this slot's f slice, through the same bounce buffer (its DMA has landed)
             double* dst = fs_out + (size_t)slot * irf_plane;
-            if (irf_plane <= g_bounce.cap) GP_TRY(chunked_d2h(dst, gd.snap_fs[b], irf_plane, b, gd.copy));
+            if (irf_plane <= bo->cap) GP_TRY(d2h(dst, snap_fs[b], irf_plane, b));
             else {
-                GP_CUDA(cudaMemcpyAsync(dst, gd.snap_fs[b], irf_plane * sizeof(double), cudaMemcpyDeviceToHost, gd.copy));
-                GP_CUDA(cudaStreamSynchronize(gd.copy));
+                GP_CUDA(cudaMemcpyAsync(dst, snap_fs[b], irf_plane * sizeof(double), cudaMemcpyDeviceToHost, copy));
+                GP_CUDA(cudaStreamSynchronize(copy));
             }
         }
-        worker.busy_s += now() - ts0;
+        worker->busy_s += now() - ts0;
         return GPIRT_B200_OK;
     };
-    worker.start();
-    struct WorkerStop {   // declared after everything the drain closure refers to: the worker is joined before any of it dies
-        StoreWorker* w;
-        bool trace;
-        ~WorkerStop() {
-            timespec a, b;
-            clock_gettime(CLOCK_MONOTONIC, &a);
-            w->stop();
-            clock_gettime(CLOCK_MONOTONIC, &b);
-            if (trace) fprintf(stderr, "gpirt_b200_mcmc: storage thread joined in %.3fs\n", (b.tv_sec - a.tv_sec) + 1e-9 * (b.tv_nsec - a.tv_nsec));
-        }
-    } worker_stop{gd.worker, trace};
-    // Stopping early (interrupt from the progress callback, failed Cholesky / ESS seen in the polled status words, a failed
-    // store) must be a COMMON decision when items are sharded: a rank that returned alone would leave its peers blocked in
-    // the next sweep's collectives.  Every rank therefore enqueues, every 8th iteration, a one-word all-reduce of its local
-    // stop request on the sampler's stream and acts on the agreed value after the host sync that follows it — the same
-    // program point on every rank.  An unsharded chain stops as soon as it sees a reason.
-    bool want_stop = false;
-    int stop_code = GPIRT_B200_OK;
-    auto local_stop_code = [&]() -> int {
-        std::string msg;
-        const int wrc = worker.status(&msg);
-        if (wrc != GPIRT_B200_OK) { set_last_error("%s", msg.c_str()); return wrc; }
-        if (gd.h_poll[0] || w_poll[0]) { set_last_error("chol(): decomposition failed"); return GPIRT_B200_ERR_NOT_PD; }
-        if (gd.h_poll[1] || w_poll[1]) { set_last_error("elliptical slice sampler did not terminate (NaN log-likelihood?)"); return GPIRT_B200_ERR_ESS; }
-        if (want_stop) { set_last_error("interrupted by the progress callback"); return GPIRT_B200_ERR_INTERRUPT; }
-        return GPIRT_B200_OK;
-    };
-    auto enqueue_agreement = [&]() -> int {
-        if (!sharded) return GPIRT_B200_OK;
-        const double mine = local_stop_code() != GPIRT_B200_OK ? 1.0 : 0.0;   // pageable source: staged at call time
-        GP_CUDA(cudaMemcpyAsync(gd.agree_dev, &mine, sizeof(double), cudaMemcpyHostToDevice, s->stream));
-        GP_TRY(comm_allreduce_sum_f64(s->comm, gd.agree_dev, 1, s->stream));
-        GP_CUDA(cudaMemcpyAsync(h_ring + (agree_count & 7), gd.agree_dev, sizeof(double), cudaMemcpyDeviceToHost, s->stream));
-        agree_count += 1;
-        return GPIRT_B200_OK;
-    };
-    auto stop_now = [&](int agreement) -> bool {   // after a host sync that covers agreement number `agreement`
-        stop_code = local_stop_code();
-        if (sharded) {
-            if (agreement < 0 || h_ring[agreement & 7] == 0.0) return false;
-            if (stop_code == GPIRT_B200_OK) { set_last_error("stopped: another rank was interrupted or failed"); stop_code = GPIRT_B200_ERR_INTERRUPT; }
-            return true;
-        }
-        return stop_code != GPIRT_B200_OK;
-    };
+    worker->start();
     GP_TRY(snapshot(0));                                                            // :53-55 initial values
-    worker.push(0);
-    const int total = sample_iterations + burn_iterations;
-    const double inc = total > 0 ? 100.0 / total : 0.0;
-    double progress = 0.0;
-    int n_summarised = 0;
-    for (int iter = 0; iter < total; ++iter) {
-        if (cb && cb(progress, cb_ctx)) want_stop = true;                           // Rcpp::checkUserInterrupt, :66,85
-        if (!sharded && stop_now(-1)) return stop_code;                             // interrupt, failed store, failed chain seen by the worker
-        progress += inc;
-        const bool sampling = iter >= burn_iterations;
-        const int si = iter - burn_iterations + 1;                                  // 1-based sampling iteration
-        const bool store = sampling && si % thin == 0;
-        GP_TRY(s->sweep(sampling ? 1 : 0));                                         // enqueue sweep (asynchronous)
-        if (sampling && summarise_f) {
-            dim3 grid((unsigned)m, (unsigned)ceil_div(n, 256));
-            GP_LAUNCH(k_f_welford, grid, 256, 0, s->stream, s->f, s->ldn, (int)n, (double)(++n_summarised), gd.f_mean, gd.f_m2);
-        }
-        if (sampling && fit)
-            GP_TRY(launch_predictive_accumulate(s->stream, s->f, s->ldn, gd.pred_code, s->ldy8, s->theta, s->beta, (int)n, (int)m,
-                                                (double)si, gd.pred_acc));
-        if (sampling && irf)   // the f* this sweep drew (fstar, not the means in Dmat); nothing on a side stream writes it
-            GP_TRY(launch_irf_accumulate(s->stream, s->fstar, s->ldN, N_GRID, irf_cells, si, gd.irf_buf, gd.irf_buf + irf_plane,
-                                         irf_lo, irf_plan.klo, irf_hi, irf_plan.khi));
-        if (store) {
-            const int slot = si / thin;                                             // :99-103
-            worker.wait_buffer_free(slot & 1);                                      // slot - 2 has left this snapshot buffer
-            GP_TRY(snapshot(slot));
-            worker.push(slot);
-        }
-        if ((iter & 7) == 7) {                                                      // bounded run-ahead; progress / interrupts stay honest
-            GP_TRY(enqueue_agreement());
-            GP_CUDA(cudaMemcpyAsync(gd.h_poll, s->status, 4 * sizeof(int), cudaMemcpyDeviceToHost, s->stream));
-            GP_CUDA(cudaStreamSynchronize(s->stream));
-            if (stop_now(agree_count - 1)) return stop_code;
-        }
+    worker->push(0);
+    return GPIRT_B200_OK;
+}
+
+int ChainRun::iterate(int iter) {
+    const bool sampling = iter >= B;
+    const int si = iter - B + 1;                                                    // 1-based sampling iteration
+    const bool store = sampling && si % thin == 0;
+    GP_TRY(s->sweep(sampling ? 1 : 0));                                             // enqueue sweep (asynchronous)
+    if (sampling && summarise_f) {
+        dim3 grid((unsigned)m, (unsigned)ceil_div(n, 256));
+        GP_LAUNCH(k_f_welford, grid, 256, 0, s->stream, s->f, s->ldn, (int)n, (double)(++n_summarised), f_mean, f_m2);
     }
-    worker.wait_idle();
-    const double t_store = worker.busy_s;
+    if (sampling && fit)
+        GP_TRY(launch_predictive_accumulate(s->stream, s->f, s->ldn, pred_code, s->ldy8, s->theta, s->beta, (int)n, (int)m,
+                                            (double)si, pred_acc));
+    if (sampling && irf)   // the f* this sweep drew (fstar, not the means in Dmat); nothing on a side stream writes it
+        GP_TRY(launch_irf_accumulate(s->stream, s->fstar, s->ldN, N_GRID, irf_cells, si, irf_buf, irf_buf + irf_plane,
+                                     irf_lo, irf_plan.klo, irf_hi, irf_plan.khi));
+    if (sampling && (diag_trace || diag_halves))   // theta | beta as the snapshot would copy them, and f* as above
+        GP_TRY(launch_chain_halves(s->stream, s->fstar, s->ldN, N_GRID, irf_cells, si, S, diag_halves, s->theta, (int)n,
+                                   s->beta, 2 * (int)m, diag_trace));
+    if (store) {
+        const int slot = si / thin;                                                 // :99-103
+        worker->wait_buffer_free(slot & 1);                                         // slot - 2 has left this snapshot buffer
+        GP_TRY(snapshot(slot));
+        worker->push(slot);
+    }
+    if ((iter & 7) == 7) {                                                          // bounded run-ahead; progress / interrupts stay honest
+        GP_TRY(enqueue_agreement());
+        GP_CUDA(cudaMemcpyAsync(h_poll, s->status, 4 * sizeof(int), cudaMemcpyDeviceToHost, s->stream));
+        GP_CUDA(cudaStreamSynchronize(s->stream));
+        if (stop_now(agree_count - 1)) return stop_code;
+    }
+    return GPIRT_B200_OK;
+}
+
+int ChainRun::finish() {
+    worker->wait_idle();
+    const double t_store = worker->busy_s;
     {
         std::string msg;
-        const int wrc = worker.status(&msg);
+        const int wrc = worker->status(&msg);
         if (wrc != GPIRT_B200_OK) { set_last_error("%s", msg.c_str()); return wrc; }
     }
-    GP_CUDA(cudaMemcpyAsync(gd.h_poll, s->status, 4 * sizeof(int), cudaMemcpyDeviceToHost, s->stream));
+    GP_CUDA(cudaMemcpyAsync(h_poll, s->status, 4 * sizeof(int), cudaMemcpyDeviceToHost, s->stream));
     GP_CUDA(cudaStreamSynchronize(s->stream));
     if (!sharded && stop_now(-1)) return stop_code;
     GP_TRY(s->check_status());
     {
         int h[4] = {0, 0, 0, 0};
         GP_CUDA(cudaMemcpy(h, s->status, sizeof(h), cudaMemcpyDeviceToHost));
-        g_last_degenerate_theta = h[2];   // theta draws whose CDF was degenerate (grid point 0 taken; the reference reads out of bounds there)
+        degenerate = h[2];   // theta draws whose CDF was degenerate (grid point 0 taken; the reference reads out of bounds there)
     }
     // IRFs = plogis(IRFs / S)   (:106-111; S = 0 gives NaN exactly as the reference's 0 * inf)
-    const double inv = 1.0 / (double)sample_iterations;
+    const double inv = 1.0 / (double)S;
     GP_TRY(launch_irf_finish(s->stream, s->irf_sum, s->ldN, N_GRID, (int)m, inv, s->Dmat));
     GP_CUDA(cudaMemcpyAsync(irf_out, s->Dmat, (size_t)N_GRID * m * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
     if (summarise_f) {
         if (n_summarised == 0) {
-            GP_CUDA(cudaMemsetAsync(gd.f_mean, 0xff, nm * sizeof(double), s->stream));   // all-ones bit pattern = NaN: no sampling iterations
-            GP_CUDA(cudaMemsetAsync(gd.f_m2, 0xff, nm * sizeof(double), s->stream));
+            GP_CUDA(cudaMemsetAsync(f_mean, 0xff, nm * sizeof(double), s->stream));   // all-ones bit pattern = NaN: no sampling iterations
+            GP_CUDA(cudaMemsetAsync(f_m2, 0xff, nm * sizeof(double), s->stream));
         } else {
-            GP_LAUNCH(k_f_sd, (unsigned)ceil_div((int64_t)nm, 256), 256, 0, s->stream, gd.f_m2, nm, (double)(n_summarised - 1));
+            GP_LAUNCH(k_f_sd, (unsigned)ceil_div((int64_t)nm, 256), 256, 0, s->stream, f_m2, nm, (double)(n_summarised - 1));
         }
         // fresh pageable destinations: the chunked pinned-bounce copy with host threads, as for the f draws
         GP_CUDA(cudaStreamSynchronize(s->stream));
-        if (f_mean_out) GP_TRY(chunked_d2h(f_mean_out, gd.f_mean, nm, 0, gd.copy));
-        if (f_sd_out) GP_TRY(chunked_d2h(f_sd_out, gd.f_m2, nm, 1, gd.copy));
+        if (f_mean_out) GP_TRY(d2h(f_mean_out, f_mean, nm, 0));
+        if (f_sd_out) GP_TRY(d2h(f_sd_out, f_m2, nm, 1));
     }
     if (fit) {
-        const double S = (double)sample_iterations;
-        if (sample_iterations == 0) {   // NaN accumulators: every output NaN, the cell counts still hold
-            GP_CUDA(cudaMemsetAsync(gd.pred_acc, 0xff, pred_plane * sizeof(double), s->stream));
-            GP_CUDA(cudaMemsetAsync(gd.pred_acc + 2 * pred_plane, 0xff, pred_plane * sizeof(double), s->stream));
+        const double Sd = (double)S;
+        if (S == 0) {   // NaN accumulators: every output NaN, the cell counts still hold
+            GP_CUDA(cudaMemsetAsync(pred_acc, 0xff, pred_plane * sizeof(double), s->stream));
+            GP_CUDA(cudaMemsetAsync(pred_acc + 2 * pred_plane, 0xff, pred_plane * sizeof(double), s->stream));
         }
-        GP_TRY(launch_predictive_reduce(s->stream, gd.pred_acc, s->ldn, gd.pred_code, s->ldy8, (int)n, (int)m, S, pred_stats,
+        GP_TRY(launch_predictive_reduce(s->stream, pred_acc, s->ldn, pred_code, s->ldy8, (int)n, (int)m, Sd, pred_stats,
                                         pred_partial, PRED_CHUNKS, pred_resp));
         if (sharded) GP_TRY(comm_allreduce_sum_f64(s->comm, pred_resp, (size_t)n + PRED_STATS, s->stream));
         double tot[PRED_STATS];
@@ -1884,9 +1897,9 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         double* const outs[3] = {fit->pred, fit->lpd_cell, fit->pwaic_cell};
         for (int w = 0; w < 3; ++w) {
             if (!outs[w]) continue;
-            GP_TRY(launch_predictive_cells(s->stream, gd.pred_acc, s->ldn, gd.pred_code, s->ldy8, (int)n, (int)m, S, w, gd.pred_acc + pred_plane));
+            GP_TRY(launch_predictive_cells(s->stream, pred_acc, s->ldn, pred_code, s->ldy8, (int)n, (int)m, Sd, w, pred_acc + pred_plane));
             GP_CUDA(cudaStreamSynchronize(s->stream));
-            GP_TRY(chunked_d2h(outs[w], gd.pred_acc + pred_plane, nm, 0, gd.copy));
+            GP_TRY(d2h(outs[w], pred_acc + pred_plane, nm, 0));
         }
         GP_CUDA(cudaStreamSynchronize(s->stream));
         const double N = tot[5], sum_e = tot[2], var = (tot[3] - sum_e * sum_e / N) / (N - 1.0);
@@ -1895,31 +1908,227 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
         fit->elpd_waic = tot[0] - tot[1];
         fit->waic = -2.0 * fit->elpd_waic;
         fit->se_elpd_waic = std::sqrt(N * (var < 0.0 ? 0.0 : var));   // loo's convention; NaN stays NaN
-        fit->lpd_holdout = sample_iterations ? tot[4] : NAN;   // S = 0: NaN even where no cell is held out
+        fit->lpd_holdout = S ? tot[4] : NAN;   // S = 0: NaN even where no cell is held out
         fit->n_obs = (int64_t)tot[5];
         fit->n_holdout = (int64_t)tot[6];
     }
     if (irf) {
-        double* const mean = gd.irf_buf;
+        double* const mean = irf_buf;
         double* const m2 = mean + irf_plane;
-        if (sample_iterations == 0) {   // all-ones bit pattern = NaN: no sampling iterations
+        if (S == 0) {   // all-ones bit pattern = NaN: no sampling iterations
             GP_CUDA(cudaMemsetAsync(mean, 0xff, 2 * irf_plane * sizeof(double), s->stream));
         } else {   // sd over M2 in place; the band ends over heap slot 0 of each heap (read before written, per cell)
-            GP_TRY(launch_irf_finish_bands(s->stream, irf_cells, sample_iterations, m2, m2, irf_lo, irf_hi, irf_plan, true,
+            GP_TRY(launch_irf_finish_bands(s->stream, irf_cells, S, m2, m2, irf_lo, irf_hi, irf_plan, true,
                                            irf_lo, irf_hi));
         }
         GP_CUDA(cudaStreamSynchronize(s->stream));
-        if (irf->prob_mean) GP_TRY(chunked_d2h(irf->prob_mean, mean, irf_plane, 0, gd.copy));
-        if (irf->prob_sd) GP_TRY(chunked_d2h(irf->prob_sd, m2, irf_plane, 1, gd.copy));
-        if (irf->lower) GP_TRY(chunked_d2h(irf->lower, irf_bands ? irf_lo : m2, irf_plane, 0, gd.copy));   // S = 0: the NaN plane
-        if (irf->upper) GP_TRY(chunked_d2h(irf->upper, irf_bands ? irf_hi : m2, irf_plane, 1, gd.copy));
+        if (irf->prob_mean) GP_TRY(d2h(irf->prob_mean, mean, irf_plane, 0));
+        if (irf->prob_sd) GP_TRY(d2h(irf->prob_sd, m2, irf_plane, 1));
+        if (irf->lower) GP_TRY(d2h(irf->lower, irf_bands ? irf_lo : m2, irf_plane, 0));   // S = 0: the NaN plane
+        if (irf->upper) GP_TRY(d2h(irf->upper, irf_bands ? irf_hi : m2, irf_plane, 1));
     }
     GP_CUDA(cudaStreamSynchronize(s->stream));
-    if (cb) cb(100.0, cb_ctx);
     if (trace)
         fprintf(stderr, "gpirt_b200_mcmc: create %.3fs, copy buffers %.3fs, init draws %.3fs, %d sweeps + stores %.3fs (stores %.3fs)\n",
-                t_b - t_a, t_c - t_b, t_d - t_c, total, now() - t_d, t_store);
-    exit_trace.t_body_end = now();
+                t_b - t_a, t_c - t_b, t_d - t_c, S + B, now() - t_d, t_store);
+    return GPIRT_B200_OK;
+}
+
+// Several chains in one call (opts.chains): C ChainRuns on the current device, each with its own seed, sampler, streams,
+// graph, snapshot buffers and storage worker; this thread enqueues sweep t of chain 0, 1, ..., C - 1 in turn, so no two
+// chains' graph captures interleave.  Diagnostics over all S sampling iterations on the device (k_chain_diag,
+// k_chain_irf_rhat) after the last sweep.
+int mcmc_chains(const double* y, int64_t n, int64_t m, const double* theta_init, int S, int B, const double* pm,
+                const double* psd, const double* pstep, const gpirt_b200_opts* opts, double* theta_out, double* beta_out,
+                double* f_out, double* irf_out, gpirt_b200_progress_cb cb, void* cb_ctx, bool trace) {
+    gpirt_b200_chains* const ch = opts->chains;
+    ch->diag_bytes = 0;
+    const int C = ch->chains;
+    if (C < 1 || C > 32) { set_last_error("bad argument: chains must lie in [1, 32], got %d", C); return GPIRT_B200_ERR_ARG; }
+    if (opts->world_size > 1) { set_last_error("several chains with items sharded across GPUs are not built"); return GPIRT_B200_ERR_ARG; }
+    if (opts->fit || opts->irf || opts->f_mean_out || opts->f_sd_out) {
+        set_last_error("fit, irf, f_mean_out and f_sd_out are not built for several chains");
+        return GPIRT_B200_ERR_ARG;
+    }
+    if (!theta_init) { set_last_error("bad argument: theta_init is NULL"); return GPIRT_B200_ERR_ARG; }
+    const bool want_diag = ch->theta_rhat || ch->theta_ess || ch->beta_rhat || ch->beta_ess;
+    const bool diag_on = S >= 4;                          // fewer iterations: every diagnostic is NaN
+    const int64_t P = n + 2 * m, cells = (int64_t)N_GRID * m;
+    const size_t trace_elems = want_diag && diag_on ? (size_t)S * P * C : 0;
+    const size_t halves_elems = ch->irf_rhat && diag_on ? (size_t)4 * cells * C : 0;
+    const size_t out_elems = (trace_elems ? 2 * (size_t)P : 0) + (halves_elems ? (size_t)cells : 0);
+    ch->diag_bytes = (int64_t)((trace_elems + halves_elems) * sizeof(double));
+    const int threads = host_threads_for_copy(C);
+    int dev = 0;
+    if (opts->device >= 0) GP_CUDA(cudaSetDevice(opts->device));
+    GP_CUDA(cudaGetDevice(&dev));
+    cudaMemPool_t pool;
+    GP_CUDA(cudaDeviceGetDefaultMemPool(&pool, dev));
+    // Destroyed last: the diagnostics buffer is freed, and with C > 1 the pool is trimmed so that C samplers' memory does
+    // not stay reserved on a shared device after the call.
+    struct CallEnd {
+        int C; cudaMemPool_t pool; double* diag = nullptr;
+        ~CallEnd() {
+            if (diag) cudaFree(diag);
+            if (C > 1) { cudaDeviceSynchronize(); cudaMemPoolTrimTo(pool, 0); }
+        }
+    } end{C, pool};
+    if (C > 1) { GP_CUDA(cudaDeviceSynchronize()); GP_CUDA(cudaMemPoolTrimTo(pool, 0)); }
+    struct OwnBounces {                                   // pinned staging of chains 1..C-1 (chain 0: g_bounce)
+        std::unique_ptr<Bounce[]> b;
+        int C;
+        ~OwnBounces() {
+            for (int c = 1; c < C; ++c) {
+                b[c].release();
+                for (auto& v : b[c].ev) for (cudaEvent_t e : v) cudaEventDestroy(e);
+            }
+        }
+    } own{std::unique_ptr<Bounce[]>(new Bounce[C]), C};
+    std::vector<gpirt_b200_opts> copt(C, *opts);
+    std::vector<std::unique_ptr<ChainRun>> runs;
+    for (int c = 0; c < C; ++c) {
+        copt[c].seed = ch->seeds ? ch->seeds[c] : opts->seed + (uint64_t)c;
+        copt[c].chains = nullptr;
+        const size_t slots = (size_t)((opts->thin > 1 ? S / opts->thin : S) + 1);
+        runs.emplace_back(new ChainRun{y, n, m, theta_init + (size_t)c * n, S, B, pm, psd, pstep, &copt[c],
+                                       theta_out + (size_t)c * slots * n, beta_out + (size_t)c * 2 * m * slots,
+                                       f_out ? f_out + (size_t)c * slots * n * m : nullptr, irf_out + (size_t)c * cells,
+                                       c == 0 ? &g_bounce : &own.b[c], threads, trace && c == 0});
+        runs[c]->untraced = c > 0;
+    }
+    auto failed = [&](int c, int rc) {
+        const std::string msg = last_error();
+        set_last_error("chain %d: %s", c, msg.c_str());
+        return rc;
+    };
+    // Memory, before the first sweep: chain 0's footprint is the drop of free device memory across its set-up; the other
+    // chains and the diagnostics must fit in what is left.
+    size_t free0 = 0, free1 = 0, total = 0;
+    GP_CUDA(cudaMemGetInfo(&free0, &total));
+    if (int rc = runs[0]->setup()) return failed(0, rc);
+    GP_CUDA(cudaStreamSynchronize(runs[0]->s->stream));
+    GP_CUDA(cudaMemGetInfo(&free1, &total));
+    const double footprint = free0 > free1 ? (double)(free0 - free1) : 0.0;
+    const double need = (C - 1) * footprint + (double)(trace_elems + halves_elems + out_elems) * sizeof(double);
+    if (need > (double)free1) {
+        set_last_error("%d chains need %.0f more bytes of device memory (%.0f per further chain, %lld for the diagnostics); "
+                       "%zu bytes are free on this device", C, need, footprint, (long long)ch->diag_bytes, free1);
+        return GPIRT_B200_ERR_NOMEM;
+    }
+    double *trace_dev = nullptr, *halves_dev = nullptr, *out_dev = nullptr;
+    if (const size_t elems = trace_elems + halves_elems + out_elems) {
+        const cudaError_t e = cudaMalloc((void**)&end.diag, elems * sizeof(double));
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            end.diag = nullptr;
+            set_last_error("device allocation of %zu bytes for the chain diagnostics failed: %s", elems * sizeof(double), cudaGetErrorString(e));
+            return GPIRT_B200_ERR_NOMEM;
+        }
+        trace_dev = trace_elems ? end.diag : nullptr;
+        halves_dev = halves_elems ? end.diag + trace_elems : nullptr;
+        out_dev = end.diag + trace_elems + halves_elems;
+    }
+    for (int c = 0; c < C; ++c) {
+        if (trace_dev) runs[c]->diag_trace = trace_dev + (size_t)c * P * S;
+        if (halves_dev) runs[c]->diag_halves = halves_dev + (size_t)c * 4 * cells;
+        if (c > 0) if (int rc = runs[c]->setup()) return failed(c, rc);
+    }
+    const int total_it = S + B;
+    const double inc = total_it > 0 ? 100.0 / total_it : 0.0;
+    double progress = 0.0;
+    for (int iter = 0; iter < total_it; ++iter) {
+        if (cb && cb(progress, cb_ctx)) for (auto& r : runs) r->want_stop = true;   // Rcpp::checkUserInterrupt, :66,85
+        for (int c = 0; c < C; ++c) if (runs[c]->stopped()) return failed(c, runs[c]->stop_code);
+        progress += inc;
+        for (int c = 0; c < C; ++c) if (int rc = runs[c]->iterate(iter)) return failed(c, rc);
+    }
+    int64_t degenerate = 0;
+    for (int c = 0; c < C; ++c) {
+        const int rc = runs[c]->finish();
+        degenerate += runs[c]->degenerate;
+        g_last_degenerate_theta = degenerate;
+        if (rc != GPIRT_B200_OK) return failed(c, rc);
+    }
+    // every chain's stream has drained (finish): the diagnostics run on chain 0's
+    cudaStream_t st = runs[0]->s->stream;
+    auto put = [&](double* dst, const double* src, size_t count) -> int {
+        if (!dst) return GPIRT_B200_OK;
+        if (!src) { std::fill(dst, dst + count, (double)NAN); return GPIRT_B200_OK; }
+        GP_CUDA(cudaMemcpyAsync(dst, src, count * sizeof(double), cudaMemcpyDeviceToHost, st));
+        return GPIRT_B200_OK;
+    };
+    double *rhat_dev = nullptr, *ess_dev = nullptr, *irf_rhat_dev = nullptr;
+    if (trace_dev) {
+        rhat_dev = out_dev;
+        ess_dev = out_dev + P;
+        GP_TRY(launch_chain_diag(st, trace_dev, (int)P, S, C, rhat_dev, ess_dev));
+    }
+    if (halves_dev) {
+        irf_rhat_dev = out_dev + (trace_dev ? 2 * P : 0);
+        GP_TRY(launch_chain_irf_rhat(st, halves_dev, cells, S, C, irf_rhat_dev));
+    }
+    GP_TRY(put(ch->theta_rhat, rhat_dev, (size_t)n));
+    GP_TRY(put(ch->theta_ess, ess_dev, (size_t)n));
+    GP_TRY(put(ch->beta_rhat, rhat_dev ? rhat_dev + n : nullptr, 2 * (size_t)m));
+    GP_TRY(put(ch->beta_ess, ess_dev ? ess_dev + n : nullptr, 2 * (size_t)m));
+    GP_TRY(put(ch->irf_rhat, irf_rhat_dev, (size_t)cells));
+    GP_CUDA(cudaStreamSynchronize(st));
+    if (cb) cb(100.0, cb_ctx);
+    return GPIRT_B200_OK;
+}
+}  // namespace
+
+int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_init, int sample_iterations,
+                    int burn_iterations, const double* pm, const double* psd, const double* pstep,
+                    const gpirt_b200_opts* opts, double* theta_out, double* beta_out, double* f_out, double* irf_out,
+                    gpirt_b200_progress_cb cb, void* cb_ctx) {
+    if (sample_iterations < 0 || burn_iterations < 0 || !theta_out || !beta_out || !irf_out) {
+        set_last_error("bad argument: negative iteration count or null output");
+        return GPIRT_B200_ERR_ARG;
+    }
+    const bool keep_f = !(opts && opts->skip_f_draws);
+    if (keep_f && !f_out) { set_last_error("f_out is NULL but f draws were requested"); return GPIRT_B200_ERR_ARG; }
+    if (opts && opts->thin < 0) { set_last_error("bad argument: thin < 0"); return GPIRT_B200_ERR_ARG; }
+    gpirt_b200_irf* const irf = opts ? opts->irf : nullptr;
+    if (irf && (irf->lower || irf->upper) && !(std::isfinite(irf->band) && irf->band > 0.0 && irf->band < 1.0)) {
+        set_last_error("bad argument: the IRF band level must lie in (0, 1), got %g", irf->band);
+        return GPIRT_B200_ERR_ARG;
+    }
+    const bool trace = getenv("GPIRT_TIMING") != nullptr;
+    g_last_degenerate_theta = 0;
+    struct ExitTrace {   // first local: destroyed last
+        bool on; double t_enter; double t_body_end = 0.0;
+        ~ExitTrace() {
+            if (!on) return;
+            const double t = ChainRun::now();
+            fprintf(stderr, "gpirt_b200_mcmc: total %.3fs in the call, %.3fs after the body\n", t - t_enter, t_body_end > 0.0 ? t - t_body_end : 0.0);
+        }
+    } exit_trace{trace, ChainRun::now()};
+    // the pinned bounce buffers are process-wide: a call that moves f through them owns them until it returns
+    std::unique_lock<std::mutex> bounce_lock(g_bounce_mu);
+    if (opts && opts->chains) {
+        const int rc = mcmc_chains(y, n, m, theta_init, sample_iterations, burn_iterations, pm, psd, pstep, opts, theta_out,
+                                   beta_out, f_out, irf_out, cb, cb_ctx, trace);
+        exit_trace.t_body_end = ChainRun::now();
+        return rc;
+    }
+    ChainRun run{y, n, m, theta_init, sample_iterations, burn_iterations, pm, psd, pstep, opts, theta_out, beta_out, f_out,
+                 irf_out, &g_bounce, host_threads_for_copy(1), trace};
+    GP_TRY(run.setup());
+    const int total = sample_iterations + burn_iterations;
+    const double inc = total > 0 ? 100.0 / total : 0.0;
+    double progress = 0.0;
+    for (int iter = 0; iter < total; ++iter) {
+        if (cb && cb(progress, cb_ctx)) run.want_stop = true;                      // Rcpp::checkUserInterrupt, :66,85
+        if (run.stopped()) return run.stop_code;
+        progress += inc;
+        GP_TRY(run.iterate(iter));
+    }
+    const int rc = run.finish();
+    g_last_degenerate_theta = run.degenerate;
+    if (rc != GPIRT_B200_OK) return rc;
+    if (cb) cb(100.0, cb_ctx);
+    exit_trace.t_body_end = ChainRun::now();
     return GPIRT_B200_OK;
 }
 

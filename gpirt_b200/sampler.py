@@ -10,7 +10,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import Fit, GpirtError, Irf, Opts, N_GRID
+from ._lib import Chains, Fit, GpirtError, Irf, Opts, N_GRID
 from .response_matrix import DEFAULT_CODES, as_response_matrix
 
 
@@ -48,7 +48,7 @@ def nccl_unique_id():
 def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_prior_means=None, beta_prior_sds=None,
               beta_proposal_sds=None, theta_init=None, *, seed=None, progress=None, store_f=True, fstar_mode=0,
               device=-1, shard=None, thin=1, f_summary=False, use_graph=0, predictive=False, y_holdout=None,
-              irf_band=None, store_fstar=False):
+              irf_band=None, store_fstar=False, chains=None, chain_diagnostics=False):
     """Drop-in for the reference's gpirtMCMC().  Keyword-only extras (not in the reference): seed (Philox key; default
     drawn from numpy's global RNG, as the R shim draws it from R's), progress(percent) -> truthy to interrupt,
     store_f=False to skip the n*m*(S+1) f draws, shard=(rank, world, m_global, item_offset, unique_id) for item
@@ -63,26 +63,59 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
     irf_band=b (0 < b < 1) to also return "IRF_summary": dict(mean, sd, lower, upper) of P(y = +1 | theta*) on the grid
     (1001 x m, over all sampling iterations; lower / upper are the exact pointwise type-7 quantiles at (1 -+ b) / 2 of f*
     mapped through plogis), band = b and band_bytes = the device memory of its tail buffers; store_fstar=True to also return
-    the f* draws "fstar" (1001 x m x slots, the slots of theta / beta).  With shard both cover the local items."""
+    the f* draws "fstar" (1001 x m x slots, the slots of theta / beta).  With shard both cover the local items.
+    chains=C (1..32) runs C chains concurrently on one GPU in this call: theta_init may be n x C (None: each chain's drawn
+    from numpy's global RNG), an integer seed gives chain c the seed seed + c (chain 0 equals a call with that seed), a
+    sequence of C seeds is used as given, and theta, beta, f and IRFs gain a trailing chain axis.  chain_diagnostics=True
+    also returns "diagnostics": dict(theta_rhat, theta_ess (n), beta_rhat, beta_ess (2 x m), irf_rhat (1001 x m),
+    diag_bytes), split-R-hat and summed Geyer ESS over all S sampling iterations (any thin), computed on the device
+    (definitions in include/gpirt_b200.h).  chains cannot be combined with shard, predictive, irf_band, store_fstar or
+    f_summary."""
+    C_ = None
+    if chains is not None:
+        if isinstance(chains, (bool, np.bool_)) or not isinstance(chains, (int, np.integer)) or not 1 <= int(chains) <= 32:
+            raise ValueError("chains must be an integer in [1, 32], got %r" % (chains,))
+        C_ = int(chains)
+        for name, v in (("shard", shard is not None), ("predictive", predictive), ("irf_band", irf_band is not None),
+                        ("store_fstar", store_fstar), ("f_summary", f_summary)):
+            if v:
+                raise ValueError("chains cannot be combined with %s" % name)
+    elif chain_diagnostics:
+        raise ValueError("chain_diagnostics needs chains")
     if irf_band is not None:
         irf_band = float(irf_band)
         if not 0.0 < irf_band < 1.0:   # NaN fails too
             raise ValueError("irf_band must lie in (0, 1), got %r" % irf_band)
-    L = _lib.load()
     y = as_response_matrix(data, vote_codes or DEFAULT_CODES)                        # R/gpirtMCMC.R:93
     y = np.asfortranarray(np.asarray(y, dtype=np.float64))
     n, m = y.shape
-    if theta_init is None:
-        theta_init = np.random.standard_normal(n)                                   # R/gpirtMCMC.R:95-97
-    theta_init = np.ascontiguousarray(theta_init, dtype=np.float64)
-    if theta_init.shape != (n,):
-        raise ValueError("theta_init must have length nrow(data)")
+    if C_ is not None:
+        if theta_init is None:
+            theta_init = np.stack([np.random.standard_normal(n) for _ in range(C_)], axis=1)
+        theta_init = np.asfortranarray(theta_init, dtype=np.float64)
+        if theta_init.shape != (n, C_):
+            raise ValueError("theta_init must be nrow(data) x chains = %r, got %r" % ((n, C_), theta_init.shape))
+        if seed is not None and not isinstance(seed, (int, np.integer)):
+            seed = [int(v) for v in seed]
+            if len(seed) != C_:
+                raise ValueError("seed must be an integer or a sequence of %d seeds, got %d" % (C_, len(seed)))
+    else:
+        if theta_init is None:
+            theta_init = np.random.standard_normal(n)                               # R/gpirtMCMC.R:95-97
+        theta_init = np.ascontiguousarray(theta_init, dtype=np.float64)
+        if theta_init.shape != (n,):
+            raise ValueError("theta_init must have length nrow(data)")
     pm = _F(np.zeros((2, m)) if beta_prior_means is None else beta_prior_means, (2, m))   # R/gpirtMCMC.R:88
     psd = _F(np.full((2, m), 3.0) if beta_prior_sds is None else beta_prior_sds, (2, m))  # :89
     pstep = _F(np.full((2, m), 0.1) if beta_proposal_sds is None else beta_proposal_sds, (2, m))  # :90
     S, B = int(sample_iterations), int(burn_iterations)                             # RcppExports.cpp:22-23 coerce to int
     if seed is None:
         seed = int(np.random.randint(0, 2 ** 31 - 1)) | (int(np.random.randint(0, 2 ** 31 - 1)) << 32)
+    seeds = None
+    if C_ is not None:
+        given = [int(seed) + c for c in range(C_)] if isinstance(seed, (int, np.integer)) else seed
+        seeds = np.array([v & 0xFFFFFFFFFFFFFFFF for v in given], dtype=np.uint64)
+        seed = int(seeds[0])
     kw = {}
     if shard is not None:
         kw = dict(rank=shard[0], world_size=shard[1], m_global=shard[2], item_offset=shard[3], nccl_unique_id=shard[4])
@@ -91,10 +124,22 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
         raise ValueError("thin must be >= 1")
     opts = make_opts(seed=seed, device=device, fstar_mode=fstar_mode, skip_f_draws=not store_f, thin=thin, use_graph=use_graph, **kw)
     slots = S // thin + 1
-    theta = np.empty((slots, n), order="F")
-    beta = np.empty((2, m, slots), order="F")
-    f = np.empty((n, m, slots), order="F") if store_f else None
-    irf = np.empty((N_GRID, m), order="F")
+    ch = () if C_ is None else (C_,)
+    theta = np.empty((slots, n) + ch, order="F")
+    beta = np.empty((2, m, slots) + ch, order="F")
+    f = np.empty((n, m, slots) + ch, order="F") if store_f else None
+    irf = np.empty((N_GRID, m) + ch, order="F")
+    chains_s = diag = None
+    if C_ is not None:
+        chains_s = Chains()
+        chains_s.chains = C_
+        chains_s.seeds = seeds.ctypes.data_as(C.POINTER(C.c_uint64))
+        if chain_diagnostics:
+            diag = dict(theta_rhat=np.empty(n), theta_ess=np.empty(n), beta_rhat=np.empty((2, m), order="F"),
+                        beta_ess=np.empty((2, m), order="F"), irf_rhat=np.empty((N_GRID, m), order="F"))
+            for k, a in diag.items():
+                setattr(chains_s, k, _lib.ptr(a))
+        opts.chains = C.pointer(chains_s)
     f_mean = f_sd = None
     fit = None
     if y_holdout is not None and not predictive:
@@ -132,6 +177,7 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
         except KeyboardInterrupt:
             return 1
     cb = _lib.PROGRESS_CB(_cb)
+    L = _lib.load()
     rc = L.gpirt_b200_mcmc(_lib.ptr(y), n, m, _lib.ptr(theta_init), S, B, _lib.ptr(pm), _lib.ptr(psd), _lib.ptr(pstep),
                            C.byref(opts), _lib.ptr(theta), _lib.ptr(beta), _lib.ptr(f), _lib.ptr(irf), cb, None)
     _lib.check(rc)
@@ -148,6 +194,8 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
         out["IRF_summary"] = dict(summ, band=irf_band, band_bytes=int(irf_s.band_bytes))
     if store_fstar:
         out["fstar"] = fstar
+    if diag is not None:
+        out["diagnostics"] = dict(diag, diag_bytes=int(chains_s.diag_bytes))
     return out
 
 

@@ -84,6 +84,36 @@ typedef struct gpirt_b200_irf {
     int64_t band_bytes;   /* out: device bytes of the tail buffers, 8 * 1001 * m * (K_lo + K_hi) (0 without bands) */
 } gpirt_b200_irf;
 
+/* Several chains in one gpirt_b200_mcmc call, run concurrently on one device (one host thread enqueues them round-robin),
+ * with convergence diagnostics computed on the device.  With opts.chains set, C = chains and every array takes a trailing
+ * chain dimension; chain c's block is exactly what a call without opts.chains, with seed seeds[c] (NULL: opts.seed + c)
+ * and theta_init[:, c], writes:
+ *   theta_init n x C,  theta_out slots x n x C,  beta_out 2 x m x slots x C,  f_out n x m x slots x C (or NULL with
+ *   skip_f_draws),  irf_out 1001 x m x C.
+ * thin, skip_f_draws, use_graph, device and fstar_mode apply to every chain.  Not built (GPIRT_B200_ERR_ARG): world_size
+ * > 1, opts.fit, opts.irf, f_mean_out or f_sd_out set, chains outside [1, 32].
+ * Diagnostics use all S sampling iterations whatever thin is, with the formulas of gpirt_b200_theta_diagnostics:
+ *   half = floor(S / 2); each chain contributes its first and its last `half` iterations (the middle one of an odd S is
+ *   dropped).  split-R-hat = sqrt(var+ / W) over the 2C half-chains, NaN when W = 0.  ESS: per chain, autocovariances with
+ *   denominator S and Geyer's initial monotone sequence over lag pairs (NaN for a constant chain), summed over chains.
+ *   irf_rhat is the split-R-hat of P = plogis(f*) per grid cell.  S < 4: every diagnostic output is NaN.
+ * Before the first sweep the call checks that C - 1 more samplers of chain 0's footprint and the diagnostics buffers fit
+ * in free device memory (else GPIRT_B200_ERR_NOMEM, the bytes needed in the message).  If any chain fails or the progress
+ * callback interrupts, every chain stops and gpirt_b200_last_error names the chain.  The callback is called on the calling
+ * thread only, once per iteration of all chains.  gpirt_b200_last_degenerate_theta() returns the sum over chains. */
+typedef struct gpirt_b200_chains {
+    int32_t chains;          /* C, 1 <= C <= 32 */
+    int32_t reserved0;
+    const uint64_t* seeds;   /* optional C Philox keys; NULL: chain c uses opts.seed + c */
+    double* theta_rhat;      /* optional n        split-R-hat over the 2C half-chains, all S sampling iterations */
+    double* theta_ess;       /* optional n        sum over chains of Geyer's initial-monotone ESS per chain */
+    double* beta_rhat;       /* optional 2 x m */
+    double* beta_ess;        /* optional 2 x m */
+    double* irf_rhat;        /* optional 1001 x m split-R-hat of P = plogis(f*) per grid cell */
+    int64_t diag_bytes;      /* out: device bytes of the traces (8 S (n + 2m) C with theta / beta diagnostics) and
+                                half-chain accumulators (32 x 1001 m C with irf_rhat) */
+} gpirt_b200_chains;
+
 /* Options beyond the reference's seven arguments.  Zero-initialise, then set what you need. */
 typedef struct gpirt_b200_opts {
     uint64_t seed;        /* Philox4x32-10 key; the R shim derives it from R's RNG so set.seed() reproduces runs */
@@ -112,6 +142,8 @@ typedef struct gpirt_b200_opts {
                              NULL = none.  Costs 25 bytes of device memory per cell for the run */
     gpirt_b200_irf* irf;  /* optional: posterior mean, sd, pointwise credible bands and draws of f* on the grid
                              (gpirt_b200_irf); NULL = none */
+    gpirt_b200_chains* chains; /* optional: several chains in this call and their diagnostics (gpirt_b200_chains);
+                             NULL = one chain */
 } gpirt_b200_opts;
 
 /* Progress / interrupt callback: called once per iteration with percent complete (as the reference's Rprintf,
