@@ -13,7 +13,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "_obj")
 LIB = os.path.join(HERE, "libgpirt_b200.so")
-SOURCES = ["gemm.cu", "linalg.cu", "kernels.cu", "softplus_table.cu", "theta_int8.cu", "dgemm_i8.cu", "comm.cu", "sampler.cu", "capi.cu"]
+SOURCES = ["gemm.cu", "linalg.cu", "kernels.cu", "softplus_table.cu", "theta_int8.cu", "dgemm_i8.cu", "ppc.cu", "comm.cu", "sampler.cu", "capi.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC",
          "--cudart", "static"]

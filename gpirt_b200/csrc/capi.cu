@@ -10,6 +10,7 @@
 #include "dgemm_i8.cuh"
 #include "kernels.cuh"
 #include "linalg.cuh"
+#include "ppc.cuh"
 #include "theta_int8.cuh"
 
 using namespace gpirt;
@@ -415,6 +416,68 @@ int gpirt_b200_irf_bands(const double* draws, int64_t cols, int64_t S, double ba
         ms[0] = t_upd / ((double)reps * (double)S);
         ms[1] = t_fin / reps;
     }
+    return GPIRT_B200_OK;
+}
+
+int gpirt_b200_ppc_pairs(const double* y, const double* y_reps, int64_t n, int64_t m, int R, double* log_or, double* exceed,
+                         int reps, double* ms) {
+    if (!y || (R > 0 && !y_reps) || n <= 0 || m <= 0 || n > (1 << 28) || m > (1 << 20) || R < 0 || reps < 0 || (reps > 0 && (!ms || R == 0))) {
+        set_last_error("bad argument: ppc_pairs needs y, y_reps (R > 0), 1 <= n <= 2^28, 1 <= m <= 2^20, R >= 0, reps >= 0 "
+                       "(reps > 0: ms and R > 0)");
+        return GPIRT_B200_ERR_ARG;
+    }
+    GP_TRY(have_device());
+    const int64_t ldy = round_up(n, 16);
+    const size_t cells = (size_t)n * m;
+    DevBuf src, planes;
+    GP_TRY(src.alloc(cells));
+    GP_TRY(planes.alloc(((size_t)ldy * m + 2 * sizeof(unsigned long long) + 7) / 8));
+    int8_t* y8 = reinterpret_cast<int8_t*>(planes.p);
+    unsigned long long* counts = reinterpret_cast<unsigned long long*>(planes.p + ((size_t)ldy * m + 7) / 8);
+    GP_CUDA(cudaMemset(planes.p, 0, ((size_t)ldy * m + 7) / 8 * 8 + 2 * sizeof(unsigned long long)));
+    auto plane = [&](const double* host, const int8_t* mask, int8_t* dst) -> int {
+        GP_CUDA(cudaMemcpy(src.p, host, cells * sizeof(double), cudaMemcpyHostToDevice));
+        GP_TRY(launch_ppc_plane(0, src.p, (int)n, (int)m, mask, dst, ldy, counts));
+        unsigned long long c[2];
+        GP_CUDA(cudaMemcpy(c, counts, sizeof(c), cudaMemcpyDeviceToHost));
+        if (c[1]) { set_last_error("y or y_reps hold %llu values that are not +1, -1 (or NA in y)", c[1]); return GPIRT_B200_ERR_Y_VALUE; }
+        return GPIRT_B200_OK;
+    };
+    GP_TRY(plane(y, nullptr, y8));
+    unsigned long long missing = 0;
+    GP_CUDA(cudaMemcpy(&missing, counts, sizeof(missing), cudaMemcpyDeviceToHost));
+    PpcPairs pp;
+    struct Free { PpcPairs& p; ~Free() { p.destroy(); } } free_pp{pp};
+    GP_TRY(pp.init(0, y8, ldy, (int)n, (int)m, missing != 0));
+    cudaEvent_t e[2];
+    for (auto& v : e) GP_CUDA(cudaEventCreate(&v));
+    struct FreeEv { cudaEvent_t* e; ~FreeEv() { cudaEventDestroy(e[0]); cudaEventDestroy(e[1]); } } free_ev{e};
+    if (reps > 0) {   // the observed pass rewrites the same counts; the timed draw launches are undone before the counted ones
+        float t = 0.f;
+        GP_TRY(plane(y_reps, y8, pp.yrep));
+        GP_CUDA(cudaEventRecord(e[0], 0));
+        for (int r = 0; r < reps; ++r) GP_TRY(pp.observed_pass(0, y8));
+        GP_CUDA(cudaEventRecord(e[1], 0));
+        GP_CUDA(cudaEventSynchronize(e[1]));
+        GP_CUDA(cudaEventElapsedTime(&t, e[0], e[1]));
+        ms[1] = t / reps;
+        GP_CUDA(cudaEventRecord(e[0], 0));
+        for (int r = 0; r < reps; ++r) GP_TRY(pp.iterate(0));
+        GP_CUDA(cudaEventRecord(e[1], 0));
+        GP_CUDA(cudaEventSynchronize(e[1]));
+        GP_CUDA(cudaEventElapsedTime(&t, e[0], e[1]));
+        ms[0] = t / reps;
+        GP_TRY(pp.clear_counters(0));
+    }
+    for (int r = 0; r < R; ++r) {
+        GP_TRY(plane(y_reps + (size_t)r * cells, y8, pp.yrep));
+        GP_TRY(pp.iterate(0));
+    }
+    GP_TRY(pp.finish(0, 1.0, false, log_or, exceed, [](double* dst, const double* src, size_t count) -> int {
+        GP_CUDA(cudaMemcpy(dst, src, count * sizeof(double), cudaMemcpyDeviceToHost));
+        return GPIRT_B200_OK;
+    }));
+    GP_CUDA(cudaDeviceSynchronize());
     return GPIRT_B200_OK;
 }
 

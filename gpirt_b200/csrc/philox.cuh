@@ -8,7 +8,8 @@
 namespace gpirt {
 
 enum Purpose : uint32_t {
-    P_INIT_F_Z = 0, P_INIT_BETA = 1, P_ESS_Z = 2, P_ESS_U = 3, P_FSTAR_Z = 4, P_THETA_U = 5, P_BETA_Z = 6, P_BETA_U = 7
+    P_INIT_F_Z = 0, P_INIT_BETA = 1, P_ESS_Z = 2, P_ESS_U = 3, P_FSTAR_Z = 4, P_THETA_U = 5, P_BETA_Z = 6, P_BETA_U = 7,
+    P_PPC_U = 8   // posterior predictive replicates (opts.ppc): drawn outside the chain, which never reads them
 };
 
 // sweep_dev (optional): device word added to `sweep` at run time — lets a CUDA graph of a whole sweep be replayed with a

@@ -21,6 +21,7 @@
 #include "gemm_f64.cuh"
 #include "kernels.cuh"
 #include "linalg.cuh"
+#include "ppc.cuh"
 #include <climits>
 
 #include "theta_int8.cuh"
@@ -1513,6 +1514,23 @@ __global__ void __launch_bounds__(256) k_f_sd(double* __restrict__ m2, size_t co
 }
 
 namespace {
+// Free device memory for a buffer of `need` bytes.  Memory the pool holds unused is free for this purpose: when short, the
+// pool is handed back first.
+int free_memory_for(double need, cudaStream_t st, size_t* free_b) {
+    size_t total_b = 0;
+    GP_CUDA(cudaMemGetInfo(free_b, &total_b));
+    if (need > (double)*free_b) {
+        int dev = 0;
+        cudaMemPool_t pool;
+        GP_CUDA(cudaStreamSynchronize(st));
+        GP_CUDA(cudaGetDevice(&dev));
+        GP_CUDA(cudaDeviceGetDefaultMemPool(&pool, dev));
+        GP_CUDA(cudaMemPoolTrimTo(pool, 0));
+        GP_CUDA(cudaMemGetInfo(free_b, &total_b));
+    }
+    return GPIRT_B200_OK;
+}
+
 // One chain of gpirtMCMC(): the sampler, its draw storage (snapshot buffers, copy stream, StoreWorker), the status polling
 // and the on-device accumulators, driven by setup(), one iterate() per sweep and finish().  gpirt_b200_mcmc drives one;
 // with opts.chains it drives several on one device, round-robin from the calling thread.  The progress callback belongs
@@ -1540,6 +1558,7 @@ struct ChainRun {
     double* h_small[2] = {nullptr, nullptr}; cudaEvent_t ev_small[2] = {nullptr, nullptr};
     double* pred_acc = nullptr; int8_t* pred_code = nullptr; double* pred_aux = nullptr;   // opts.fit
     double* irf_buf = nullptr; double* snap_fs[2] = {nullptr, nullptr};                     // opts.irf
+    gpirt_b200_ppc* ppc = nullptr; PpcChi2 ppc_chi2; PpcPairs ppc_pairs;                     // opts.ppc
     // state of the run
     double* h_ring = nullptr; volatile int* w_poll = nullptr; int agree_count = 0;
     static constexpr int PRED_CHUNKS = 64;
@@ -1570,6 +1589,8 @@ struct ChainRun {
         pool_free(pred_acc, s->stream); pool_free(pred_code, s->stream); pool_free(pred_aux, s->stream);
         for (int i = 0; i < 2; ++i) pool_free(snap_fs[i], s->stream);
         if (irf_buf) { cudaStreamSynchronize(s->stream); cudaFree(irf_buf); }   // not the pool: GBs of tail buffers must not stay reserved after the call
+        if (ppc_pairs.buf) { cudaStreamSynchronize(s->stream); ppc_pairs.destroy(); }   // likewise
+        ppc_chi2.destroy();
         const double t2 = now();
         gpirt_b200_sampler_destroy(s);
         if (trace) fprintf(stderr, "gpirt_b200_mcmc: teardown worker/copy stream %.3fs, host + pool frees %.3fs, sampler %.3fs\n", t1 - t0, t2 - t1, now() - t2);
@@ -1640,6 +1661,7 @@ int ChainRun::setup() {
     summarise_f = f_mean_out || f_sd_out;
     fit = opts ? opts->fit : nullptr;
     irf = opts ? opts->irf : nullptr;
+    ppc = opts ? opts->ppc : nullptr;
     t_a = now();
     t_untraced_create = untraced;
     const int crc = gpirt_b200_sampler_create(&s, y, n, m, theta_init, pm, psd, pstep, opts);
@@ -1725,17 +1747,8 @@ int ChainRun::setup() {
         irf->band_bytes = 0;
         const double tail_bytes = 8.0 * (double)irf_cells * ((double)irf_plan.klo + (double)irf_plan.khi);
         const double need = tail_bytes + 16.0 * (double)irf_cells;
-        size_t free_b = 0, total_b = 0;
-        GP_CUDA(cudaMemGetInfo(&free_b, &total_b));
-        if (need > (double)free_b) {   // memory the pool holds unused is free for this purpose: hand it back first
-            int dev = 0;
-            cudaMemPool_t pool;
-            GP_CUDA(cudaStreamSynchronize(s->stream));
-            GP_CUDA(cudaGetDevice(&dev));
-            GP_CUDA(cudaDeviceGetDefaultMemPool(&pool, dev));
-            GP_CUDA(cudaMemPoolTrimTo(pool, 0));
-            GP_CUDA(cudaMemGetInfo(&free_b, &total_b));
-        }
+        size_t free_b = 0;
+        GP_TRY(free_memory_for(need, s->stream, &free_b));
         double short_all = need > (double)free_b ? 1.0 : 0.0;
         if (sharded) {   // every rank refuses together, as for y_holdout
             GP_CUDA(cudaMemcpyAsync(agree_dev, &short_all, sizeof(double), cudaMemcpyHostToDevice, s->stream));
@@ -1766,6 +1779,26 @@ int ChainRun::setup() {
             // pinned bounce buffers large enough for an f* plane now: the storage worker must never reallocate them while
             // the other buffer's transfer is in flight (without pinned memory the plane goes by a plain copy)
             bo->ensure(std::max(keep_f ? nm : (size_t)0, irf_plane));
+        }
+    }
+    // posterior predictive checks: the chi-square counters from the pool; the pair state (observed counts of every pair,
+    // counters, replicate plane) in one cudaMalloc, checked against the free device memory before the first sweep, and
+    // the observed counts computed now
+    if (ppc) {
+        ppc->ppp = NAN;
+        ppc->pair_bytes = 0;
+        GP_TRY(ppc_chi2.init(s->stream, s->y8, s->ldy8, (int)n, (int)m));
+        if (ppc->pair_ppp || ppc->pair_log_or) {
+            const double need = (double)PpcPairs::bytes_needed(n, m, s->has_missing);
+            ppc->pair_bytes = (int64_t)need;   // also reported when the call is refused
+            size_t free_b = 0;
+            GP_TRY(free_memory_for(need, s->stream, &free_b));
+            if (need > (double)free_b) {
+                set_last_error("the pair checks of %lld items over %lld respondents need %.0f bytes of device memory; %zu bytes "
+                               "are free on this device", (long long)m, (long long)n, need, free_b);
+                return GPIRT_B200_ERR_NOMEM;
+            }
+            GP_TRY(ppc_pairs.init(s->stream, s->y8, s->ldy8, (int)n, (int)m, s->has_missing));
         }
     }
     t_c = now();
@@ -1829,6 +1862,11 @@ int ChainRun::iterate(int iter) {
     if (sampling && irf)   // the f* this sweep drew (fstar, not the means in Dmat); nothing on a side stream writes it
         GP_TRY(launch_irf_accumulate(s->stream, s->fstar, s->ldN, N_GRID, irf_cells, si, irf_buf, irf_buf + irf_plane,
                                      irf_lo, irf_plan.klo, irf_hi, irf_plan.khi));
+    if (sampling && ppc) {   // the replicate of the state this sweep left, under the counter of that sweep (B + si)
+        GP_TRY(ppc_chi2.iterate(s->stream, s->f, s->ldn, s->y8, s->ldy8, s->theta, s->beta, s->key_at(s->sweep_counter),
+                                s->item_offset, ppc_pairs.buf ? ppc_pairs.yrep : nullptr));
+        if (ppc_pairs.buf) GP_TRY(ppc_pairs.iterate(s->stream));
+    }
     if (sampling && (diag_trace || diag_halves))   // theta | beta as the snapshot would copy them, and f* as above
         GP_TRY(launch_chain_halves(s->stream, s->fstar, s->ldN, N_GRID, irf_cells, si, S, diag_halves, s->theta, (int)n,
                                    s->beta, 2 * (int)m, diag_trace));
@@ -1927,6 +1965,11 @@ int ChainRun::finish() {
         if (irf->lower) GP_TRY(d2h(irf->lower, irf_bands ? irf_lo : m2, irf_plane, 0));   // S = 0: the NaN plane
         if (irf->upper) GP_TRY(d2h(irf->upper, irf_bands ? irf_hi : m2, irf_plane, 1));
     }
+    if (ppc) {
+        GP_TRY(ppc_chi2.finish(s->stream, S, ppc->item_ppp, ppc->resp_ppp, &ppc->ppp));
+        auto copy = [this](double* dst, const double* src, size_t count) { return d2h(dst, src, count, 0); };
+        if (ppc_pairs.buf) GP_TRY(ppc_pairs.finish(s->stream, 1.0 / (double)S, S == 0, ppc->pair_log_or, ppc->pair_ppp, copy));
+    }
     GP_CUDA(cudaStreamSynchronize(s->stream));
     if (trace)
         fprintf(stderr, "gpirt_b200_mcmc: create %.3fs, copy buffers %.3fs, init draws %.3fs, %d sweeps + stores %.3fs (stores %.3fs)\n",
@@ -1946,8 +1989,8 @@ int mcmc_chains(const double* y, int64_t n, int64_t m, const double* theta_init,
     const int C = ch->chains;
     if (C < 1 || C > 32) { set_last_error("bad argument: chains must lie in [1, 32], got %d", C); return GPIRT_B200_ERR_ARG; }
     if (opts->world_size > 1) { set_last_error("several chains with items sharded across GPUs are not built"); return GPIRT_B200_ERR_ARG; }
-    if (opts->fit || opts->irf || opts->f_mean_out || opts->f_sd_out) {
-        set_last_error("fit, irf, f_mean_out and f_sd_out are not built for several chains");
+    if (opts->fit || opts->irf || opts->ppc || opts->f_mean_out || opts->f_sd_out) {
+        set_last_error("fit, irf, ppc, f_mean_out and f_sd_out are not built for several chains");
         return GPIRT_B200_ERR_ARG;
     }
     if (!theta_init) { set_last_error("bad argument: theta_init is NULL"); return GPIRT_B200_ERR_ARG; }
@@ -2092,6 +2135,10 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
     gpirt_b200_irf* const irf = opts ? opts->irf : nullptr;
     if (irf && (irf->lower || irf->upper) && !(std::isfinite(irf->band) && irf->band > 0.0 && irf->band < 1.0)) {
         set_last_error("bad argument: the IRF band level must lie in (0, 1), got %g", irf->band);
+        return GPIRT_B200_ERR_ARG;
+    }
+    if (opts && opts->ppc && opts->world_size > 1) {   // every rank sees its own opts: all refuse before any collective
+        set_last_error("posterior predictive checks with items sharded across GPUs are not built");
         return GPIRT_B200_ERR_ARG;
     }
     const bool trace = getenv("GPIRT_TIMING") != nullptr;

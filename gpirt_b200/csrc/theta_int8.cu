@@ -15,10 +15,9 @@
 // ring; one elected thread issues tcgen05.mma (M = 128, N = 256, K = 32), the int32 accumulator lives in TMEM
 // (256 columns).  The epilogue warps read TMEM with tcgen05.ld, combine the 8 digit planes of each grid point in
 // registers and write the FP64 result straight into logP^T — the int32 products never touch HBM.
-#include <cuda.h>
-
 #include <mutex>
 
+#include "tcgen05_i8.cuh"
 #include "theta_int8.cuh"
 
 namespace gpirt {
@@ -30,55 +29,8 @@ constexpr int TI_A_BYTES = TI_BM * TI_BK, TI_B_BYTES = TI_BN * TI_BK, TI_STAGE_B
 constexpr int TI_SMEM = TI_STAGES * TI_STAGE_BYTES + 1024 /* alignment slack */ + 256 /* barriers */;
 constexpr int TI_TMEM_COLS = 256;
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-// one lane of a converged warp (ptxas then emits the TMA / tensor-core instructions of the region back to back)
-__device__ __forceinline__ uint32_t elect_one() {
-    uint32_t pred = 0;
-    asm volatile("{\n\t.reg .pred P1;\n\telect.sync _|P1, 0xffffffff;\n\tselp.u32 %0, 1, 0, P1;\n\t}" : "=r"(pred));
-    return pred;
-}
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile(
-            "{\n\t.reg .pred p;\n\t"
-            "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-            "selp.u32 %0, 1, 0, p;\n\t}"
-            : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    } while (!ok);
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t bar) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                 ::"r"(dst), "l"(map), "r"(c0), "r"(c1), "r"(bar) : "memory");
-}
-// shared-memory matrix descriptor, K-major operand, 128-byte swizzle, tile rows are 128 bytes (one swizzle span):
-// start address >> 4 | SBO (8 rows x 128 B = 1024 B) >> 4 at bit 32 | version 1 at bit 46 | SWIZZLE_128B (2) at bit 61
-__device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t saddr) {
-    uint64_t d = (uint64_t)((saddr & 0x3FFFF) >> 4);
-    d |= (uint64_t)(1024 >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
-}
-// instruction descriptor: D = S32 (2 << 4), A = B = signed int8 (1 << 7, 1 << 10), both K-major, N >> 3 at 17, M >> 4 at 24
-constexpr uint32_t TI_IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TI_BN >> 3) << 17) | ((uint32_t)(TI_BM >> 4) << 24);
-
-__device__ __forceinline__ void umma_i8(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(da), "l"(db), "r"(TI_IDESC), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
+using namespace i8tc;
+constexpr uint32_t TI_IDESC = idesc_i8(TI_BM, TI_BN);
 
 __global__ void __launch_bounds__(256, 1)
 k_igemm_theta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, int num_kblocks,
@@ -129,7 +81,7 @@ k_igemm_theta(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
             const uint32_t sa = smem_u32(smem + s * TI_STAGE_BYTES), sb = sa + TI_A_BYTES;
 #pragma unroll
             for (int k4 = 0; k4 < TI_BK / TI_UMMA_K; ++k4)
-                umma_i8(tmem_base, umma_desc_sw128(sa + k4 * TI_UMMA_K), umma_desc_sw128(sb + k4 * TI_UMMA_K),
+                umma_i8<TI_IDESC>(tmem_base, umma_desc_sw128(sa + k4 * TI_UMMA_K), umma_desc_sw128(sb + k4 * TI_UMMA_K),
                         (uint32_t)((kb | k4) != 0));
             umma_commit(empty0 + 8 * s);   // frees the shared-memory slot once these MMAs have read it
         }
@@ -211,7 +163,7 @@ __global__ void __launch_bounds__(128, 1) k_peak_umma_i8(int iters, unsigned* si
             for (int it = 0; it < iters; ++it) {
 #pragma unroll
                 for (int k4 = 0; k4 < TI_BK / TI_UMMA_K; ++k4)
-                    umma_i8(tmem_base + (uint32_t)((it & 1) * TI_TMEM_COLS), umma_desc_sw128(sa + k4 * TI_UMMA_K),
+                    umma_i8<TI_IDESC>(tmem_base + (uint32_t)((it & 1) * TI_TMEM_COLS), umma_desc_sw128(sa + k4 * TI_UMMA_K),
                             umma_desc_sw128(sb + k4 * TI_UMMA_K), (uint32_t)(it > 1 || k4 != 0));
             }
             umma_commit(done);
@@ -308,11 +260,13 @@ __global__ void __launch_bounds__(256) k_slice_digits(const double* __restrict__
     }
 }
 
+}  // namespace
+
 typedef CUresult (*encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-int make_map(CUtensorMap* map, void* base, uint64_t rows, uint64_t row_bytes, uint32_t box_rows) {
+int i8tc::make_map_k_major(CUtensorMap* map, void* base, uint64_t rows, uint64_t cols, uint64_t row_stride, uint32_t box_rows) {
     static encode_fn fn = nullptr;
     if (!fn) {
         void* p = nullptr;
@@ -321,17 +275,15 @@ int make_map(CUtensorMap* map, void* base, uint64_t rows, uint64_t row_bytes, ui
         if (!p || qres != cudaDriverEntryPointSuccess) { set_last_error("cuTensorMapEncodeTiled is not available"); return GPIRT_B200_ERR_CUDA; }
         fn = (encode_fn)p;
     }
-    const cuuint64_t dims[2] = {row_bytes, rows};
-    const cuuint64_t strides[1] = {row_bytes};
-    const cuuint32_t box[2] = {(cuuint32_t)TI_BK, box_rows};
+    const cuuint64_t dims[2] = {cols, rows};
+    const cuuint64_t strides[1] = {row_stride};
+    const cuuint32_t box[2] = {128u, box_rows};   // 128 bytes: one swizzle span
     const cuuint32_t estr[2] = {1, 1};
     CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                     CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { set_last_error("cuTensorMapEncodeTiled failed (%d)", (int)r); return GPIRT_B200_ERR_CUDA; }
     return GPIRT_B200_OK;
 }
-
-}  // namespace
 
 struct ThetaInt8::Maps { CUtensorMap a, a_abs, b; };
 
@@ -352,15 +304,15 @@ int ThetaInt8::init(cudaStream_t st, const int8_t* y8, int64_t ldy, int n_, int 
     GP_LAUNCH(k_build_yt, grid, 256, 0, st, y8, ldy, n, m, yt, m_pad, 0);
     GP_CUDA(cudaGetLastError());
     maps = new Maps();
-    GP_TRY(make_map(&maps->a, yt, (uint64_t)n_pad, (uint64_t)m_pad, TI_BM));
+    GP_TRY(make_map_k_major(&maps->a, yt, (uint64_t)n_pad, (uint64_t)m_pad, (uint64_t)m_pad, TI_BM));
     if (with_observed_mask) {   // |y| in {0,1}: the observed-cell operand of the second product (missing data)
         GP_TRY(pool_alloc((void**)&yt_abs, (size_t)n_pad * m_pad, st));
         GP_CUDA(cudaMemsetAsync(yt_abs, 0, (size_t)n_pad * m_pad, st));
         GP_LAUNCH(k_build_yt, grid, 256, 0, st, y8, ldy, n, m, yt_abs, m_pad, 1);
         GP_CUDA(cudaGetLastError());
-        GP_TRY(make_map(&maps->a_abs, yt_abs, (uint64_t)n_pad, (uint64_t)m_pad, TI_BM));
+        GP_TRY(make_map_k_major(&maps->a_abs, yt_abs, (uint64_t)n_pad, (uint64_t)m_pad, (uint64_t)m_pad, TI_BM));
     }
-    GP_TRY(make_map(&maps->b, Q, (uint64_t)c_pad, (uint64_t)m_pad, TI_BN));
+    GP_TRY(make_map_k_major(&maps->b, Q, (uint64_t)c_pad, (uint64_t)m_pad, (uint64_t)m_pad, TI_BN));
     GP_CUDA(cudaFuncSetAttribute(k_igemm_theta, cudaFuncAttributeMaxDynamicSharedMemorySize, TI_SMEM));
     ready = true;
     return GPIRT_B200_OK;

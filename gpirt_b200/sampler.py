@@ -10,7 +10,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import Chains, Fit, GpirtError, Irf, Opts, N_GRID
+from ._lib import Chains, Fit, GpirtError, Irf, Opts, Ppc, N_GRID
 from .response_matrix import DEFAULT_CODES, as_response_matrix
 
 
@@ -48,7 +48,7 @@ def nccl_unique_id():
 def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_prior_means=None, beta_prior_sds=None,
               beta_proposal_sds=None, theta_init=None, *, seed=None, progress=None, store_f=True, fstar_mode=0,
               device=-1, shard=None, thin=1, f_summary=False, use_graph=0, predictive=False, y_holdout=None,
-              irf_band=None, store_fstar=False, chains=None, chain_diagnostics=False):
+              irf_band=None, store_fstar=False, chains=None, chain_diagnostics=False, ppc=False, ppc_pairs=False):
     """Drop-in for the reference's gpirtMCMC().  Keyword-only extras (not in the reference): seed (Philox key; default
     drawn from numpy's global RNG, as the R shim draws it from R's), progress(percent) -> truthy to interrupt,
     store_f=False to skip the n*m*(S+1) f draws, shard=(rank, world, m_global, item_offset, unique_id) for item
@@ -69,19 +69,28 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
     sequence of C seeds is used as given, and theta, beta, f and IRFs gain a trailing chain axis.  chain_diagnostics=True
     also returns "diagnostics": dict(theta_rhat, theta_ess (n), beta_rhat, beta_ess (2 x m), irf_rhat (1001 x m),
     diag_bytes), split-R-hat and summed Geyer ESS over all S sampling iterations (any thin), computed on the device
-    (definitions in include/gpirt_b200.h).  chains cannot be combined with shard, predictive, irf_band, store_fstar or
-    f_summary."""
+    (definitions in include/gpirt_b200.h).  chains cannot be combined with shard, predictive, irf_band, store_fstar,
+    f_summary or ppc.
+    ppc=True also returns "ppc": posterior predictive checks over all S sampling iterations (any thin), computed on the
+    device (definitions in include/gpirt_b200.h): dict(item_ppp (m), resp_ppp (n), ppp), the PPP-values of the Pearson
+    chi-square per item, per respondent and in all; ppc_pairs=True adds pair_ppp and pair_log_or (m x m, symmetric), the
+    PPP-values and observed values of the pairwise log odds ratios (local dependence), and pair_bytes, the device memory
+    of their state.  ppc cannot be combined with shard."""
     C_ = None
     if chains is not None:
         if isinstance(chains, (bool, np.bool_)) or not isinstance(chains, (int, np.integer)) or not 1 <= int(chains) <= 32:
             raise ValueError("chains must be an integer in [1, 32], got %r" % (chains,))
         C_ = int(chains)
         for name, v in (("shard", shard is not None), ("predictive", predictive), ("irf_band", irf_band is not None),
-                        ("store_fstar", store_fstar), ("f_summary", f_summary)):
+                        ("store_fstar", store_fstar), ("f_summary", f_summary), ("ppc", ppc)):
             if v:
                 raise ValueError("chains cannot be combined with %s" % name)
     elif chain_diagnostics:
         raise ValueError("chain_diagnostics needs chains")
+    if ppc_pairs and not ppc:
+        raise ValueError("ppc_pairs needs ppc")
+    if ppc and shard is not None:
+        raise ValueError("ppc cannot be combined with shard")
     if irf_band is not None:
         irf_band = float(irf_band)
         if not 0.0 < irf_band < 1.0:   # NaN fails too
@@ -170,6 +179,15 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
             irf_s.prob_mean, irf_s.prob_sd = _lib.ptr(summ["mean"]), _lib.ptr(summ["sd"])
             irf_s.lower, irf_s.upper = _lib.ptr(summ["lower"]), _lib.ptr(summ["upper"])
         opts.irf = C.pointer(irf_s)
+    ppc_s = None
+    if ppc:
+        ppc_s = Ppc()
+        checks = dict(item_ppp=np.empty(m), resp_ppp=np.empty(n))
+        if ppc_pairs:
+            checks.update(pair_ppp=np.empty((m, m), order="F"), pair_log_or=np.empty((m, m), order="F"))
+        for k, a in checks.items():
+            setattr(ppc_s, k, _lib.ptr(a))
+        opts.ppc = C.pointer(ppc_s)
 
     def _cb(pct, _ctx):
         try:
@@ -194,6 +212,10 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
         out["IRF_summary"] = dict(summ, band=irf_band, band_bytes=int(irf_s.band_bytes))
     if store_fstar:
         out["fstar"] = fstar
+    if ppc:
+        out["ppc"] = dict(checks, ppp=float(ppc_s.ppp))
+        if ppc_pairs:
+            out["ppc"]["pair_bytes"] = int(ppc_s.pair_bytes)
     if diag is not None:
         out["diagnostics"] = dict(diag, diag_bytes=int(chains_s.diag_bytes))
     return out
@@ -400,6 +422,29 @@ def irf_bands(draws, band, reps=0):
     _lib.check(_lib.load().gpirt_b200_irf_bands(_lib.ptr(d), cols, S, float(band), _lib.ptr(lo), _lib.ptr(hi), int(reps),
                                                 _lib.ptr(ms)))
     return (lo, hi, (float(ms[0]), float(ms[1]))) if reps > 0 else (lo, hi)
+
+
+def ppc_pairs(y, y_reps, reps=0):
+    """The odds-ratio check of gpirtMCMC(ppc=True, ppc_pairs=True) on given data, through the same device kernels: y is
+    n x m in {+1, -1, NaN}, y_reps n x m x R replicates (+1 / -1 where y is observed, read there only).  Returns
+    (log_or, exceed): the observed pairwise log odds ratios and the number of replicates whose odds ratio is at least the
+    observed one (m x m each, NaN on the diagonal and for pairs nobody answered both of); with reps > 0 also
+    (ms per per-draw launch, ms per observed pass), CUDA events over reps repetitions"""
+    y = _F(y)
+    if y.ndim != 2:
+        raise ValueError("y must be an n x m matrix")
+    n, m = y.shape
+    r = np.asarray(y_reps, dtype=np.float64)
+    if r.ndim == 2:
+        r = r[:, :, None]
+    if r.ndim != 3 or r.shape[:2] != (n, m):
+        raise ValueError("y_reps must be n x m x R with n x m = %r, got %r" % ((n, m), r.shape))
+    r = np.asfortranarray(r)
+    R = r.shape[2]
+    log_or = np.empty((m, m), order="F"); exceed = np.empty((m, m), order="F"); ms = np.zeros(2)
+    _lib.check(_lib.load().gpirt_b200_ppc_pairs(_lib.ptr(y), _lib.ptr(r) if R else None, n, m, R, _lib.ptr(log_or),
+                                                _lib.ptr(exceed), int(reps), _lib.ptr(ms)))
+    return (log_or, exceed, (float(ms[0]), float(ms[1]))) if reps > 0 else (log_or, exceed)
 
 
 def rng_probe(seed, sweep, purpose, stream, idx0, count):

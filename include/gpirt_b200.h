@@ -114,6 +114,36 @@ typedef struct gpirt_b200_chains {
                                 half-chain accumulators (32 x 1001 m C with irf_rhat) */
 } gpirt_b200_chains;
 
+/* Posterior predictive model checks, accumulated on the device over all S sampling iterations (burn-in excluded, thin has
+ * no effect).  Sampling iteration s (s = 1..S) uses the end-of-sweep state opts.fit uses: g_ij = f_ij + beta0_j +
+ * beta1_j theta_i, p_ij = 1 / (1 + exp(-g_ij)).  Only observed cells are replicated (missing cells stay missing):
+ *   y^rep_ij = +1 if u_ij < p_ij, else -1,  u_ij = the Philox uniform of purpose 8 (gpirt_b200_rng_probe(seed, B + s, 8,
+ *   j, i, 1)), stream = global item index j, idx = respondent i, sweep = B + s (the counter of the sweep that produced
+ *   the state; the chain's own draws do not change).
+ * Pearson chi-square: the term of an observed cell is (y01 - p)^2 / (p (1 - p)) = exp(-y g) for y in {+1, -1}.
+ *   D_j(y; s) sums the terms of the observed cells of item j, D_i(y; s) those of respondent i, D(y; s) all of them, and
+ *   D(y^rep; s) the same with y^rep for y.  Observed and replicated sums run in the same fixed order (a replicate equal to
+ *   y gives bit-equal sums, which counts as ">=").
+ *   item_ppp[j] = (1/S) #{s : D_j(y^rep; s) >= D_j(y; s)}; resp_ppp and ppp likewise.  NaN where the item / respondent has
+ *   no observed cell.
+ * Pairs of items j != k, over the respondents who answered both: a = n11, b = n10, c = n01, d = n00.
+ *   pair_log_or = log(((a + 1/2)(d + 1/2)) / ((b + 1/2)(c + 1/2))) of the observed y (FP64).
+ *   pair_ppp = (1/S) #{s : OR(y^rep; s) >= OR(y)}, compared exactly in integers:
+ *     (2a_r+1)(2d_r+1)(2b_o+1)(2c_o+1) >= (2a_o+1)(2d_o+1)(2b_r+1)(2c_r+1)   (128-bit products).
+ *   Both m x m and symmetric; NaN on the diagonal and for pairs with no jointly observed respondent.
+ * S = 0: every output is NaN.  Not built (GPIRT_B200_ERR_ARG): world_size > 1, opts.chains.  The pair state (observed
+ * counts and exceedance counters of every pair, about 20 bytes per pair of the upper triangle, plus the replicate plane)
+ * is one device allocation for the call, checked against free device memory before the first sweep
+ * (GPIRT_B200_ERR_NOMEM, the bytes needed in the message). */
+typedef struct gpirt_b200_ppc {
+    double* item_ppp;     /* optional m */
+    double* resp_ppp;     /* optional n */
+    double* pair_ppp;     /* optional m x m, symmetric */
+    double* pair_log_or;  /* optional m x m, symmetric: observed log odds ratio */
+    double  ppp;          /* out: global PPP of the total chi-square */
+    int64_t pair_bytes;   /* out: device bytes of the pair state (0 without pair outputs) */
+} gpirt_b200_ppc;
+
 /* Options beyond the reference's seven arguments.  Zero-initialise, then set what you need. */
 typedef struct gpirt_b200_opts {
     uint64_t seed;        /* Philox4x32-10 key; the R shim derives it from R's RNG so set.seed() reproduces runs */
@@ -144,6 +174,8 @@ typedef struct gpirt_b200_opts {
                              (gpirt_b200_irf); NULL = none */
     gpirt_b200_chains* chains; /* optional: several chains in this call and their diagnostics (gpirt_b200_chains);
                              NULL = one chain */
+    gpirt_b200_ppc* ppc;  /* optional: posterior predictive checks of item, person and pair fit (gpirt_b200_ppc);
+                             NULL = none */
 } gpirt_b200_opts;
 
 /* Progress / interrupt callback: called once per iteration with percent complete (as the reference's Rprintf,
@@ -281,6 +313,13 @@ int gpirt_b200_predictive_accumulate_time(int64_t n, int64_t m, int reps, double
  * reps times, timed with CUDA events: ms[0] = mean time of one update launch, ms[1] = mean time of the finish. */
 int gpirt_b200_irf_bands(const double* draws, int64_t cols, int64_t S, double band, double* lower, double* upper, int reps,
                          double* ms);
+/* The odds-ratio check of gpirt_b200_ppc on caller data (tests, measurement), through the observed-count and per-draw
+ * kernels gpirt_b200_mcmc uses: y is n x m {+1, -1, NaN}, y_reps n x m x R replicates read where y is observed (+1 / -1
+ * there; any other value, or one in y: GPIRT_B200_ERR_Y_VALUE).  log_or (optional, m x m) = pair_log_or of y;
+ * exceed (optional, m x m) = the number of replicates r with OR(y_reps[:, :, r]) >= OR(y), NaN where pair_ppp is NaN.
+ * reps > 0: ms[0] = mean CUDA-event time of one per-draw launch, ms[1] = of the observed pass, over reps repetitions. */
+int gpirt_b200_ppc_pairs(const double* y, const double* y_reps, int64_t n, int64_t m, int R, double* log_or, double* exceed,
+                         int reps, double* ms);
 /* ---- the host steps either side of the sampler (SURVEY 8 f4) ---- */
 /* Response coding, the producer of y (reference R/response_matrix.R:79-98) for numeric code matrices, on the device:
  * codes n x m (column-major doubles, NaN = NA); yea / nay / missing code lists; cells with a code in none of the lists are
