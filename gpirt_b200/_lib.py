@@ -19,7 +19,7 @@ EXPORTS = [
     "gpirt_b200_sampler_launches", "gpirt_b200_sampler_uses",
     "gpirt_b200_sampler_destroy", "gpirt_b200_se_cov", "gpirt_b200_chol_lower", "gpirt_b200_dgemm", "gpirt_b200_dgemm_i8",
     "gpirt_b200_trsm_lower", "gpirt_b200_ll_bar", "gpirt_b200_fp64_peak_tflops", "gpirt_b200_int8_peak_tops", "gpirt_b200_int8_peak_tops_random", "gpirt_b200_rng_probe", "gpirt_b200_response_matrix", "gpirt_b200_theta_diagnostics",
-    "gpirt_b200_predictive_accumulate_time", "gpirt_b200_irf_bands", "gpirt_b200_ppc_pairs",
+    "gpirt_b200_predictive_accumulate_time", "gpirt_b200_irf_bands", "gpirt_b200_ppc_pairs", "gpirt_b200_psis_loo",
 ]
 
 # enums of include/gpirt_b200.h
@@ -66,12 +66,22 @@ class Ppc(C.Structure):
                 ("pair_log_or", C.POINTER(C.c_double)), ("ppp", C.c_double), ("pair_bytes", C.c_int64)]
 
 
+class Loo(C.Structure):
+    """gpirt_b200_loo: PSIS-LOO cross-validation with Pareto k per observed cell (include/gpirt_b200.h)"""
+    _fields_ = [("elpd_loo_cell", C.POINTER(C.c_double)), ("p_loo_cell", C.POINTER(C.c_double)),
+                ("pareto_k", C.POINTER(C.c_double)), ("elpd_loo_item", C.POINTER(C.c_double)),
+                ("elpd_loo_resp", C.POINTER(C.c_double)), ("elpd_loo", C.c_double), ("p_loo", C.c_double),
+                ("looic", C.c_double), ("se_elpd_loo", C.c_double), ("k_threshold", C.c_double), ("n_obs", C.c_int64),
+                ("n_k_high", C.c_int64), ("tail_len", C.c_int64), ("tail_bytes", C.c_int64)]
+
+
 class Opts(C.Structure):
     _fields_ = [("seed", C.c_uint64), ("device", C.c_int32), ("fstar_mode", C.c_int32), ("skip_f_draws", C.c_int32),
                 ("use_graph", C.c_int32), ("rank", C.c_int32), ("world_size", C.c_int32), ("m_global", C.c_int64),
                 ("item_offset", C.c_int64), ("nccl_unique_id", C.c_void_p), ("thin", C.c_int32), ("reserved0", C.c_int32),
                 ("f_mean_out", C.POINTER(C.c_double)), ("f_sd_out", C.POINTER(C.c_double)), ("fit", C.POINTER(Fit)),
-                ("irf", C.POINTER(Irf)), ("chains", C.POINTER(Chains)), ("ppc", C.POINTER(Ppc))]
+                ("irf", C.POINTER(Irf)), ("chains", C.POINTER(Chains)), ("ppc", C.POINTER(Ppc)),
+                ("loo", C.POINTER(Loo))]
 
 
 PROGRESS_CB = C.CFUNCTYPE(C.c_int, C.c_double, C.c_void_p)
@@ -129,6 +139,7 @@ def load():
     L.gpirt_b200_predictive_accumulate_time.argtypes = [C.c_int64, C.c_int64, C.c_int, _dp, _dp]
     L.gpirt_b200_irf_bands.argtypes = [_dp, C.c_int64, C.c_int64, C.c_double, _dp, _dp, C.c_int, _dp]
     L.gpirt_b200_ppc_pairs.argtypes = [_dp, _dp, C.c_int64, C.c_int64, C.c_int, _dp, _dp, C.c_int, _dp]
+    L.gpirt_b200_psis_loo.argtypes = [_dp, C.c_int64, C.c_int64, _dp, _dp, _dp, C.c_int, _dp]
     L.gpirt_b200_rng_probe.argtypes = [C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, _dp, _dp]
     _lib = L
     return L

@@ -10,6 +10,7 @@
 #include "dgemm_i8.cuh"
 #include "kernels.cuh"
 #include "linalg.cuh"
+#include "loo.cuh"
 #include "ppc.cuh"
 #include "theta_int8.cuh"
 
@@ -478,6 +479,50 @@ int gpirt_b200_ppc_pairs(const double* y, const double* y_reps, int64_t n, int64
         return GPIRT_B200_OK;
     }));
     GP_CUDA(cudaDeviceSynchronize());
+    return GPIRT_B200_OK;
+}
+
+int gpirt_b200_psis_loo(const double* loglik, int64_t cols, int64_t S, double* elpd_loo, double* p_loo, double* pareto_k,
+                        int reps, double* ms) {
+    if ((S > 0 && !loglik) || cols <= 0 || cols > INT_MAX || S < 0 || S > INT_MAX || reps < 0 || (reps > 0 && !ms)) {
+        set_last_error("bad argument: psis_loo needs loglik, 1 <= cols <= INT_MAX, 0 <= S <= INT_MAX, reps >= 0 (reps > 0: ms)");
+        return GPIRT_B200_ERR_ARG;
+    }
+    const int K = (int)loo_tail_len(S) + 1;
+    if (K > LOO_MAX_HEAP) {
+        set_last_error("bad argument: PSIS-LOO over %lld draws keeps a tail of %d draws per unit; at most %d are built",
+                       (long long)S, K - 1, LOO_MAX_HEAP - 1);
+        return GPIRT_B200_ERR_ARG;
+    }
+    GP_TRY(have_device());
+    DevBuf x, state;
+    GP_TRY(x.alloc((size_t)cols * S));
+    GP_TRY(state.alloc((size_t)cols * (K + LOO_STATE_EXTRA)));
+    if (S > 0) GP_CUDA(cudaMemcpy(x.p, loglik, (size_t)cols * S * sizeof(double), cudaMemcpyHostToDevice));
+    cudaEvent_t e[3];
+    for (auto& v : e) GP_CUDA(cudaEventCreate(&v));
+    struct FreeEv { cudaEvent_t* e; ~FreeEv() { for (int i = 0; i < 3; ++i) cudaEventDestroy(e[i]); } } free_ev{e};
+    float t_upd = 0.f, t_fin = 0.f;
+    for (int pass = 0; pass < std::max(reps, 1); ++pass) {   // every pass starts the state afresh (draw 1 initialises it)
+        GP_CUDA(cudaEventRecord(e[0], 0));
+        for (int64_t s = 0; s < S; ++s)
+            GP_TRY(launch_loo_update_ll(0, x.p + (size_t)s * cols, cols, (int)s + 1, K, state.p));
+        GP_CUDA(cudaEventRecord(e[1], 0));
+        GP_TRY(launch_loo_finish(0, state.p, cols, S, nullptr, 0, (int)cols));
+        GP_CUDA(cudaEventRecord(e[2], 0));
+        GP_CUDA(cudaEventSynchronize(e[2]));
+        float a = 0.f, b = 0.f;
+        GP_CUDA(cudaEventElapsedTime(&a, e[0], e[1]));
+        GP_CUDA(cudaEventElapsedTime(&b, e[1], e[2]));
+        t_upd += a; t_fin += b;
+    }
+    double* const outs[3] = {elpd_loo, p_loo, pareto_k};
+    for (int k = 0; k < 3; ++k)
+        if (outs[k]) GP_CUDA(cudaMemcpy(outs[k], state.p + (size_t)k * cols, (size_t)cols * sizeof(double), cudaMemcpyDeviceToHost));
+    if (reps > 0) {
+        ms[0] = S > 0 ? t_upd / ((double)reps * (double)S) : 0.0;
+        ms[1] = t_fin / reps;
+    }
     return GPIRT_B200_OK;
 }
 

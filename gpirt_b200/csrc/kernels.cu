@@ -8,6 +8,7 @@
 
 #include "kernels.cuh"
 #include "softplus_table.cuh"
+#include "tails.cuh"
 
 namespace gpirt {
 
@@ -964,12 +965,6 @@ int launch_predictive_code(cudaStream_t st, const int8_t* y8, int64_t ldy8, cons
     return GPIRT_B200_OK;
 }
 
-// sigma(a) and log sigma(a) from one exp and one log1p, both stable for either sign of a
-__device__ __forceinline__ void log_sigmoid(double a, double& sig, double& ls) {
-    const double e = exp(-fabs(a));
-    sig = (a >= 0.0 ? 1.0 : e) / (1.0 + e);
-    ls = -(fmax(-a, 0.0) + log1p(e));
-}
 __device__ __forceinline__ void predictive_update(double g, int8_t c, double count, double& s, double& mu, double& q) {
     double sig, ls;
     log_sigmoid(c < 0 ? -g : g, sig, ls);
@@ -1117,6 +1112,16 @@ int launch_predictive_reduce(cudaStream_t st, const double* acc, int64_t ld, con
     GP_CUDA(cudaGetLastError());
     return GPIRT_B200_OK;
 }
+int launch_reduce_partials(cudaStream_t st, const double* partial, int N, int n_chunks, double* out) {
+    GP_LAUNCH(k_reduce_partials, (unsigned)ceil_div(N, 128), 128, 0, st, partial, N, n_chunks, out);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
+int launch_stat_totals(cudaStream_t st, const double* stats, int n_stats, int m, double* totals) {
+    GP_LAUNCH(k_predictive_totals, (unsigned)n_stats, 256, 0, st, stats, m, totals);
+    GP_CUDA(cudaGetLastError());
+    return GPIRT_B200_OK;
+}
 
 // ------------------------------------------------------------------------------------------------------------------
 // IRF posterior summaries (opts.irf).  One thread per grid cell, cells contiguous in k.  Per draw: the Welford mean / M2
@@ -1139,44 +1144,6 @@ IrfBandPlan irf_band_plan(int S, double band) {
     return p;
 }
 
-// MAXH: max-heap (root = largest kept value); `above(a, b)`: a belongs nearer the root than b
-template <bool MAXH>
-__device__ __forceinline__ bool heap_above(double a, double b) { return MAXH ? a > b : a < b; }
-// adds v to the heap of cell c, which holds `size` values (capacity K): while not full every value goes in (sift up);
-// once full v replaces the root only if it belongs strictly below it in the kept tail (sift down)
-template <bool MAXH>
-__device__ __forceinline__ void heap_add(double* h, int64_t cells, int64_t c, int K, int size, double v) {
-    auto at = [&](int i) -> double& { return h[(int64_t)i * cells + c]; };
-    if (size < K) {
-        int i = size;
-        while (i > 0) {
-            const int p = (i - 1) >> 1;
-            const double pv = at(p);
-            if (!heap_above<MAXH>(v, pv)) break;
-            at(i) = pv;
-            i = p;
-        }
-        at(i) = v;
-        return;
-    }
-    if (!heap_above<MAXH>(at(0), v)) return;   // v is not inside the kept tail (ties keep the value already there)
-    int i = 0;
-    for (;;) {
-        const int l = 2 * i + 1;
-        if (l >= K) break;
-        int ci = l;
-        double cv = at(l);
-        if (l + 1 < K) {
-            const double rv = at(l + 1);
-            if (heap_above<MAXH>(rv, cv)) { ci = l + 1; cv = rv; }
-        }
-        if (!heap_above<MAXH>(cv, v)) break;
-        at(i) = cv;
-        i = ci;
-    }
-    at(i) = v;
-}
-
 __global__ void __launch_bounds__(256) k_irf_accumulate(const double* __restrict__ x, int64_t ld, int rows, int64_t cells,
                                                         int s, double* __restrict__ mean, double* __restrict__ m2,
                                                         double* __restrict__ lo, int klo, double* __restrict__ hi, int khi) {
@@ -1194,8 +1161,9 @@ __global__ void __launch_bounds__(256) k_irf_accumulate(const double* __restrict
         m2[c] = fma(d, p - mu2, m2[c]);
     }
     if (klo > 0) {
-        heap_add<true>(lo, cells, c, klo, min(s - 1, klo), v);
-        heap_add<false>(hi, cells, c, khi, min(s - 1, khi), v);
+        double left;
+        heap_add<true>(lo, cells, c, klo, min(s - 1, klo), v, &left);
+        heap_add<false>(hi, cells, c, khi, min(s - 1, khi), v, &left);
     }
 }
 int launch_irf_accumulate(cudaStream_t st, const double* x, int64_t ld, int rows, int64_t cells, int s, double* mean,

@@ -77,6 +77,10 @@ int launch_predictive_cells(cudaStream_t st, const double* acc, int64_t ld, cons
 // scratch.  Every sum runs in a fixed order (bit-identical run to run, no floating-point atomics).
 int launch_predictive_reduce(cudaStream_t st, const double* acc, int64_t ld, const int8_t* code, int64_t ldc, int n, int m,
                              double S, double* stats, double* partial, int n_chunks, double* resp_totals);
+// the two fixed-order steps of that reduction on their own: out[k] = sum over c < n_chunks of partial[c * N + k], in order
+// of c; totals[k] = sum over j < m of stats[k * m + j] for k < n_stats (one CTA per statistic)
+int launch_reduce_partials(cudaStream_t st, const double* partial, int N, int n_chunks, double* out);
+int launch_stat_totals(cudaStream_t st, const double* stats, int n_stats, int m, double* totals);
 
 // ---- IRF posterior summaries (opts.irf, definitions in include/gpirt_b200.h) ----
 // Which order statistics a band at level `band` over S draws needs (type 7 quantiles at q_lo = (1 - b)/2, q_hi = (1 + b)/2)

@@ -21,6 +21,7 @@
 #include "gemm_f64.cuh"
 #include "kernels.cuh"
 #include "linalg.cuh"
+#include "loo.cuh"
 #include "ppc.cuh"
 #include <climits>
 
@@ -1559,6 +1560,7 @@ struct ChainRun {
     double* pred_acc = nullptr; int8_t* pred_code = nullptr; double* pred_aux = nullptr;   // opts.fit
     double* irf_buf = nullptr; double* snap_fs[2] = {nullptr, nullptr};                     // opts.irf
     gpirt_b200_ppc* ppc = nullptr; PpcChi2 ppc_chi2; PpcPairs ppc_pairs;                     // opts.ppc
+    gpirt_b200_loo* loo = nullptr; double* loo_state = nullptr; double* loo_aux = nullptr; int loo_K = 0;   // opts.loo
     // state of the run
     double* h_ring = nullptr; volatile int* w_poll = nullptr; int agree_count = 0;
     static constexpr int PRED_CHUNKS = 64;
@@ -1590,6 +1592,8 @@ struct ChainRun {
         for (int i = 0; i < 2; ++i) pool_free(snap_fs[i], s->stream);
         if (irf_buf) { cudaStreamSynchronize(s->stream); cudaFree(irf_buf); }   // not the pool: GBs of tail buffers must not stay reserved after the call
         if (ppc_pairs.buf) { cudaStreamSynchronize(s->stream); ppc_pairs.destroy(); }   // likewise
+        if (loo_state) { cudaStreamSynchronize(s->stream); cudaFree(loo_state); }          // likewise
+        pool_free(loo_aux, s->stream);
         ppc_chi2.destroy();
         const double t2 = now();
         gpirt_b200_sampler_destroy(s);
@@ -1662,6 +1666,7 @@ int ChainRun::setup() {
     fit = opts ? opts->fit : nullptr;
     irf = opts ? opts->irf : nullptr;
     ppc = opts ? opts->ppc : nullptr;
+    loo = opts ? opts->loo : nullptr;
     t_a = now();
     t_untraced_create = untraced;
     const int crc = gpirt_b200_sampler_create(&s, y, n, m, theta_init, pm, psd, pstep, opts);
@@ -1801,6 +1806,36 @@ int ChainRun::setup() {
             GP_TRY(ppc_pairs.init(s->stream, s->y8, s->ldy8, (int)n, (int)m, s->has_missing));
         }
     }
+    // PSIS-LOO: the per-cell state (tail heap, running max, outside sum, sum of sigma) in one cudaMalloc, checked against
+    // the free device memory before the first sweep; the reduction scratch from the pool
+    if (loo) {
+        const double need = loo_state_bytes(S, (int64_t)nm);
+        loo->tail_len = loo_tail_len(S);
+        loo->tail_bytes = (int64_t)need;   // also reported when the call is refused
+        size_t free_b = 0;
+        GP_TRY(free_memory_for(need, s->stream, &free_b));
+        if (need > (double)free_b) {
+            set_last_error("PSIS-LOO over %d sampling iterations keeps a tail of %lld draws per cell and needs %.0f bytes of "
+                           "device memory for %lld cells; %zu bytes are free on this device", S, (long long)loo->tail_len,
+                           need, (long long)nm, free_b);
+            return GPIRT_B200_ERR_NOMEM;
+        }
+        loo_K = (int)loo->tail_len + 1;
+        if (loo_K > LOO_MAX_HEAP) {
+            set_last_error("bad argument: PSIS-LOO over %d sampling iterations keeps a tail of %d draws per cell; at most %d "
+                           "are built", S, loo_K - 1, LOO_MAX_HEAP - 1);
+            return GPIRT_B200_ERR_ARG;
+        }
+        const cudaError_t e = cudaMalloc((void**)&loo_state, (size_t)need);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            loo_state = nullptr;
+            set_last_error("device allocation of %.0f bytes for the PSIS-LOO state failed: %s", need, cudaGetErrorString(e));
+            return GPIRT_B200_ERR_NOMEM;
+        }
+        const size_t aux = (size_t)LOO_STATS * m + (size_t)LOO_CHUNKS * n + (size_t)n + LOO_STATS;
+        GP_TRY(pool_alloc((void**)&loo_aux, aux * sizeof(double), s->stream));
+    }
     t_c = now();
     GP_TRY(s->init_draws());
     t_d = now();
@@ -1859,6 +1894,9 @@ int ChainRun::iterate(int iter) {
     if (sampling && fit)
         GP_TRY(launch_predictive_accumulate(s->stream, s->f, s->ldn, pred_code, s->ldy8, s->theta, s->beta, (int)n, (int)m,
                                             (double)si, pred_acc));
+    if (sampling && loo)
+        GP_TRY(launch_loo_accumulate(s->stream, s->f, s->ldn, s->y8, s->ldy8, s->theta, s->beta, (int)n, (int)m, si, loo_K,
+                                     loo_state));
     if (sampling && irf)   // the f* this sweep drew (fstar, not the means in Dmat); nothing on a side stream writes it
         GP_TRY(launch_irf_accumulate(s->stream, s->fstar, s->ldN, N_GRID, irf_cells, si, irf_buf, irf_buf + irf_plane,
                                      irf_lo, irf_plan.klo, irf_hi, irf_plan.khi));
@@ -1970,6 +2008,34 @@ int ChainRun::finish() {
         auto copy = [this](double* dst, const double* src, size_t count) { return d2h(dst, src, count, 0); };
         if (ppc_pairs.buf) GP_TRY(ppc_pairs.finish(s->stream, 1.0 / (double)S, S == 0, ppc->pair_log_or, ppc->pair_ppp, copy));
     }
+    if (loo) {   // per-cell outputs into state planes 0..2 (in place), then the fixed-order sums over them
+        const double kthr = loo_k_threshold(S);
+        double* const stats = loo_aux;
+        double* const partial = stats + (size_t)LOO_STATS * m;
+        double* const resp = partial + (size_t)LOO_CHUNKS * n;
+        GP_TRY(launch_loo_finish(s->stream, loo_state, (int64_t)nm, S, s->y8, s->ldy8, (int)n));
+        GP_TRY(launch_loo_reduce(s->stream, loo_state, s->y8, s->ldy8, (int)n, (int)m, kthr, stats, partial, resp));
+        double tot[LOO_STATS];
+        GP_CUDA(cudaMemcpyAsync(tot, resp + n, sizeof(tot), cudaMemcpyDeviceToHost, s->stream));
+        if (loo->elpd_loo_resp) GP_CUDA(cudaMemcpyAsync(loo->elpd_loo_resp, resp, (size_t)n * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+        if (loo->elpd_loo_item) GP_CUDA(cudaMemcpyAsync(loo->elpd_loo_item, stats, (size_t)m * sizeof(double), cudaMemcpyDeviceToHost, s->stream));
+        GP_CUDA(cudaStreamSynchronize(s->stream));
+        double* const outs[3] = {loo->elpd_loo_cell, loo->p_loo_cell, loo->pareto_k};
+        for (int w = 0; w < 3; ++w)
+            if (outs[w]) GP_TRY(d2h(outs[w], loo_state + (size_t)w * nm, nm, 0));
+        if (S == 0) {   // the sums over observed cells are NaN, and so are the units without one
+            if (loo->elpd_loo_resp) std::fill(loo->elpd_loo_resp, loo->elpd_loo_resp + n, NAN);
+            if (loo->elpd_loo_item) std::fill(loo->elpd_loo_item, loo->elpd_loo_item + m, NAN);
+        }
+        const double N = tot[3], sum_e = tot[0], var = (tot[1] - sum_e * sum_e / N) / (N - 1.0);
+        loo->elpd_loo = S ? tot[0] : NAN;
+        loo->p_loo = S ? tot[2] : NAN;
+        loo->looic = -2.0 * loo->elpd_loo;
+        loo->se_elpd_loo = S ? std::sqrt(N * (var < 0.0 ? 0.0 : var)) : NAN;   // loo's convention; NaN stays NaN
+        loo->k_threshold = kthr;
+        loo->n_obs = (int64_t)N;
+        loo->n_k_high = (int64_t)tot[4];
+    }
     GP_CUDA(cudaStreamSynchronize(s->stream));
     if (trace)
         fprintf(stderr, "gpirt_b200_mcmc: create %.3fs, copy buffers %.3fs, init draws %.3fs, %d sweeps + stores %.3fs (stores %.3fs)\n",
@@ -1993,6 +2059,7 @@ int mcmc_chains(const double* y, int64_t n, int64_t m, const double* theta_init,
         set_last_error("fit, irf, ppc, f_mean_out and f_sd_out are not built for several chains");
         return GPIRT_B200_ERR_ARG;
     }
+    if (opts->loo) { set_last_error("PSIS-LOO (opts.loo) is not built for several chains"); return GPIRT_B200_ERR_ARG; }
     if (!theta_init) { set_last_error("bad argument: theta_init is NULL"); return GPIRT_B200_ERR_ARG; }
     const bool want_diag = ch->theta_rhat || ch->theta_ess || ch->beta_rhat || ch->beta_ess;
     const bool diag_on = S >= 4;                          // fewer iterations: every diagnostic is NaN
@@ -2139,6 +2206,10 @@ int gpirt_b200_mcmc(const double* y, int64_t n, int64_t m, const double* theta_i
     }
     if (opts && opts->ppc && opts->world_size > 1) {   // every rank sees its own opts: all refuse before any collective
         set_last_error("posterior predictive checks with items sharded across GPUs are not built");
+        return GPIRT_B200_ERR_ARG;
+    }
+    if (opts && opts->loo && opts->world_size > 1) {   // likewise
+        set_last_error("PSIS-LOO with items sharded across GPUs is not built");
         return GPIRT_B200_ERR_ARG;
     }
     const bool trace = getenv("GPIRT_TIMING") != nullptr;

@@ -10,7 +10,7 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from ._lib import Chains, Fit, GpirtError, Irf, Opts, Ppc, N_GRID
+from ._lib import Chains, Fit, GpirtError, Irf, Loo, Opts, Ppc, N_GRID
 from .response_matrix import DEFAULT_CODES, as_response_matrix
 
 
@@ -48,7 +48,8 @@ def nccl_unique_id():
 def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_prior_means=None, beta_prior_sds=None,
               beta_proposal_sds=None, theta_init=None, *, seed=None, progress=None, store_f=True, fstar_mode=0,
               device=-1, shard=None, thin=1, f_summary=False, use_graph=0, predictive=False, y_holdout=None,
-              irf_band=None, store_fstar=False, chains=None, chain_diagnostics=False, ppc=False, ppc_pairs=False):
+              irf_band=None, store_fstar=False, chains=None, chain_diagnostics=False, ppc=False, ppc_pairs=False,
+              loo=False):
     """Drop-in for the reference's gpirtMCMC().  Keyword-only extras (not in the reference): seed (Philox key; default
     drawn from numpy's global RNG, as the R shim draws it from R's), progress(percent) -> truthy to interrupt,
     store_f=False to skip the n*m*(S+1) f draws, shard=(rank, world, m_global, item_offset, unique_id) for item
@@ -75,14 +76,20 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
     device (definitions in include/gpirt_b200.h): dict(item_ppp (m), resp_ppp (n), ppp), the PPP-values of the Pearson
     chi-square per item, per respondent and in all; ppc_pairs=True adds pair_ppp and pair_log_or (m x m, symmetric), the
     PPP-values and observed values of the pairwise log odds ratios (local dependence), and pair_bytes, the device memory
-    of their state.  ppc cannot be combined with shard."""
+    of their state.  ppc cannot be combined with shard.
+    loo=True also returns "loo": leave-one-out cross-validation by Pareto-smoothed importance sampling over all S sampling
+    iterations (any thin), computed on the device with every observed cell one left-out unit (definitions in
+    include/gpirt_b200.h): dict(elpd_loo_cell, p_loo_cell, pareto_k (n x m, NaN on unobserved cells), elpd_loo_item (m),
+    elpd_loo_resp (n), elpd_loo, p_loo, looic, se_elpd_loo, k_threshold, n_obs, n_k_high (cells whose Pareto k exceeds
+    k_threshold: their elpd_loo_cell is unreliable), tail_len, tail_bytes (the device memory of its state, 8 (tail_len + 4)
+    bytes per cell)).  loo cannot be combined with chains or shard."""
     C_ = None
     if chains is not None:
         if isinstance(chains, (bool, np.bool_)) or not isinstance(chains, (int, np.integer)) or not 1 <= int(chains) <= 32:
             raise ValueError("chains must be an integer in [1, 32], got %r" % (chains,))
         C_ = int(chains)
         for name, v in (("shard", shard is not None), ("predictive", predictive), ("irf_band", irf_band is not None),
-                        ("store_fstar", store_fstar), ("f_summary", f_summary), ("ppc", ppc)):
+                        ("store_fstar", store_fstar), ("f_summary", f_summary), ("ppc", ppc), ("loo", loo)):
             if v:
                 raise ValueError("chains cannot be combined with %s" % name)
     elif chain_diagnostics:
@@ -91,6 +98,8 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
         raise ValueError("ppc_pairs needs ppc")
     if ppc and shard is not None:
         raise ValueError("ppc cannot be combined with shard")
+    if loo and shard is not None:
+        raise ValueError("loo cannot be combined with shard")
     if irf_band is not None:
         irf_band = float(irf_band)
         if not 0.0 < irf_band < 1.0:   # NaN fails too
@@ -188,6 +197,14 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
         for k, a in checks.items():
             setattr(ppc_s, k, _lib.ptr(a))
         opts.ppc = C.pointer(ppc_s)
+    loo_s = None
+    if loo:
+        loo_s = Loo()
+        loo_out = dict(elpd_loo_cell=np.empty((n, m), order="F"), p_loo_cell=np.empty((n, m), order="F"),
+                       pareto_k=np.empty((n, m), order="F"), elpd_loo_item=np.empty(m), elpd_loo_resp=np.empty(n))
+        for k, a in loo_out.items():
+            setattr(loo_s, k, _lib.ptr(a))
+        opts.loo = C.pointer(loo_s)
 
     def _cb(pct, _ctx):
         try:
@@ -216,6 +233,12 @@ def gpirtMCMC(data, sample_iterations, burn_iterations, vote_codes=None, beta_pr
         out["ppc"] = dict(checks, ppp=float(ppc_s.ppp))
         if ppc_pairs:
             out["ppc"]["pair_bytes"] = int(ppc_s.pair_bytes)
+    if loo:
+        for k in ("elpd_loo", "p_loo", "looic", "se_elpd_loo", "k_threshold"):
+            loo_out[k] = float(getattr(loo_s, k))
+        for k in ("n_obs", "n_k_high", "tail_len", "tail_bytes"):
+            loo_out[k] = int(getattr(loo_s, k))
+        out["loo"] = loo_out
     if diag is not None:
         out["diagnostics"] = dict(diag, diag_bytes=int(chains_s.diag_bytes))
     return out
@@ -445,6 +468,21 @@ def ppc_pairs(y, y_reps, reps=0):
     _lib.check(_lib.load().gpirt_b200_ppc_pairs(_lib.ptr(y), _lib.ptr(r) if R else None, n, m, R, _lib.ptr(log_or),
                                                 _lib.ptr(exceed), int(reps), _lib.ptr(ms)))
     return (log_or, exceed, (float(ms[0]), float(ms[1]))) if reps > 0 else (log_or, exceed)
+
+
+def psis_loo(loglik, reps=0):
+    """PSIS-LOO of gpirtMCMC(loo=True) on given log-likelihood draws, through the same device update and finish: loglik is
+    cols x S (row = left-out unit, column = draw; sigma = exp(loglik)), for example per-respondent sums of the per-cell
+    log-likelihoods for leave-one-respondent-out.  Returns (elpd_loo, p_loo, pareto_k), each of length cols, and with
+    reps > 0 also (ms per update launch, ms per finish) over reps passes, CUDA events"""
+    ll = _F(loglik)
+    if ll.ndim != 2:
+        raise ValueError("loglik must be a cols x S matrix")
+    cols, S = ll.shape
+    elpd = np.empty(cols); p = np.empty(cols); k = np.empty(cols); ms = np.zeros(2)
+    _lib.check(_lib.load().gpirt_b200_psis_loo(_lib.ptr(ll) if S else None, cols, S, _lib.ptr(elpd), _lib.ptr(p),
+                                               _lib.ptr(k), int(reps), _lib.ptr(ms)))
+    return (elpd, p, k, (float(ms[0]), float(ms[1]))) if reps > 0 else (elpd, p, k)
 
 
 def rng_probe(seed, sweep, purpose, stream, idx0, count):

@@ -144,6 +144,55 @@ typedef struct gpirt_b200_ppc {
     int64_t pair_bytes;   /* out: device bytes of the pair state (0 without pair outputs) */
 } gpirt_b200_ppc;
 
+/* Leave-one-out cross-validation by Pareto-smoothed importance sampling (PSIS-LOO; Vehtari, Gelman & Gabry 2017), computed
+ * on the device over all S sampling iterations (burn-in excluded, thin has no effect) from the end-of-sweep state opts.fit
+ * uses: g_ij = f_ij + beta0_j + beta1_j theta_i.  Every observed cell (y_ij = +1 / -1) is one left-out unit; held-out cells
+ * (opts.fit->y_holdout) are not.  For one cell over s = 1..S:
+ *   ll_s = log sigma(y g_s), sigma_s = sigma(y g_s) (computed as opts.fit computes them); log ratios r_s = -ll_s.
+ *   lpd = log((sum_s sigma_s) / S), summed in increasing s: bit-equal to lpd_cell of opts.fit in the same call.
+ *   M = ceil(min(0.2 S, 3 sqrt(S))) in FP64 (loo's n_pareto_tail with r_eff = 1), reported in tail_len.
+ *   Sort r ascending; mx = r_(S); lw_s = r_s - mx.  The tail = the M largest lw; cutoff = the (M+1)-th largest lw (a
+ *   multiset: which of tied draws is in the tail does not matter).
+ *   The tail is smoothed only when M >= 5 and max(tail) - min(tail) >= 2^-52 / 100; otherwise it stays raw and k = +inf.
+ *     x_1 <= ... <= x_M = exp(tail lw) - exp(cutoff); N = M; G = 30 + floor(sqrt(N)); x* = x_(floor(N/4 + 0.5)) (1-based);
+ *     theta_j = 1/x_N + (1 - sqrt(G / (j - 0.5))) / (3 x*), j = 1..G;
+ *     l(theta) = N (log(-theta / kappa(theta)) - kappa(theta) - 1), kappa(theta) = mean_i log1p(-theta x_i);
+ *     w_j = exp(l_j - logsumexp l); theta^ = sum_j theta_j w_j; k = mean_i log1p(-theta^ x_i); sigma^ = -k / theta^;
+ *     pareto_k = k N / (N + 10) + 5 / (N + 10), +inf if NaN (loo's gpdfit: Zhang & Stephens 2009 with its prior).
+ *   If pareto_k is finite, the tail draw of rank i (ascending) gets lw~_i = log(sigma^ expm1(-pareto_k log1p(-p_i)) /
+ *   pareto_k + exp(cutoff)), p_i = (i - 0.5) / M (sigma^ from the unadjusted k, as loo).  Every lw~ is then truncated at 0.
+ *   elpd_loo_cell = log sum_s exp(lw~_s + ll_s) - log sum_s exp(lw~_s); p_loo_cell = lpd - elpd_loo_cell.
+ * Aggregates over the observed cells (conventions of gpirt_b200_fit): elpd_loo_item / elpd_loo_resp sums (0 where a unit
+ * has no observed cell), elpd_loo, p_loo, looic = -2 elpd_loo, se_elpd_loo = sqrt(n_obs var(elpd_loo_cell)) (sample
+ * variance), k_threshold = min(1 - 1/log10 S, 0.7), n_k_high = #{cells : pareto_k > k_threshold} (+inf counts).
+ * Per-cell outputs are NaN on unobserved cells.  S = 0: every floating-point output is NaN, tail_len = 0, n_k_high = 0.
+ * S = 1: M = 1, pareto_k = +inf, elpd_loo_cell = ll and p_loo_cell = 0 to rounding.  Smoothing can run from S = 21 on.
+ * Runs are bit-identical (fixed-order reductions, no floating-point atomics, no random numbers); the chain's draws do
+ * not change.
+ * State: per cell (observed or not) a max-heap of the M + 1 smallest ll, the running max of r, the sum of exp(r - max)
+ * over the draws outside the heap and the sum of sigma: tail_bytes = 8 (M + 4) n m bytes, no padding, in one device
+ * allocation for the call, checked against free device memory before the first sweep (GPIRT_B200_ERR_NOMEM, the bytes
+ * needed in the message; tail_bytes is reported even then) and returned when the call ends.  M <= 8191 (S <= 7 454 720),
+ * else GPIRT_B200_ERR_ARG; the memory check comes first, so a larger S whose state also exceeds free memory gives
+ * GPIRT_B200_ERR_NOMEM.  Not built (GPIRT_B200_ERR_ARG): world_size > 1, opts.chains. */
+typedef struct gpirt_b200_loo {
+    double* elpd_loo_cell;  /* optional n x m */
+    double* p_loo_cell;     /* optional n x m */
+    double* pareto_k;       /* optional n x m */
+    double* elpd_loo_item;  /* optional m */
+    double* elpd_loo_resp;  /* optional n */
+    double elpd_loo;        /* out: sum of elpd_loo_cell over the observed cells */
+    double p_loo;           /* out: sum of p_loo_cell over the observed cells */
+    double looic;           /* out: -2 elpd_loo */
+    double se_elpd_loo;     /* out: sqrt(n_obs var(elpd_loo_cell)), sample variance in the one-pass form
+                               (sum e^2 - (sum e)^2 / n_obs) / (n_obs - 1) over fixed-order sums, as se_elpd_waic */
+    double k_threshold;     /* out: min(1 - 1 / log10 S, 0.7) */
+    int64_t n_obs;          /* out: number of observed cells */
+    int64_t n_k_high;       /* out: number of observed cells with pareto_k > k_threshold */
+    int64_t tail_len;       /* out: M */
+    int64_t tail_bytes;     /* out: device bytes of the state, 8 (M + 4) n m */
+} gpirt_b200_loo;
+
 /* Options beyond the reference's seven arguments.  Zero-initialise, then set what you need. */
 typedef struct gpirt_b200_opts {
     uint64_t seed;        /* Philox4x32-10 key; the R shim derives it from R's RNG so set.seed() reproduces runs */
@@ -175,6 +224,8 @@ typedef struct gpirt_b200_opts {
     gpirt_b200_chains* chains; /* optional: several chains in this call and their diagnostics (gpirt_b200_chains);
                              NULL = one chain */
     gpirt_b200_ppc* ppc;  /* optional: posterior predictive checks of item, person and pair fit (gpirt_b200_ppc);
+                             NULL = none */
+    gpirt_b200_loo* loo;  /* optional: PSIS-LOO cross-validation with Pareto k per observed cell (gpirt_b200_loo);
                              NULL = none */
 } gpirt_b200_opts;
 
@@ -320,6 +371,14 @@ int gpirt_b200_irf_bands(const double* draws, int64_t cols, int64_t S, double ba
  * reps > 0: ms[0] = mean CUDA-event time of one per-draw launch, ms[1] = of the observed pass, over reps repetitions. */
 int gpirt_b200_ppc_pairs(const double* y, const double* y_reps, int64_t n, int64_t m, int R, double* log_or, double* exceed,
                          int reps, double* ms);
+/* PSIS-LOO of gpirt_b200_loo on caller-supplied log-likelihood draws: loglik is cols x S, column-major, on the host
+ * (column s = draw s of every unit), every column entry a left-out unit with sigma = exp(ll) (any grouping of the data
+ * into units works, for example leave-one-respondent-out from summed log-likelihoods).  The draws are uploaded once
+ * (8 cols S bytes of device memory), streamed one at a time through the update gpirt_b200_mcmc uses and finished as
+ * there.  elpd_loo, p_loo, pareto_k: cols each, optional.  0 <= S <= 7 454 720.  reps > 0: the whole pass is repeated
+ * reps times, timed with CUDA events: ms[0] = mean time of one update launch, ms[1] = mean time of the finish. */
+int gpirt_b200_psis_loo(const double* loglik, int64_t cols, int64_t S, double* elpd_loo, double* p_loo, double* pareto_k,
+                        int reps, double* ms);
 /* ---- the host steps either side of the sampler (SURVEY 8 f4) ---- */
 /* Response coding, the producer of y (reference R/response_matrix.R:79-98) for numeric code matrices, on the device:
  * codes n x m (column-major doubles, NaN = NA); yea / nay / missing code lists; cells with a code in none of the lists are
