@@ -44,6 +44,11 @@ def gpdfit(x):
     return np.where(np.isnan(khat), np.inf, khat), sigma
 
 
+def draw_order_sum(sig):
+    """sum along each row in draw order, as the device adds sigma: add.accumulate is sequential (np.sum is pairwise)"""
+    return np.cumsum(sig, axis=1)[:, -1]
+
+
 def psis_loo(ll, sig=None):
     """ll: units x S log-likelihood draws (sig: sigma of each, default exp(ll)) -> dict(elpd, p_loo, k, lpd), per unit"""
     ll = np.atleast_2d(np.asarray(ll, dtype=np.float64))
@@ -52,10 +57,7 @@ def psis_loo(ll, sig=None):
         nan = np.full(cells, np.nan)
         return dict(elpd=nan, p_loo=nan.copy(), k=nan.copy(), lpd=nan.copy())
     sig = np.exp(ll) if sig is None else np.asarray(sig, dtype=np.float64)
-    acc = sig[:, 0].copy()
-    for s in range(1, S):                       # in draw order
-        acc = acc + sig[:, s]
-    lpd = np.log(acc / S)
+    lpd = np.log(draw_order_sum(sig) / S)
     M = tail_len(S)
     rs = np.sort(-ll, axis=1)                   # log ratios, ascending
     mx = rs[:, -1]
@@ -81,6 +83,41 @@ def psis_loo(ll, sig=None):
     with np.errstate(all="ignore"):
         elpd = _lse(lwt + (-rs)) - _lse(lwt)
     return dict(elpd=elpd, p_loo=lpd - elpd, k=khat, lpd=lpd)
+
+
+ADVERSARIAL_KINDS = ("logistic", "ties at the cutoff", "all-equal tail", "constant", "Pareto 1.5", "near -700",
+                     "x* = 0", "five decades")
+
+
+def adversarial(S, rs, reps=4):
+    """reps x 8 columns of S log-likelihood draws, kind ADVERSARIAL_KINDS[i % 8] in row i, that reach the edges of the
+    finish: ties, an all-equal tail, constant columns, k > 1, underflow of exp(ll), x* = 0, a wide spread"""
+    cols = []
+    M = tail_len(S)
+    for rep in range(reps):
+        g = rs.standard_normal(S) * (1.0 + rep) + 1.0
+        cols.append(log_sigmoid(g)[1])                                     # a logistic cell
+        c = log_sigmoid(g)[1]
+        if S > M + 1:                                                      # ties at the cutoff, inside and outside the tail
+            srt = np.sort(c)
+            c[(c >= srt[M - 1]) & (c <= srt[M + 1])] = srt[M]
+        cols.append(c)
+        c = log_sigmoid(g)[1]
+        if S > M:                                                          # an all-equal tail, below a distinct cutoff
+            srt = np.sort(c)
+            c[c < srt[M]] = srt[0]
+        cols.append(c)
+        cols.append(np.full(S, -0.25 * (rep + 1)))                         # constant
+        u = rs.uniform(size=S)
+        cols.append(-np.log((u ** -1.5 - 1.0) / 1.5 + 1.0))                # Pareto ratios, shape 1.5: k > 1
+        cols.append(-700.0 - rs.exponential(0.5 + rep, S))                 # ll near -700
+        c = -rs.uniform(0.0, 1.0, S)                                       # x* = 0: a quarter of the tail on the cutoff
+        if S > M and M >= 4:
+            c[:M // 2] = -3.0 - rs.uniform(0.0, 1.0, M // 2)
+            c[M // 2:M + 1] = -3.0
+        cols.append(c)
+        cols.append(np.log(rs.uniform(size=S)) * 10.0 ** rs.uniform(-3, 2))   # spread over five decades
+    return np.stack(cols) if S else np.zeros((8 * reps, 0))
 
 
 def loglik_from_draws(out, y, rs=None):

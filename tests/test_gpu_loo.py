@@ -123,39 +123,10 @@ def test_loo_against_numpy_on_the_stored_draws(G, n, m, missing):
 
 
 # ---- psis_loo() on adversarial columns -------------------------------------------------------------------------------
-def _adversarial(S, rs):
-    cols = []
-    M = P.tail_len(S)
-    for rep in range(4):
-        g = rs.standard_normal(S) * (1.0 + rep) + 1.0
-        cols.append(P.log_sigmoid(g)[1])                                   # a logistic cell
-        c = P.log_sigmoid(g)[1]
-        if S > M + 1:                                                      # ties at the cutoff, inside and outside the tail
-            srt = np.sort(c)
-            c[(c >= srt[M - 1]) & (c <= srt[M + 1])] = srt[M]
-        cols.append(c)
-        c = P.log_sigmoid(g)[1]
-        if S > M:                                                          # an all-equal tail, below a distinct cutoff
-            srt = np.sort(c)
-            c[c < srt[M]] = srt[0]
-        cols.append(c)
-        cols.append(np.full(S, -0.25 * (rep + 1)))                         # constant
-        u = rs.uniform(size=S)
-        cols.append(-np.log((u ** -1.5 - 1.0) / 1.5 + 1.0))                # Pareto ratios, shape 1.5: k > 1
-        cols.append(-700.0 - rs.exponential(0.5 + rep, S))                 # ll near -700
-        c = -rs.uniform(0.0, 1.0, S)                                       # x* = 0: a quarter of the tail on the cutoff
-        if S > M and M >= 4:
-            c[:M // 2] = -3.0 - rs.uniform(0.0, 1.0, M // 2)
-            c[M // 2:M + 1] = -3.0
-        cols.append(c)
-        cols.append(np.log(rs.uniform(size=S)) * 10.0 ** rs.uniform(-3, 2))   # spread over five decades
-    return np.stack(cols) if S else np.zeros((32, 0))
-
-
 @pytest.mark.parametrize("S", [0, 1, 4, 20, 21, 22, 5000])
 def test_psis_loo_adversarial_columns(G, S):
     rs = np.random.default_rng(S + 1)
-    ll = _adversarial(S, rs)
+    ll = P.adversarial(S, rs)
     e, p, k = G.psis_loo(ll)
     ref = P.psis_loo(ll)
     if S == 0:
@@ -172,7 +143,7 @@ def test_psis_loo_adversarial_columns(G, S):
 
 def test_psis_loo_times_its_kernels(G):
     rs = np.random.default_rng(0)
-    ll = _adversarial(200, rs)
+    ll = P.adversarial(200, rs)
     e, p, k, (ms_update, ms_finish) = G.psis_loo(ll, reps=2)
     assert ms_update > 0.0 and ms_finish > 0.0
     assert np.array_equal(e, G.psis_loo(ll)[0])

@@ -104,6 +104,17 @@ def test_threshold():
     assert np.isnan(P.k_threshold(0))
 
 
+def test_draw_order_sum_equals_the_loop_over_draws():
+    """lpd needs the sum of sigma in draw order, bit for bit as the device adds it; cumsum must give the loop's bits"""
+    ll = P.adversarial(5000, np.random.default_rng(5))
+    sig = np.exp(ll)
+    acc = sig[:, 0].copy()
+    for s in range(1, sig.shape[1]):
+        acc = acc + sig[:, s]
+    assert np.array_equal(P.draw_order_sum(sig), acc)
+    assert not np.array_equal(np.sum(sig, axis=1), acc)   # the pairwise sum differs: the test can tell the orders apart
+
+
 def test_constant_column():
     ll = np.full((3, 50), -0.3)
     ll[1] = -2.0
