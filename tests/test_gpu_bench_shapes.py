@@ -4,17 +4,24 @@ compared with the CPU oracle here, through the C ABI.
   C2  1024 x 2000   one full lock-step sweep of the public call against the oracle's gpirtMCMC restatement
   C3  4096 x 10000  the oracle needs hours per sweep, but given theta and L every item is independent (draw-f.cpp:69-71,
                     draw-fstar.cpp:23-29, draw-beta.cpp:16-38) and every respondent's grid draw is independent given f*
-                    (draw-theta.cpp:12-34): each step runs on the FULL GPU state and >= 32 random items / >= 16 random
-                    respondents are checked against the oracle with the same addressed variates (stream maps), with the
-                    fixed-point (int8 tensor-core) products on and off, with and without 5 % missing cells
+                    (draw-theta.cpp:12-34): each step runs on the FULL GPU state and the tile strata of
+                    tests/bench_strata.py (an item in every 64-item tile of the fixed-point products, a respondent in every
+                    128-row tile of the theta contraction) are checked against the oracle with the same addressed variates
+                    (stream maps), with the fixed-point (int8 tensor-core) products on and off, with and without 5 %
+                    missing cells
   C5  16384 x 20000 the same steps on the full C5 state (fixed-point products on, 0 % / 5 % missing): K* solves by blocked
-                    substitution, streaming per-item kernels, the rebuilt factor checked on sampled rows
+                    substitution, streaming per-item kernels, the rebuilt factor checked on the first and last row of
+                    every panel
   n > 4096          the streaming launch shape of the per-item kernels (C5's shape) on small-m problems
 
 Every test asserts WHICH code path ran (gpirt_b200_sampler_uses).  Tolerances as in test_gpu_parity.py: discrete decisions
 (ESS proposal counts, theta grid indices) identical, values to 1e-9 / 1e-8 (solves: cond(S) ~ 1e7)."""
+import time
+
 import numpy as np
 import pytest
+
+import bench_strata as B
 
 pytestmark = pytest.mark.gpu
 
@@ -69,58 +76,69 @@ def _c3_state(G, missing, monkeypatch, int8, workload="c3"):
 def test_c3_sampled_items_and_respondents_against_the_oracle(G, O, monkeypatch, workload, missing, int8):
     """BASELINE configs[2] (the bench workload): one step at a time on the full 4096 x 10000 state.  The same at C5
     (BASELINE configs[4], 16384 x 20000): L Z with K = 16384, the f* solves by blocked substitution (route 1), the theta
-    contraction over 20000 items for 16384 rows and the streaming item kernels."""
+    contraction over 20000 items for 16384 rows and the streaming item kernels.  Items and respondents are the tile
+    strata of tests/bench_strata.py: every 64-item tile of the fixed-point products, every 128-row tile of the theta
+    contraction and every piece of the chunked upload of y holds a compared index."""
     from gpirt_b200 import synthetic
+    t0 = time.time()
     d, s, _lib = _c3_state(G, missing, monkeypatch, int8, workload)
     n, m = d["y"].shape
     big = n > 4096                 # C5: per-item kernels in the streaming shape, K* solves by substitution
     item_shape = ITEM_STREAM if big else ITEM_PERSISTENT
     assert s.uses(4) == (1 if big else 0)
     seed = synthetic.SEED
-    rs = np.random.RandomState(42 + int(100 * missing) + int(int8))
-    J = np.sort(rs.choice(m, 32, replace=False))
-    I = np.sort(rs.choice(n, 16, replace=False))
+    J, I = B.items(m, big), B.respondents(n, big)
     theta = s.get(_lib.THETA); beta = s.get(_lib.BETA); L = s.get(_lib.CHOL)
     assert len(np.unique(theta)) <= 1001 < n, "theta on the grid: duplicated rows, PD only through the jitter"
     yJ = np.asfortranarray(d["y"][:, J])
     ts, prior = O.grid()
+    worst = {}
 
     # ---- draw_f (draw-f.cpp:21-60): proposals nu = L z, shrink counts, new f ----
-    f0 = s.get(_lib.F)
+    f0 = s.get(_lib.F)[:, J]
     sweep = 11
     s.step(_lib.STEP_DRAW_F, sweep)
     assert s.uses(2) == item_shape
-    nu = s.get(_lib.NU); f1 = s.get(_lib.F); nprop = s.get(_lib.ESS_NPROP).astype(int)
-    rng = O.Rng.keyed(seed); rng.set_sweep(sweep); rng.set_item_map(J)
+    nu = s.get(_lib.NU)[:, J]; f1 = s.get(_lib.F)[:, J]; nprop = s.get(_lib.ESS_NPROP).astype(int)
+    # the proposal of every stratum item on all n rows: nu_j = L z_j, one BLAS-3 product for all of them
+    Z = B.keyed_normals(O, seed, sweep, O.P_ESS_Z, J, n)
+    nu_ref = L @ Z
+    # C5: the fixed-point bound K 2^-51 max|L_i| max|z| with L sliced at the fixed scale |L| < 2^L_FIXED_EXP = 2
+    tol = n * 2.0 ** -51 * 2.0 * np.abs(Z).max(axis=0) if big else 1e-11
+    worst["nu"] = np.max(np.abs(nu - nu_ref).max(axis=0) / tol)
+    assert worst["nu"] <= 1.0
+    del Z, nu
     mu = O.linear_mean(theta, beta[:, J])
-    fo, npo = O.draw_f(f0[:, J], yJ, L, mu, rng)
-    for jj, j in enumerate(J[:4]):   # the proposal itself for a few items: nu_j = L z_j
-        z = np.array([O.keyed_normal(seed, sweep, O.P_ESS_Z, int(j), i) for i in range(n)])
-        # C5: the fixed-point bound K 2^-51 max|L_i| max|z| with L sliced at the fixed scale |L| < 2^L_FIXED_EXP = 2
-        tol = n * 2.0 ** -51 * 2.0 * np.abs(z).max() if big else 1e-11
-        assert np.max(np.abs(nu[:, j] - L @ z)) <= tol
+    rng = O.Rng.keyed(seed); rng.set_sweep(sweep)     # items addressed by their global index, no map
+    fo = np.empty_like(f1); npo = np.empty(len(J), dtype=int)
+    for jj, j in enumerate(J):
+        fo[:, jj], _, npo[jj] = O.ess(f0[:, jj], yJ[:, jj], L, mu[:, jj], int(j), rng, nu=nu_ref[:, jj])
     assert np.array_equal(nprop[J], npo), "ESS proposal counts must match the oracle"
-    assert np.max(np.abs(f1[:, J] - fo)) <= 1e-9
+    worst["f"] = np.max(np.abs(f1 - fo)) / 1e-9
+    assert worst["f"] <= 1.0
+    del nu_ref, mu, f0
 
     # ---- draw_fstar (draw-fstar.cpp:10-31) ----
     sweep = 12
     s.step(_lib.STEP_DRAW_FSTAR, sweep)
     fs = s.get(_lib.FSTAR); sd = s.get(_lib.FSTAR_S)
     rng = O.Rng.keyed(seed); rng.set_sweep(sweep); rng.set_item_map(J)
-    fso, so, _ = O.draw_fstar(f1[:, J], theta, ts, L, O.linear_mean(ts, beta[:, J]), rng)
-    assert np.max(np.abs(sd - so)) <= 1e-8
-    assert np.max(np.abs(fs[:, J] - fso)) <= 1e-7 * max(1.0, np.abs(fso).max())
+    fso, so, _ = O.draw_fstar(f1, theta, ts, L, O.linear_mean(ts, beta[:, J]), rng)
+    worst["sd"] = np.max(np.abs(sd - so)) / 1e-8
+    worst["f*"] = np.max(np.abs(fs[:, J] - fso)) / (1e-7 * max(1.0, np.abs(fso).max()))
+    assert worst["sd"] <= 1.0 and worst["f*"] <= 1.0
 
-    # ---- draw_theta (draw-theta.cpp:12-34): log-posterior rows and grid index of sampled respondents ----
+    # ---- draw_theta (draw-theta.cpp:12-34): log-posterior rows and grid index of the stratum respondents ----
     sweep = 13
     s.step(_lib.STEP_DRAW_THETA, sweep)
     idx = s.get(_lib.THETA_IDX).astype(int); logp = s.get(_lib.LOGP); theta_new = s.get(_lib.THETA)
-    rng = O.Rng.keyed(seed); rng.set_sweep(sweep); rng.set_respondent_map(I)
-    tho, idxo, logpo = O.draw_theta(ts, d["y"][I, :], prior, fs, rng, mode=1)
+    tho, idxo, logpo = B.draw_theta_rows(O, ts, d["y"], prior, fs, seed, sweep, I)
     want_ll = logpo - prior[None, :]
-    assert np.max(np.abs(logp[I, :] - want_ll) / np.maximum(1.0, np.abs(want_ll))) <= 1e-12
+    worst["logP"] = np.max(np.abs(logp[I, :] - want_ll) / np.maximum(1.0, np.abs(want_ll))) / 1e-12
+    assert worst["logP"] <= 1.0
     assert np.array_equal(idx[I], idxo), "grid indices must match the oracle (stabilised CDF)"
     assert np.array_equal(theta_new[I], tho)
+    del logp, logpo, want_ll, fs
 
     # ---- draw_beta (draw-beta.cpp:16-38) with the NEW theta and the current f ----
     sweep = 14
@@ -128,21 +146,26 @@ def test_c3_sampled_items_and_respondents_against_the_oracle(G, O, monkeypatch, 
     assert s.uses(3) == item_shape
     b1 = s.get(_lib.BETA)
     rng = O.Rng.keyed(seed); rng.set_sweep(sweep); rng.set_item_map(J)
-    bo, _ = O.draw_beta(beta[:, J], theta_new, yJ, f1[:, J], d["pm"][:, J], d["psd"][:, J], d["pstep"][:, J], rng)
-    assert np.max(np.abs(b1[:, J] - bo)) <= 1e-12
+    bo, _ = O.draw_beta(beta[:, J], theta_new, yJ, f1, d["pm"][:, J], d["psd"][:, J], d["pstep"][:, J], rng)
+    worst["beta"] = np.max(np.abs(b1[:, J] - bo)) / 1e-12
+    assert worst["beta"] <= 1.0
 
     # ---- rebuild (gpirtMCMC.cpp:76-78): the Cholesky chain kernels against the definition ----
-    del nu, f0, f1, L
+    del f1, L
     s.step(_lib.STEP_REBUILD, 0)
     L2 = s.get(_lib.CHOL)
     s.close()
-    S = O.K(theta_new, theta_new) + 1e-3 * np.eye(n)
-    assert np.array_equal(np.triu(L2, 1), np.zeros_like(L2)), "strict upper triangle must be exactly zero"
+    assert not np.triu(L2, 1).any(), "strict upper triangle must be exactly zero"
     if not big:
-        assert np.max(np.abs(L2 @ L2.T - S)) <= 1e-12 * 12
-    else:   # 64 sampled rows (and the first and last) against 2 n u max|S|, as test_gpu_large_n.py::_check_factor
-        R = np.unique(np.r_[0, n - 1, rs.choice(n, 64, replace=False)])
-        assert np.max(np.abs(L2[R, :] @ L2.T - S[R, :])) <= 2 * n * 2.0 ** -53 * np.abs(S).max()
+        S = O.K(theta_new, theta_new) + 1e-3 * np.eye(n)
+        worst["LL^T"] = np.max(np.abs(L2 @ L2.T - S)) / (1e-12 * 12)
+    else:   # first and last row of every 128-row panel against 2 n u max|S|, as test_gpu_large_n.py::_check_factor
+        R = B.panel_rows(n)
+        S = O.K(theta_new[R], theta_new); S[np.arange(R.size), R] += 1e-3
+        worst["LL^T"] = np.max(np.abs(L2[R, :] @ L2.T - S)) / (2 * n * 2.0 ** -53 * np.abs(S).max())
+    assert worst["LL^T"] <= 1.0
+    print("%s %g%% missing int8 %s: %d items, %d respondents; worst error / tolerance %s; %.0f s" % (
+        workload, 100 * missing, int8, len(J), len(I), ", ".join("%s %.2e" % kv for kv in worst.items()), time.time() - t0))
 
 
 @pytest.mark.parametrize("n,m,missing", [(4097, 8, 0.0), (6000, 6, 0.1), (8192, 4, 0.0)])
